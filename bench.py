@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the render hot path on BASELINE.json's headline workload.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     torchrun --nproc-per-node N bench.py --gpus N ...        (one rank per GPU)
 
 Workload (BASELINE.json configs[2], the one the metric is quoted on): a
@@ -58,7 +58,7 @@ UNIT = "Mrays/s"
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=None, help="timed frames (default 5; 30 for c5)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     # None: taken from --config (c3: 1920x1080, 64 spp, depth 5, grid 707)
@@ -94,6 +94,8 @@ def parse_args():
                     help="BASELINE.json configs[0..3]; c3 (the default) is the one the metric is quoted on")
     ap.add_argument("--progressive", action="store_true", default=None,
                     help="accumulate spp samples per frame (CLPT_FLAG_ACCUMULATE)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed frames, write what the last one computed as DIR/<name>.npy (float32)")
     a = ap.parse_args()
     presets = {
         # the reference's own CPU-runnable case: 640x480, 1 spp, 1 bounce, ~1k triangles
@@ -108,6 +110,8 @@ def parse_args():
     for k, v in {**presets["c3"], "progressive": False, **presets[a.config]}.items():
         if getattr(a, k) is None:  # explicit flags win over the preset
             setattr(a, k, v)
+    if a.steps is None:  # the animated loop reports p99 frame times: it wants more frames
+        a.steps = 30 if a.config == "c5" and a.impl == "ours" else 5
     return a
 
 
@@ -304,8 +308,11 @@ def run_reference(a):
         op.render(scene, cam, a.width, a.height, seed=a.seed, sample_base=w * ref_spp, **kw)
     rays, t0 = 0, time.time()
     for k in range(a.steps):
-        rays += op.render(scene, cam, a.width, a.height, seed=a.seed, sample_base=k * ref_spp, **kw)["counters"]["rays"]
+        last = op.render(scene, cam, a.width, a.height, seed=a.seed, sample_base=k * ref_spp, **kw)
+        rays += last["counters"]["rays"]
     secs = time.time() - t0
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"frame": last["rgba"]})
     value = rays / secs / 1e6
     sample = (f"each step = the full {a.width}x{a.height} frame at {ref_spp} of {a.spp} spp, depth {a.depth}; the "
               f"reference's algorithm (CPU port of src/kernel.cl, oracle/oracle_kernel.c) walking THIS repository's "
@@ -359,6 +366,26 @@ def emit(obj):
         os.write(1, line)
     else:
         os.write(_REAL_STDOUT, line)
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each [..., channels] array as <out_dir>/<name>.npy in float32, so that two builds
+    can be compared output for output.  When together they exceed DUMP_LIMIT_BYTES, every array keeps
+    the same fraction of its pixels, at sorted indices drawn with seed 0: the same pixels for the same
+    arguments."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    arrays = {name: np.asarray(arr, dtype=np.float32) for name, arr in arrays.items()}
+    keep_fraction = min(1.0, DUMP_LIMIT_BYTES / sum(a.nbytes for a in arrays.values()))
+    for name, a in arrays.items():
+        if keep_fraction < 1.0:
+            pixels = a.reshape(-1, a.shape[-1])
+            keep = int(len(pixels) * keep_fraction)
+            a = pixels[np.sort(np.random.default_rng(0).choice(len(pixels), size=keep, replace=False))]
+        np.save(out / f"{name}.npy", a)
 
 
 def icosphere(subdiv=3):
@@ -445,7 +472,7 @@ def run_animated(a):
     verts[:len(tv), :3] = tv[:, :3]
     dt, g = 1.0 / 60.0, -1.5
     t_build, t_upload, t_render, t_frame, dev_build, dev_pack = [], [], [], [], [], []
-    frames = a.warmup + max(a.steps, 30)
+    frames = a.warmup + a.steps
     import gc
 
     gc.disable()  # a collection in the middle of a frame is a 10+ ms outlier that is not the renderer's
@@ -500,6 +527,10 @@ def run_animated(a):
             t_stream.append(t3 - t0)
     r.read_wait(0)
     gc.enable()
+    if a.dump_outputs:
+        frame = r.read_image()
+        if rank == 0:  # `delivered`: the RGBA8 texels the last streamed frame landed in host memory
+            dump_outputs(a.dump_outputs, {"frame": frame, "delivered": hosts[(2 * frames - 1) % 2]})
     # self-check: the LAST frame (whatever tree the last rebuild made) against the oracle walking that tree
     parity = {"checked": False}
     if not a.no_parity_check:
@@ -676,6 +707,10 @@ def main():
     if rank == 0:
         print(f"e2e steps (ms): {e2e_each}, drain {t_drain * 1e3:.3f} ms, total {e2e_s * 1e3:.3f} ms", file=sys.stderr)
     d2h_bytes = a.width * a.height * (4 if a.readback == "rgba8" else 16)
+    if a.dump_outputs:
+        frame = r.read_image()
+        if rank == 0:  # `delivered`: what the last end-to-end step landed in host memory, in the --readback format
+            dump_outputs(a.dump_outputs, {"frame": frame, "delivered": host_np[(a.steps - 1) & 1]})
 
     # ---- self-check frame: the timed parameters, read back once more (outside every timed region) ----
     import hashlib

@@ -13,7 +13,7 @@
  *
  * The kernel source is not in this repository.  `make -C oracle ref` links
  * it into oracle/_ref/libref_kernel.so as an opaque data blob taken from
- * /root/reference/src/kernel.cl where it lies (ld -r -b binary); oracle/_ref is
+ * $CLPT_REFERENCE/src/kernel.cl where it lies (ld -r -b binary); oracle/_ref is
  * git-ignored and only travels to the GPU box next to the other built
  * checkers.
  *

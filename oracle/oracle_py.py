@@ -5,8 +5,8 @@ Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline /
 
   liboracle.so            CPU restatement of src/kernel.cl (oracle_kernel.c)
   _ref/libref_host.so     the reference's own host code, compiled unmodified
-                          from /root/reference (Makefile target `ref`); present
-                          only where it was built
+                          from the checkout $CLPT_REFERENCE names (Makefile
+                          target `ref`); present only where it was built
 """
 from __future__ import annotations
 
@@ -196,7 +196,7 @@ def _ref_kernel():
 def ref_kernel_available() -> tuple[bool, str]:
     """(usable, 'platform / device' or the reason it is not)."""
     if not REF_KERNEL_LIB.exists():
-        return False, "oracle/_ref/libref_kernel.so not built (needs /root/reference at build time)"
+        return False, "oracle/_ref/libref_kernel.so not built (needs $CLPT_REFERENCE at build time)"
     msg = C.create_string_buffer(512)
     rc = _ref_kernel().refcl_available(msg, 512)
     return rc == 0, msg.value.decode(errors="replace")

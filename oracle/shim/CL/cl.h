@@ -3,7 +3,7 @@
  * TEST INFRASTRUCTURE.  This image has no OpenCL headers.  The reference's
  * host files (list/vector/matrix/camera/kd_tree/model .c) use nothing from
  * OpenCL except these scalar and 16-byte vector typedefs, so this shim is all
- * that is needed to compile them UNMODIFIED from /root/reference (see
+ * that is needed to compile them UNMODIFIED from $CLPT_REFERENCE (see
  * oracle/Makefile).  Layouts follow the Khronos cl_platform.h: 16-byte
  * unions addressed as .s[i]; the 3-component types alias the 4-component ones.
  */

@@ -1,8 +1,8 @@
 """Regenerate tests/golden/host_golden.json.
 
-Run in the build container, where /root/reference exists: the values are
+Run where $CLPT_REFERENCE names a checkout of the reference: the values are
 produced by the REFERENCE's own host code (oracle/_ref/libref_host.so, built by
-oracle/Makefile from /root/reference/src/*.c unmodified), not by this repo's
+oracle/Makefile from $CLPT_REFERENCE/src/*.c unmodified), not by this repo's
 code.  The file pins, for deterministic synthetic scenes, the sha256 of the
 reference builder's node array and tri_indices, and camera matrices as raw
 float bits.
@@ -76,7 +76,7 @@ CAMERAS = {
 
 
 def main():
-    assert op.have_ref(), "oracle/_ref/libref_host.so missing: run `make -C oracle ref` where /root/reference exists"
+    assert op.have_ref(), "oracle/_ref/libref_host.so missing: run `make -C oracle ref` with $CLPT_REFERENCE set"
     assert op.ref().ref_sizeof_kdnode() == 68 and op.ref().ref_sizeof_camera() == 48
     out = {"generated_by": "tests/golden/make_golden.py using oracle/_ref/libref_host.so (reference host code, unmodified)",
            "kd": {}, "cam": {}}

@@ -67,14 +67,6 @@ def test_gl_presentation_hook(clpt, tmp_path):
     scenes.write_obj_text(str(obj), v, c, n)
     out = subprocess.run([str(exe), "320", "240", str(obj)], capture_output=True, text=True, timeout=120)
     print(out.stdout[-2000:], out.stderr[-2000:])
-    log = ROOT / "gpurun_out"
-    if log.is_dir():
-        import os
-
-        devs = subprocess.run("ls -la /dev/dri /dev/nvidia* 2>&1 | head -30", shell=True, capture_output=True, text=True)
-        (log / "egl_present.txt").write_text(
-            f"exit {out.returncode}\n{out.stdout}\n{out.stderr}\n--- devices ---\n{devs.stdout}\n"
-            f"NVIDIA_DRIVER_CAPABILITIES={os.environ.get('NVIDIA_DRIVER_CAPABILITIES')}\n")
     if out.returncode == 77:
         pytest.skip("no usable EGL/OpenGL context here: " + out.stdout.strip().splitlines()[-1])
     if out.returncode < 0 and "CONTEXT:" not in out.stdout:

@@ -1,5 +1,6 @@
-"""The reference's own kernel.cl (unmodified, via the box's OpenCL ICD) against
-the oracle restatement and against the CUDA path.
+"""The reference's own kernel.cl (unmodified, run through an OpenCL ICD by
+tests/golden/make_ref_kernel_golden.py) against the oracle restatement and
+against the CUDA path.
 
 This is what pins the oracle: oracle/cl_harness.c runs the reference's device
 code as shipped (first-hit normal colour) on the same 68-byte node arrays.  The
@@ -13,10 +14,12 @@ a few ulp.  NVIDIA's OpenCL compiler rejects the unmodified source (a __global
 pointer passed to an unqualified parameter); oracle/cl_harness.c documents the
 one-declaration address-space patch it applies in memory, nothing else.
 
-GPU half (-m gpu): live run on the box.  CPU half: the frames such a run
-produced, committed as tests/golden/ref_kernel_golden.npz.
+The frames such a run produced are committed as tests/golden/ref_kernel_golden.npz.
+CPU half: the oracle against them.  GPU half (-m gpu): the CUDA path against
+them, and bit for bit against the oracle.
 """
 import json
+import os
 from pathlib import Path
 
 import numpy as np
@@ -106,9 +109,9 @@ def test_bounce_rewrite_is_textual(oracle):
     the renamed callee and the depth literal (oracle/cl_harness.c: bounce_source)."""
     import difflib
 
-    ref_src = Path("/root/reference/src/kernel.cl")
-    if not ref_src.exists() or not oracle.REF_KERNEL_LIB.exists():
-        pytest.skip("needs /root/reference and oracle/_ref (build container only)")
+    ref_src = Path(os.environ.get("CLPT_REFERENCE", ""), "src", "kernel.cl")
+    if not os.environ.get("CLPT_REFERENCE") or not ref_src.exists() or not oracle.REF_KERNEL_LIB.exists():
+        pytest.skip("needs the reference's kernel.cl ($CLPT_REFERENCE) and oracle/_ref built from it")
     orig = ref_src.read_text()
     lines = orig.splitlines()
     start = next(i for i, l in enumerate(lines) if l.startswith("trace_ray(Ray r,")) - 1
@@ -135,17 +138,16 @@ def test_bounce_rewrite_is_textual(oracle):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("bounce_depth", [0, 2, 5])
-@pytest.mark.parametrize("name,w,h", [("hf22_canonical", 640, 480), ("cornell", 640, 480),
-                                      ("hf60_reference", 480, 270), ("soup3000", 320, 320)])
-def test_reference_kernel_live(clpt, oracle, renderer, name, w, h, bounce_depth):
-    ok, what = oracle.ref_kernel_available()
-    if not ok:
-        pytest.skip("reference kernel cannot run here: " + what)
+@pytest.mark.parametrize("name", ["hf22_canonical", "hf22n_canonical", "hf60_reference", "cornell", "soup3000"])
+def test_cuda_vs_reference_kernel_golden(clpt, oracle, renderer, name, bounce_depth):
+    """The CUDA frame against the reference kernel's committed frame of the same case, and bit for
+    bit against the oracle's."""
+    z = np.load(GOLDEN)
+    ref_rgb = z[name if bounce_depth == 0 else f"{name}_d{bounce_depth}"]
+    h, w = ref_rgb.shape[:2]
     gen, camkw = _cases()[name]
     scene = clpt.build_kd(*gen())
     cam = clpt.cam_matrix(clpt.make_camera(**camkw), h)
-    ref_rgba, _ = oracle.ref_kernel_render(scene, cam, w, h, bounce_depth=bounce_depth)
-    assert np.all(ref_rgba[..., 3] == 1.0)
     ref = _oracle_frame(oracle, scene, cam, w, h, bounce_depth)
     want = ref["rgba"]
     renderer.set_meshes(scene)
@@ -155,5 +157,5 @@ def test_reference_kernel_live(clpt, oracle, renderer, name, w, h, bounce_depth)
     renderer.execute()
     got = renderer.read_image()
     assert np.array_equal(got.view(np.uint32), want.view(np.uint32))  # CUDA == oracle, bit for bit
-    s = _compare(ref_rgba[..., :3], dict(ref, rgba=got))                # CUDA vs the reference kernel itself
+    s = _compare(ref_rgb, dict(ref, rgba=got))                          # CUDA vs the reference kernel itself
     _check(s)
