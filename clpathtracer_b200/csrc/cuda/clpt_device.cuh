@@ -62,10 +62,6 @@ struct ClptScene {
 };
 
 #define CLPT_MAX_PEERS 8
-// A "fat" leaf for the automatic engine choice: trees whose triangle slots mostly live in
-// leaves of at least this many triangles are rendered by engine 2.
-#define CLPT_COOP_LEAF_MIN 8
-#define CLPT_FAT_ENGINE_MIN_REFS 500000
 
 struct ClptFrame {
     float cam[16]; // row-major inverse camera matrix

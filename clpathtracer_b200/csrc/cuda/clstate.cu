@@ -88,37 +88,6 @@ void nccl_check(ncclResult_t r, const char *file, int line) {
 
 ClptPackedScene g_packed; // host staging of the re-laid-out scene (page-locked once CLInit ran)
 
-template <typename T>
-struct DevBuf {
-    T *ptr = nullptr;
-    size_t count = 0, capacity = 0;
-    void release() {
-        if (ptr) CU(cudaFree(ptr));
-        ptr = nullptr;
-        count = capacity = 0;
-    }
-    // The reference frees and re-creates every buffer at its exact size on each
-    // upload (resize_buffer, src/CLState.c:92-102).  cudaFree/cudaMalloc cost a
-    // device synchronisation each, which dominates re-uploads of an animated scene,
-    // so the allocation is kept while it is big enough and not more than 2x too big.
-    void resize(size_t n) {
-        if (n > capacity || n * 2 < capacity) {
-            release();
-            if (n) CU(cudaMalloc((void **)&ptr, n * sizeof(T)));
-            capacity = n;
-        }
-        count = n;
-        if (n == 0) release();
-    }
-    void upload(const T *src, size_t n, cudaStream_t s) {
-        resize(n);
-        if (n) {
-            CU(cudaMemcpyAsync(ptr, src, n * sizeof(T), cudaMemcpyHostToDevice, s));
-            CU(cudaStreamSynchronize(s));
-        }
-    }
-};
-
 struct {
     bool inited = false;
     int device = -1; // -1: take $CLPT_DEVICE or 0
@@ -131,17 +100,14 @@ struct {
     kd host_kd = { nullptr, nullptr, nullptr, nullptr, nullptr };
     bool owns_kd = false;
 
-    DevBuf<uint2> nodes;
-    DevBuf<float4> leaves, tri, flat_n, norms;
+    ClptSceneLayout layout; // the traversal layout of the current scene, whichever path made it
+    DevBuf<float4> norms;
     DevBuf<int4> corners;
-    DevBuf<int> lut;
-    // device-side build (CLBuildMeshes): the mesh, the wire-format tree and its re-layout all live
-    // on the device; `scene` then points into gpu_packed instead of the buffers above
+    // device-side build (CLBuildMeshes): the mesh and the wire-format tree live on the device
     DevBuf<float4> verts;
     ClptGpuBuildParams build_params;
     ClptGpuTree gpu_tree;
-    ClptGpuPacked gpu_packed;
-    bool scene_on_gpu = false; // the traversal layout in use is gpu_packed
+    bool scene_on_gpu = false; // gpu_tree is the tree of the current scene
     bool mesh_on_gpu = false;  // verts/corners hold a mesh uploaded by CLBuildMeshes
     float last_build_ms = 0, last_pack_ms = 0;
     DevBuf<unsigned char> objects;
@@ -194,7 +160,7 @@ struct {
     } rd[2];
     unsigned long long rd_issued = 0;
     int engine = 0;      // 0 auto, 1 full occupancy, 2 fat-leaf variant (fewer resident blocks)
-    int auto_engine = 1; // what "auto" means for the current tree (decided in upload_scene)
+    int auto_engine = 1; // what "auto" means for the current tree (decided in adopt_layout)
     int last_engine = 1;
 
     int rank = 0, nranks = 1, tile_rows = 8;
@@ -235,17 +201,50 @@ int local_rows_for(int height) {
 
 void rebuild_scene_struct() {
     ClptScene &S = St.scene;
-    S.nodes = St.scene_on_gpu ? St.gpu_packed.nodes : St.nodes.ptr;
-    S.leaves = St.scene_on_gpu ? St.gpu_packed.leaves : St.leaves.ptr;
-    S.tri = St.scene_on_gpu ? St.gpu_packed.tri : St.tri.ptr;
+    S.nodes = St.layout.nodes.ptr;
+    S.leaves = St.layout.leaves.ptr;
+    S.tri = St.layout.tri.ptr;
     S.corners = St.corners.ptr;
-    S.flat_n = St.scene_on_gpu ? St.gpu_packed.flat_n : St.flat_n.ptr;
-    S.lut = St.scene_on_gpu ? St.gpu_packed.lut : St.lut.ptr;
+    S.flat_n = St.layout.flat_n.ptr;
+    S.lut = St.layout.lut.ptr;
     S.norms = St.norms.ptr;
     S.tri_material = St.tri_material.ptr;
     S.materials = St.materials.ptr;
     S.n_materials = (int)St.materials.count;
     S.n_norms = (int)St.norms.count;
+}
+
+// St.layout holds a new scene of `n_prims` primitives: point the launch at it and choose the engine.
+void adopt_layout(int n_prims) {
+    const ClptSceneLayout &L = St.layout;
+    ClptScene &S = St.scene;
+    S.n_nodes = L.n_nodes;
+    S.n_leaves = L.n_leaves;
+    S.n_refs = L.n_refs;
+    S.n_prims = n_prims;
+    for (int a = 0; a < 3; a++) {
+        S.root_min[a] = L.root_min[a];
+        S.root_max[a] = L.root_max[a];
+        S.lut_dim[a] = L.lut_dim[a];
+        S.lut_scale[a] = L.lut_scale[a];
+    }
+    rebuild_scene_struct();
+    St.have_scene = true;
+    // "automatic" engine for this tree: the fat-leaf variant when most triangle slots live in
+    // fat leaves AND the tree is big (the reference builder's DEPTH-15 trees from a few hundred
+    // thousand triangles up; measured at 100k triangles engine 1 is still 10% faster)
+    St.auto_engine = (L.n_refs >= CLPT_FAT_ENGINE_MIN_REFS && L.fat_refs * 2 > (size_t)L.n_refs) ? 2 : 1;
+    if (const char *e = getenv("CLPT_ENGINE")) {
+        if (atoi(e) == 1 || atoi(e) == 2) St.auto_engine = atoi(e);
+    }
+}
+
+// Host staging -> St.layout, one copy per array on the library's stream.
+template <typename T, typename S>
+void upload_layout_array(DevBuf<T> &dst, const ClptStaging<S> &src) {
+    static_assert(sizeof(T) == sizeof(S), "staging and device element sizes differ");
+    dst.reserve(src.size());
+    if (src.size()) CU(cudaMemcpyAsync(dst.ptr, src.data(), src.size() * sizeof(T), cudaMemcpyHostToDevice, St.stream));
 }
 
 void upload_scene(const kdnode *nodes, size_t node_bytes, const int *tri_indices, size_t tri_index_bytes,
@@ -265,12 +264,14 @@ void upload_scene(const kdnode *nodes, size_t node_bytes, const int *tri_indices
         exit(EXIT_FAILURE);
     }
     const auto t1 = std::chrono::steady_clock::now();
-    St.nodes.upload(reinterpret_cast<const uint2 *>(packed.nodes.data()), packed.nodes.size(), St.stream);
-    St.leaves.upload(reinterpret_cast<const float4 *>(packed.leaves.data()), packed.leaves.size(), St.stream);
-    St.tri.upload(reinterpret_cast<const float4 *>(packed.tri.data()), packed.tri.size(), St.stream);
-    St.flat_n.upload(reinterpret_cast<const float4 *>(packed.flat_n.data()), packed.flat_n.size(), St.stream);
+    upload_layout_array(St.layout.nodes, packed.nodes);
+    upload_layout_array(St.layout.leaves, packed.leaves);
+    upload_layout_array(St.layout.tri, packed.tri);
+    upload_layout_array(St.layout.flat_n, packed.flat_n);
+    upload_layout_array(St.layout.lut, packed.lut);
+    static_cast<ClptLayoutInfo &>(St.layout) = packed;
+    CU(cudaStreamSynchronize(St.stream)); // (the staging is rewritten by the next upload)
     St.corners.upload(reinterpret_cast<const int4 *>(tris), tri_bytes / sizeof(cl_int3), St.stream);
-    St.lut.upload(packed.lut.data(), packed.lut.size(), St.stream);
     if (n_norms) {
         St.norms.upload(reinterpret_cast<const float4 *>(norms), n_norms, St.stream);
     } else {
@@ -279,34 +280,7 @@ void upload_scene(const kdnode *nodes, size_t node_bytes, const int *tri_indices
     // per-triangle materials belong to the previous mesh
     St.tri_material.release();
     St.scene_on_gpu = St.mesh_on_gpu = false; // (the corner buffer now belongs to this scene)
-    ClptScene &S = St.scene;
-    S.n_nodes = packed.n_nodes;
-    S.n_leaves = packed.n_leaves;
-    S.n_refs = packed.n_refs;
-    S.n_prims = packed.n_prims;
-    for (int a = 0; a < 3; a++) {
-        S.root_min[a] = packed.root_min[a];
-        S.root_max[a] = packed.root_max[a];
-        S.lut_dim[a] = packed.lut_dim[a];
-        S.lut_scale[a] = packed.lut_scale[a];
-    }
-    rebuild_scene_struct();
-    St.have_scene = true;
-    // "automatic" engine for this tree: the fat-leaf variant when most triangle slots live in
-    // fat leaves AND the tree is big (the reference builder's DEPTH-15 trees from a few hundred
-    // thousand triangles up; measured at 100k triangles engine 1 is still 10% faster)
-    {
-        size_t fat_refs = 0;
-        for (int l = 0; l < packed.n_leaves; l++) {
-            int count;
-            memcpy(&count, &packed.leaves[4 * (size_t)l + 1].w, sizeof(int));
-            if (count >= CLPT_COOP_LEAF_MIN) fat_refs += (size_t)count;
-        }
-        St.auto_engine = (packed.n_refs >= CLPT_FAT_ENGINE_MIN_REFS && fat_refs * 2 > (size_t)packed.n_refs) ? 2 : 1;
-        if (const char *e = getenv("CLPT_ENGINE")) {
-            if (atoi(e) == 1 || atoi(e) == 2) St.auto_engine = atoi(e);
-        }
-    }
+    adopt_layout(packed.n_prims);
     if (timing) {
         const auto t2 = std::chrono::steady_clock::now();
         fprintf(stderr, "CLSetMeshes: pack %.3f ms, upload %.3f ms (%d nodes, %d leaves, %d triangle slots, %zu table cells)\n",
@@ -480,6 +454,32 @@ void p2p_setup() {
 
 void release_read_pipeline();
 
+// The AOV buffers at the size of the render target, cleared (prim_id -1: no hit).
+void alloc_aovs() {
+    const size_t px = (size_t)St.width * St.height;
+    St.aov_prim.resize(px);
+    St.aov_t.resize(px);
+    St.aov_uv.resize(px);
+    CU(cudaMemsetAsync(St.aov_prim.ptr, 0xff, px * sizeof(int), St.stream));
+    CU(cudaMemsetAsync(St.aov_t.ptr, 0, px * sizeof(float), St.stream));
+    CU(cudaMemsetAsync(St.aov_uv.ptr, 0, px * sizeof(float2), St.stream));
+    CU(cudaStreamSynchronize(St.stream));
+}
+
+// Frees the render target and the buffers frames made for it (the caller has torn down the peer
+// mappings and the read-back pipeline first).
+void release_targets() {
+    St.image.release();
+    St.slab.release();
+    St.gathered.release();
+    St.scratch.release();
+    St.accum.release();
+    St.accum_sum.release();
+    St.aov_prim.release();
+    St.aov_t.release();
+    St.aov_uv.release();
+}
+
 void alloc_targets() {
     p2p_teardown();
     release_read_pipeline();
@@ -495,14 +495,7 @@ void alloc_targets() {
         St.slab.release();
         St.gathered.release();
     }
-    if (St.aov) {
-        St.aov_prim.resize(px);
-        St.aov_t.resize(px);
-        St.aov_uv.resize(px);
-        CU(cudaMemsetAsync(St.aov_prim.ptr, 0xff, px * sizeof(int), St.stream));
-        CU(cudaMemsetAsync(St.aov_t.ptr, 0, px * sizeof(float), St.stream));
-        CU(cudaMemsetAsync(St.aov_uv.ptr, 0, px * sizeof(float2), St.stream));
-    }
+    if (St.aov) alloc_aovs();
     St.scratch.release();
     St.accum.release();
     St.accum_sum.release();
@@ -872,39 +865,17 @@ void CLTerminate(void) {
         St.comm_ranks = 0;
     }
     if (clpt_gl_registered()) clpt_gl_unregister();
-    St.nodes.release();
-    St.leaves.release();
-    St.tri.release();
-    St.flat_n.release();
+    St.layout.release();
     St.norms.release();
     St.corners.release();
-    St.lut.release();
     St.verts.release();
-    {
-        auto drop = [](auto *&p) {
-            if (p) CU(cudaFree(p));
-            p = nullptr;
-        };
-        drop(St.gpu_tree.wire), drop(St.gpu_tree.tri_indices);
-        drop(St.gpu_packed.nodes), drop(St.gpu_packed.leaves), drop(St.gpu_packed.tri), drop(St.gpu_packed.lut);
-        drop(St.gpu_packed.flat_n);
-        St.gpu_tree = ClptGpuTree();
-        St.gpu_packed = ClptGpuPacked();
-        St.scene_on_gpu = St.mesh_on_gpu = false;
-        clpt_gpu_build_release();
-    }
+    St.gpu_tree.release();
+    St.scene_on_gpu = St.mesh_on_gpu = false;
+    clpt_gpu_build_release();
     St.objects.release();
     St.materials.release();
     St.tri_material.release();
-    St.image.release();
-    St.slab.release();
-    St.gathered.release();
-    St.scratch.release();
-    St.accum.release();
-    St.accum_sum.release();
-    St.aov_prim.release();
-    St.aov_t.release();
-    St.aov_uv.release();
+    release_targets();
     St.counters.release();
     St.work_counter.release();
     St.row_cost.release();
@@ -961,8 +932,7 @@ void CLSetMeshes(kd *models) {
     kd m = models[0];                                                     // models[0] only, :130
     // The reference never frees on a re-set (src/CLState.c:124-131 overwrites State.kd), so calling
     // CLSetMeshes again with the SAME kd -- an in-place updated scene, or simply a repeat -- is legal
-    // there.  The previously adopted lists are released only when they are different lists.
-    // A previously adopted list is released only if the new kd does not carry it again.
+    // there.  A previously adopted list is released only if the new kd does not carry it again.
     if (St.owns_kd) {
         const void *incoming[5] = { m.node_vec, m.tri_indices, m.vert_vec, m.norm_vec, m.tri_vec };
         void *held[5] = { St.host_kd.node_vec, St.host_kd.tri_indices, St.host_kd.vert_vec, St.host_kd.norm_vec,
@@ -1010,7 +980,7 @@ void rebuild_on_device(const char *who) {
         exit(EXIT_FAILURE);
     }
     CU(cudaEventRecord(St.ev_build[1], St.stream));
-    if (!clpt_gpu_pack(St.gpu_tree, St.verts.ptr, St.corners.ptr, (int)(n_corners / 3), St.gpu_packed, St.stream, err,
+    if (!clpt_gpu_pack(St.gpu_tree, St.verts.ptr, St.corners.ptr, (int)(n_corners / 3), St.layout, St.stream, err,
                        sizeof err)) {
         fprintf(stderr, "%s: invalid scene: %s\n", who, err);
         exit(EXIT_FAILURE);
@@ -1020,26 +990,7 @@ void rebuild_on_device(const char *who) {
     CU(cudaEventElapsedTime(&St.last_build_ms, St.ev_build[0], St.ev_build[1]));
     CU(cudaEventElapsedTime(&St.last_pack_ms, St.ev_build[1], St.ev_build[2]));
     St.scene_on_gpu = true;
-    ClptScene &S = St.scene;
-    S.n_nodes = St.gpu_packed.n_nodes;
-    S.n_leaves = St.gpu_packed.n_leaves;
-    S.n_refs = St.gpu_packed.n_refs;
-    S.n_prims = (int)(n_corners / 3);
-    for (int a = 0; a < 3; a++) {
-        S.root_min[a] = St.gpu_packed.root_min[a];
-        S.root_max[a] = St.gpu_packed.root_max[a];
-        S.lut_dim[a] = St.gpu_packed.lut_dim[a];
-        S.lut_scale[a] = St.gpu_packed.lut_scale[a];
-    }
-    rebuild_scene_struct();
-    St.have_scene = true;
-    St.auto_engine = (St.gpu_packed.n_refs >= CLPT_FAT_ENGINE_MIN_REFS &&
-                      St.gpu_packed.fat_refs * 2 > (size_t)St.gpu_packed.n_refs)
-                         ? 2
-                         : 1;
-    if (const char *e = getenv("CLPT_ENGINE")) {
-        if (atoi(e) == 1 || atoi(e) == 2) St.auto_engine = atoi(e);
-    }
+    adopt_layout((int)(n_corners / 3));
 }
 } // namespace
 
@@ -1105,8 +1056,8 @@ void CLDownloadKd(kd *out) {
     out->vert_vec = (Vector4 *)init_list(St.verts.count, sizeof(Vector4));
     out->tri_vec = (cl_int3 *)init_list(St.corners.count, sizeof(cl_int3));
     out->norm_vec = (Vector4 *)init_list(St.norms.count, sizeof(Vector4));
-    CU(cudaMemcpy(out->node_vec, St.gpu_tree.wire, n * sizeof(kdnode), cudaMemcpyDeviceToHost));
-    if (r) CU(cudaMemcpy(out->tri_indices, St.gpu_tree.tri_indices, r * sizeof(int), cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(out->node_vec, St.gpu_tree.wire.ptr, n * sizeof(kdnode), cudaMemcpyDeviceToHost));
+    if (r) CU(cudaMemcpy(out->tri_indices, St.gpu_tree.tri_indices.ptr, r * sizeof(int), cudaMemcpyDeviceToHost));
     CU(cudaMemcpy(out->vert_vec, St.verts.ptr, St.verts.count * sizeof(Vector4), cudaMemcpyDeviceToHost));
     CU(cudaMemcpy(out->tri_vec, St.corners.ptr, St.corners.count * sizeof(cl_int3), cudaMemcpyDeviceToHost));
     if (St.norms.count) {
@@ -1180,15 +1131,7 @@ void CLDeleteImage(void) {
     p2p_teardown(); // collective: no rank frees a frame its peers still map
     release_read_pipeline();
     if (clpt_gl_registered()) clpt_gl_unregister();
-    St.image.release();
-    St.slab.release();
-    St.gathered.release();
-    St.scratch.release();
-    St.accum.release();
-    St.accum_sum.release();
-    St.aov_prim.release();
-    St.aov_t.release();
-    St.aov_uv.release();
+    release_targets();
     St.have_image = St.headless = false;
     St.width = St.height = 0;
 }
@@ -1250,17 +1193,7 @@ void CLReadImageWait(int leave_pending) {
 void CLEnableAOV(int enable) {
     require_init("CLEnableAOV");
     St.aov = enable != 0;
-    if (St.have_image) {
-        const size_t px = (size_t)St.width * St.height;
-        if (St.aov && St.aov_prim.count != px) {
-            St.aov_prim.resize(px);
-            St.aov_t.resize(px);
-            St.aov_uv.resize(px);
-            CU(cudaMemset(St.aov_prim.ptr, 0xff, px * sizeof(int)));
-            CU(cudaMemset(St.aov_t.ptr, 0, px * sizeof(float)));
-            CU(cudaMemset(St.aov_uv.ptr, 0, px * sizeof(float2)));
-        }
-    }
+    if (St.have_image && St.aov && St.aov_prim.count != (size_t)St.width * St.height) alloc_aovs();
 }
 
 void CLReadAOV(int *prim_id, float *t_hit, float *uv) {

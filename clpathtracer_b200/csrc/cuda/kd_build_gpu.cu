@@ -712,36 +712,20 @@ __global__ void push_ropes_kernel(int *__restrict__ wire, const LevelState *__re
 }
 
 bool g_last_build_recorded = false;
-size_t g_reallocations = 0; // (a recorded build holds raw pointers: it is re-recorded when any buffer moved)
-
-template <typename T>
-void ensure(T *&ptr, size_t &cap, size_t want) {
-    if (want <= cap) return;
-    g_reallocations++;
-    if (ptr) CU(cudaFree(ptr));
-    const size_t n = want + want / 4 + 1024;
-    CU(cudaMalloc((void **)&ptr, n * sizeof(T)));
-    cap = n;
-}
 
 // Working storage, kept between builds (an animated scene rebuilds every frame).
 struct Workspace {
-    float *lo = nullptr, *hi = nullptr;
-    size_t bounds_cap = 0, bounds_cap2 = 0;
-    int *ref_tri[2] = { nullptr, nullptr }, *ref_node[2] = { nullptr, nullptr };
-    size_t ref_cap[2][2] = { { 0, 0 }, { 0, 0 } };
-    ANode *nodes[2] = { nullptr, nullptr };
-    size_t node_cap[2] = { 0, 0 };
-    Decision *dec = nullptr;
-    size_t dec_cap = 0;
-    unsigned *hist = nullptr;
-    size_t hist_cap = 0;
-    Triple *ref_scan = nullptr, *node_scan = nullptr, *tiles = nullptr, *totals = nullptr;
-    size_t ref_scan_cap = 0, node_scan_cap = 0, tiles_cap = 0, totals_cap = 0;
-    int *box_keys = nullptr, *bad = nullptr, *box_init = nullptr;
-    size_t box_cap = 0, bad_cap = 0, box_init_cap = 0;
-    LevelState *level = nullptr; // [0] the build's, [1] scratch (`n` of a stand-alone scan)
-    size_t level_cap = 0;
+    DevBuf<float> lo, hi;
+    DevBuf<int> ref_tri[2], ref_node[2];
+    DevBuf<ANode> nodes[2];
+    DevBuf<Decision> dec;
+    DevBuf<unsigned> hist;
+    DevBuf<Triple> ref_scan, node_scan, tiles, totals;
+    DevBuf<int> box_keys, bad, box_init;
+    DevBuf<LevelState> level; // [0] the build's, [1] scratch (`n` of a stand-alone scan)
+    // the re-layout's (clpt_gpu_pack)
+    DevBuf<int> new_of;
+    DevBuf<Triple> wire_scan;
     struct Pinned { // what comes back to the host
         Triple totals[2]; // [0] references, [1] nodes
         int bad;
@@ -766,8 +750,8 @@ struct Workspace {
 
 void ensure_host() {
     if (!W.host) CU(cudaMallocHost((void **)&W.host, sizeof(Workspace::Pinned)));
-    ensure(W.level, W.level_cap, (size_t)2);
-    ensure(W.totals, W.totals_cap, (size_t)2);
+    W.level.reserve(2);
+    W.totals.reserve(2);
 }
 
 void drop_graph() {
@@ -783,7 +767,7 @@ template <typename FA, typename FB>
 void scan2(const int *na, size_t cap_a, FA fa, Triple *out_a, const int *nb, size_t cap_b, FB fb, Triple *out_b,
            Triple *total_dev, cudaStream_t s) {
     const int ta = scan_tiles(cap_a), tb = scan_tiles(cap_b);
-    Triple *sums_a = W.tiles, *sums_b = W.tiles + ta;
+    Triple *sums_a = W.tiles.ptr, *sums_b = W.tiles.ptr + ta;
     scan_tile_sums_kernel<<<ta + tb, SCAN_BLOCK, 0, s>>>(ta, na, fa, sums_a, nb, fb, sums_b);
     scan_tile_offsets_kernel<<<2, 1024, 0, s>>>(sums_a, ta, sums_b, tb, total_dev);
     scan_write_kernel<<<ta + tb, SCAN_BLOCK, 0, s>>>(ta, na, fa, sums_a, out_a, nb, fb, sums_b, out_b, total_dev);
@@ -801,13 +785,14 @@ struct BuildArgs {
 
 // Triangle bounds, scene box, the root node and its reference list, the level state.
 void enqueue_prologue(const BuildArgs &A, cudaStream_t s) {
-    CU(cudaMemsetAsync(W.bad, 0, sizeof(int), s));
-    tri_bounds_kernel<<<(A.n_tris + T - 1) / T, T, 0, s>>>(A.verts, A.corners, A.n_tris, A.n_verts, W.lo, W.hi, W.bad);
-    CU(cudaMemcpyAsync(W.box_keys, W.box_init, 6 * sizeof(int), cudaMemcpyDeviceToDevice, s));
-    scene_box_kernel<<<std::min(1024, (A.n_tris + T - 1) / T), T, 0, s>>>(W.lo, W.hi, A.n_tris, W.box_keys);
-    CU(cudaMemcpyAsync(&W.host->bad, W.bad, sizeof(int), cudaMemcpyDeviceToHost, s));
-    root_kernel<<<(A.n_tris + T - 1) / T, T, 0, s>>>(W.box_keys, A.n_tris, A.max_depth, W.nodes[0], W.ref_tri[0],
-                                                     W.ref_node[0], W.level, W.bad);
+    CU(cudaMemsetAsync(W.bad.ptr, 0, sizeof(int), s));
+    tri_bounds_kernel<<<(A.n_tris + T - 1) / T, T, 0, s>>>(A.verts, A.corners, A.n_tris, A.n_verts, W.lo.ptr, W.hi.ptr,
+                                                           W.bad.ptr);
+    CU(cudaMemcpyAsync(W.box_keys.ptr, W.box_init.ptr, 6 * sizeof(int), cudaMemcpyDeviceToDevice, s));
+    scene_box_kernel<<<std::min(1024, (A.n_tris + T - 1) / T), T, 0, s>>>(W.lo.ptr, W.hi.ptr, A.n_tris, W.box_keys.ptr);
+    CU(cudaMemcpyAsync(&W.host->bad, W.bad.ptr, sizeof(int), cudaMemcpyDeviceToHost, s));
+    root_kernel<<<(A.n_tris + T - 1) / T, T, 0, s>>>(W.box_keys.ptr, A.n_tris, A.max_depth, W.nodes[0].ptr,
+                                                     W.ref_tri[0].ptr, W.ref_node[0].ptr, W.level.ptr, W.bad.ptr);
 }
 
 size_t hist_words(size_t refs) { // nodes with histograms hold more than EXACT_MAX references
@@ -818,20 +803,22 @@ size_t hist_words(size_t refs) { // nodes with histograms hold more than EXACT_M
 // `nodes` size the launches (the true counts, or upper bounds -- the kernels read the true
 // counts from the level state).  The histograms must be zero on entry and are zero on exit.
 void enqueue_decide(const BuildArgs &A, int cur, size_t refs, size_t nodes, cudaStream_t s) {
-    const LevelState *ls = W.level;
+    const LevelState *ls = W.level.ptr;
+    const ANode *nodes_cur = W.nodes[cur].ptr;
+    const int *ref_tri = W.ref_tri[cur].ptr, *ref_node = W.ref_node[cur].ptr;
     if (refs > 0) {
-        bin_kernel<<<(unsigned)((refs + 255) / 256), 256, 0, s>>>(ls, W.nodes[cur], W.ref_tri[cur], W.ref_node[cur], W.lo,
-                                                                  W.hi, A.n_tris, A.min_split, W.hist);
+        bin_kernel<<<(unsigned)((refs + 255) / 256), 256, 0, s>>>(ls, nodes_cur, ref_tri, ref_node, W.lo.ptr, W.hi.ptr,
+                                                                  A.n_tris, A.min_split, W.hist.ptr);
     }
     // nodes of more than SMALL_MAX references: there are at most refs / SMALL_MAX of them
     const size_t big = std::min(nodes, refs / SMALL_MAX + 1);
     const int g32 = (int)std::max<size_t>(1, std::min<size_t>(CHOOSE_MAX_BLOCKS, (big * 32 + 255) / 256));
     const int g8 = (int)std::max<size_t>(1, std::min<size_t>(CHOOSE_MAX_BLOCKS, (nodes * 8 + 255) / 256));
-    choose_kernel<<<g32 + g8, 256, 0, s>>>(g32, ls, W.nodes[cur], W.hist, W.ref_tri[cur], W.lo, W.hi, A.n_tris,
-                                           A.min_split, A.ct, A.ci, A.empty_bonus, W.dec);
-    RefFlagFn rf{ W.nodes[cur], W.dec, W.ref_tri[cur], W.ref_node[cur], W.lo, W.hi, A.n_tris };
-    SplitFlagFn sf{ W.dec };
-    scan2(&ls->n_refs, refs, rf, W.ref_scan, &ls->n_nodes, nodes, sf, W.node_scan, W.totals, s);
+    choose_kernel<<<g32 + g8, 256, 0, s>>>(g32, ls, nodes_cur, W.hist.ptr, ref_tri, W.lo.ptr, W.hi.ptr, A.n_tris,
+                                           A.min_split, A.ct, A.ci, A.empty_bonus, W.dec.ptr);
+    RefFlagFn rf{ nodes_cur, W.dec.ptr, ref_tri, ref_node, W.lo.ptr, W.hi.ptr, A.n_tris };
+    SplitFlagFn sf{ W.dec.ptr };
+    scan2(&ls->n_refs, refs, rf, W.ref_scan.ptr, &ls->n_nodes, nodes, sf, W.node_scan.ptr, W.totals.ptr, s);
 }
 
 // The second half: wire nodes and the next level's nodes written, references moved to their
@@ -839,13 +826,15 @@ void enqueue_decide(const BuildArgs &A, int cur, size_t refs, size_t nodes, cuda
 void enqueue_split(const BuildArgs &A, int cur, size_t refs, size_t nodes, const Room &room, ClptGpuTree &out,
                    cudaStream_t s) {
     const int nxt = cur ^ 1;
-    SplitArgs sa = { W.nodes[cur], W.dec,        W.node_scan,   W.ref_scan,    W.totals,        W.ref_tri[cur],
-                     W.ref_node[cur], W.lo,      W.hi,          A.n_tris,      out.wire,        W.nodes[nxt],
-                     W.bad,        W.ref_tri[nxt], W.ref_node[nxt], out.tri_indices, room };
+    SplitArgs sa = { W.nodes[cur].ptr,    W.dec.ptr,          W.node_scan.ptr,     W.ref_scan.ptr,
+                     W.totals.ptr,        W.ref_tri[cur].ptr, W.ref_node[cur].ptr, W.lo.ptr,
+                     W.hi.ptr,            A.n_tris,           out.wire.ptr,        W.nodes[nxt].ptr,
+                     W.bad.ptr,           W.ref_tri[nxt].ptr, W.ref_node[nxt].ptr, out.tri_indices.ptr,
+                     room };
     const int emit_blocks = (int)std::max<size_t>(1, (nodes + T - 1) / T);
     const int scatter_blocks = (int)((refs + T - 1) / T);
-    split_kernel<<<emit_blocks + scatter_blocks, T, 0, s>>>(emit_blocks, W.level, sa);
-    commit_kernel<<<1, 32, 0, s>>>(W.level, W.totals, room, W.bad);
+    split_kernel<<<emit_blocks + scatter_blocks, T, 0, s>>>(emit_blocks, W.level.ptr, sa);
+    commit_kernel<<<1, 32, 0, s>>>(W.level.ptr, W.totals.ptr, room, W.bad.ptr);
 }
 
 // Meshes up to this size are built without the host in the loop (below).
@@ -866,25 +855,25 @@ bool build_recorded(const BuildArgs &A, int room_pc, ClptGpuTree &out, cudaStrea
         cap_out = std::max<size_t>(2, cap_out * pc / 100), cap_leaf = std::max<size_t>(2, cap_leaf * pc / 100);
     }
     for (int k = 0; k < 2; k++) {
-        ensure(W.ref_tri[k], W.ref_cap[k][0], cap_refs);
-        ensure(W.ref_node[k], W.ref_cap[k][1], cap_refs);
-        ensure(W.nodes[k], W.node_cap[k], cap_nodes);
+        W.ref_tri[k].reserve(cap_refs);
+        W.ref_node[k].reserve(cap_refs);
+        W.nodes[k].reserve(cap_nodes);
     }
-    ensure(W.dec, W.dec_cap, cap_nodes);
-    ensure(W.hist, W.hist_cap, hist_words(cap_refs));
-    ensure(W.ref_scan, W.ref_scan_cap, cap_refs + 1);
-    ensure(W.node_scan, W.node_scan_cap, cap_nodes + 1);
+    W.dec.reserve(cap_nodes);
+    W.hist.reserve(hist_words(cap_refs));
+    W.ref_scan.reserve(cap_refs + 1);
+    W.node_scan.reserve(cap_nodes + 1);
     // (the second term: what the re-layout of this tree will ask for)
-    ensure(W.tiles, W.tiles_cap, (size_t)std::max(scan_tiles(cap_refs) + scan_tiles(cap_nodes), scan_tiles(cap_out) + 1));
-    ensure(out.wire, out.wire_cap, cap_out * 17);
-    ensure(out.tri_indices, out.tri_indices_cap, cap_leaf);
-    const Workspace::GraphKey key = { A.verts, A.corners, out.wire, out.tri_indices, g_reallocations, cap_refs, A.n_verts, A.n_tris,
-                                      A.max_depth, A.min_split, A.ct, A.ci, A.empty_bonus };
+    W.tiles.reserve((size_t)std::max(scan_tiles(cap_refs) + scan_tiles(cap_nodes), scan_tiles(cap_out) + 1));
+    out.wire.reserve(cap_out * 17);
+    out.tri_indices.reserve(cap_leaf);
+    const Workspace::GraphKey key = { A.verts, A.corners, out.wire.ptr, out.tri_indices.ptr, clpt_devbuf_reallocations,
+                                      cap_refs, A.n_verts, A.n_tris, A.max_depth, A.min_split, A.ct, A.ci, A.empty_bonus };
     if (!W.graph || !(key == W.graph_key)) {
         drop_graph();
         cudaGraph_t g = nullptr;
         CU(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-        CU(cudaMemsetAsync(W.hist, 0, hist_words(cap_refs) * sizeof(unsigned), s)); // (each level leaves it zeroed)
+        CU(cudaMemsetAsync(W.hist.ptr, 0, hist_words(cap_refs) * sizeof(unsigned), s)); // (each level leaves it zeroed)
         enqueue_prologue(A, s);
         int cur = 0;
         for (int level = 0; level <= A.max_depth; level++) {
@@ -896,8 +885,8 @@ bool build_recorded(const BuildArgs &A, int room_pc, ClptGpuTree &out, cudaStrea
             enqueue_split(A, cur, refs, nodes, Room{ (int)nodes_next, (int)cap_refs, (int)cap_out, (int)cap_leaf }, out, s);
             cur ^= 1;
         }
-        push_ropes_kernel<<<(unsigned)((cap_out * 6 + T - 1) / T), T, 0, s>>>(out.wire, W.level);
-        CU(cudaMemcpyAsync(&W.host->level, W.level, sizeof(LevelState), cudaMemcpyDeviceToHost, s));
+        push_ropes_kernel<<<(unsigned)((cap_out * 6 + T - 1) / T), T, 0, s>>>(out.wire.ptr, W.level.ptr);
+        CU(cudaMemcpyAsync(&W.host->level, W.level.ptr, sizeof(LevelState), cudaMemcpyDeviceToHost, s));
         CU(cudaStreamEndCapture(s, &g));
         CU(cudaGraphInstantiate(&W.graph, g, 0));
         CU(cudaGraphDestroy(g));
@@ -934,14 +923,14 @@ bool clpt_gpu_build(const float4 *verts, int n_verts, const int4 *corners, int n
         A.max_depth = 8 + (13 * lg) / 10;
     }
     ensure_host();
-    ensure(W.lo, W.bounds_cap, (size_t)n_tris * 3);
-    ensure(W.hi, W.bounds_cap2, (size_t)n_tris * 3);
-    ensure(W.box_keys, W.box_cap, (size_t)8);
-    ensure(W.bad, W.bad_cap, (size_t)1);
-    if (!W.box_init) {
-        ensure(W.box_init, W.box_init_cap, (size_t)8);
+    W.lo.reserve((size_t)n_tris * 3);
+    W.hi.reserve((size_t)n_tris * 3);
+    W.box_keys.reserve(8);
+    W.bad.reserve(1);
+    if (!W.box_init.ptr) {
+        W.box_init.reserve(8);
         const int init_keys[6] = { INT_MAX, INT_MAX, INT_MAX, INT_MIN, INT_MIN, INT_MIN };
-        CU(cudaMemcpy(W.box_init, init_keys, sizeof(init_keys), cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(W.box_init.ptr, init_keys, sizeof(init_keys), cudaMemcpyHostToDevice));
     }
 
     const char *no_graph = getenv("CLPT_BUILD_NO_GRAPH"); // measurement and tests: always level by level
@@ -964,26 +953,26 @@ bool clpt_gpu_build(const float4 *verts, int n_verts, const int4 *corners, int n
     // Level by level with the host in the loop: two counters come back per level to size the
     // next level's buffers and launches exactly (any mesh size).
     int cur = 0;
-    ensure(W.ref_tri[0], W.ref_cap[0][0], (size_t)n_tris);
-    ensure(W.ref_node[0], W.ref_cap[0][1], (size_t)n_tris);
-    ensure(W.nodes[0], W.node_cap[0], (size_t)1);
+    W.ref_tri[0].reserve((size_t)n_tris);
+    W.ref_node[0].reserve((size_t)n_tris);
+    W.nodes[0].reserve(1);
     enqueue_prologue(A, s);
     size_t n_out = 1;       // wire nodes allocated so far (the root)
     size_t n_leaf_refs = 0; // tri_indices written so far
     size_t n_nodes = 1, n_refs = (size_t)n_tris;
-    ensure(out.wire, out.wire_cap, (size_t)17 * 1024);
+    out.wire.reserve((size_t)17 * 1024);
     int levels = 0;
     while (n_nodes > 0) {
         levels++;
-        ensure(W.dec, W.dec_cap, n_nodes);
-        ensure(W.hist, W.hist_cap, hist_words(n_refs));
-        ensure(W.ref_scan, W.ref_scan_cap, n_refs + 1);
-        ensure(W.node_scan, W.node_scan_cap, n_nodes + 1);
-        ensure(W.tiles, W.tiles_cap, (size_t)(scan_tiles(n_refs) + scan_tiles(n_nodes)));
+        W.dec.reserve(n_nodes);
+        W.hist.reserve(hist_words(n_refs));
+        W.ref_scan.reserve(n_refs + 1);
+        W.node_scan.reserve(n_nodes + 1);
+        W.tiles.reserve((size_t)(scan_tiles(n_refs) + scan_tiles(n_nodes)));
         // (the buffer may just have moved; otherwise the previous level left it zeroed and this is redundant)
-        CU(cudaMemsetAsync(W.hist, 0, hist_words(n_refs) * sizeof(unsigned), s));
+        CU(cudaMemsetAsync(W.hist.ptr, 0, hist_words(n_refs) * sizeof(unsigned), s));
         enqueue_decide(A, cur, n_refs, n_nodes, s);
-        CU(cudaMemcpyAsync(W.host->totals, W.totals, 2 * sizeof(Triple), cudaMemcpyDeviceToHost, s));
+        CU(cudaMemcpyAsync(W.host->totals, W.totals.ptr, 2 * sizeof(Triple), cudaMemcpyDeviceToHost, s));
         CU(cudaStreamSynchronize(s));
         if (levels == 1 && W.host->bad) {
             snprintf(err, errlen, "triangle corner references a missing vertex");
@@ -995,33 +984,12 @@ bool clpt_gpu_build(const float4 *verts, int n_verts, const int4 *corners, int n
             snprintf(err, errlen, "tree too large (%zu references, %zu nodes)", next_refs, n_out + next_nodes);
             return false;
         }
-        // grow the outputs, keeping what is there
-        if ((n_out + next_nodes) * 17 > out.wire_cap) {
-            int *bigger = nullptr;
-            const size_t cap = (n_out + next_nodes) * 17 * 2;
-            CU(cudaMalloc((void **)&bigger, cap * sizeof(int)));
-            CU(cudaMemcpyAsync(bigger, out.wire, n_out * 17 * sizeof(int), cudaMemcpyDeviceToDevice, s));
-            CU(cudaStreamSynchronize(s));
-            CU(cudaFree(out.wire));
-            out.wire = bigger;
-            out.wire_cap = cap;
-        }
-        if (n_leaf_refs + rt.f > out.tri_indices_cap) {
-            int *bigger = nullptr;
-            const size_t cap = (n_leaf_refs + rt.f) * 2 + (size_t)n_tris;
-            CU(cudaMalloc((void **)&bigger, cap * sizeof(int)));
-            if (out.tri_indices) {
-                CU(cudaMemcpyAsync(bigger, out.tri_indices, n_leaf_refs * sizeof(int), cudaMemcpyDeviceToDevice, s));
-                CU(cudaStreamSynchronize(s));
-                CU(cudaFree(out.tri_indices));
-            }
-            out.tri_indices = bigger;
-            out.tri_indices_cap = cap;
-        }
+        out.wire.grow_keep((n_out + next_nodes) * 17, n_out * 17, s);
+        out.tri_indices.grow_keep(n_leaf_refs + rt.f, n_leaf_refs, s);
         const int nxt = cur ^ 1;
-        ensure(W.ref_tri[nxt], W.ref_cap[nxt][0], next_refs);
-        ensure(W.ref_node[nxt], W.ref_cap[nxt][1], next_refs);
-        ensure(W.nodes[nxt], W.node_cap[nxt], next_nodes);
+        W.ref_tri[nxt].reserve(next_refs);
+        W.ref_node[nxt].reserve(next_refs);
+        W.nodes[nxt].reserve(next_nodes);
         enqueue_split(A, cur, n_refs, n_nodes, Room{ INT_MAX, INT_MAX, INT_MAX, INT_MAX }, out, s);
         n_out += next_nodes;
         n_leaf_refs += rt.f;
@@ -1029,7 +997,7 @@ bool clpt_gpu_build(const float4 *verts, int n_verts, const int4 *corners, int n
         n_refs = next_refs;
         cur = nxt;
     }
-    push_ropes_kernel<<<(unsigned)((n_out * 6 + T - 1) / T), T, 0, s>>>(out.wire, W.level);
+    push_ropes_kernel<<<(unsigned)((n_out * 6 + T - 1) / T), T, 0, s>>>(out.wire.ptr, W.level.ptr);
     CU(cudaGetLastError());
     out.n_nodes = (int)n_out;
     out.n_refs = (int)n_leaf_refs;
@@ -1174,14 +1142,9 @@ __global__ void pack_lut_kernel(const int *__restrict__ wire, const int *__restr
     lut[cell] = new_of[o];
 }
 
-int *g_new_of = nullptr;
-size_t g_new_of_cap = 0;
-Triple *g_wire_scan = nullptr;
-size_t g_wire_scan_cap = 0;
-
 } // namespace
 
-bool clpt_gpu_pack(const ClptGpuTree &tree, const float4 *verts, const int4 *corners, int n_prims, ClptGpuPacked &out,
+bool clpt_gpu_pack(const ClptGpuTree &tree, const float4 *verts, const int4 *corners, int n_prims, ClptSceneLayout &out,
                    cudaStream_t s, char *err, size_t errlen) {
     const int n = tree.n_nodes;
     if (n <= 0) {
@@ -1189,38 +1152,41 @@ bool clpt_gpu_pack(const ClptGpuTree &tree, const float4 *verts, const int4 *cor
         return false;
     }
     ensure_host();
-    ensure(g_new_of, g_new_of_cap, (size_t)n);
-    ensure(g_wire_scan, g_wire_scan_cap, (size_t)n + 2);
-    ensure(W.tiles, W.tiles_cap, (size_t)scan_tiles((size_t)n) + 1);
+    W.new_of.reserve((size_t)n);
+    W.wire_scan.reserve((size_t)n + 2);
+    W.tiles.reserve((size_t)scan_tiles((size_t)n) + 1);
     W.host->n = n;
-    int *n_dev = &W.level[1].n_nodes;
+    int *n_dev = &W.level.ptr[1].n_nodes;
     CU(cudaMemcpyAsync(n_dev, &W.host->n, sizeof(int), cudaMemcpyHostToDevice, s));
-    WireTypeFn tf{ tree.wire };
-    int *zero_dev = &W.level[1].n_refs; // (an empty second sequence)
+    WireTypeFn tf{ tree.wire.ptr };
+    int *zero_dev = &W.level.ptr[1].n_refs; // (an empty second sequence)
     CU(cudaMemsetAsync(zero_dev, 0, sizeof(int), s));
-    scan2(n_dev, (size_t)n, tf, g_wire_scan, zero_dev, 0, NoItemsFn{}, g_wire_scan /* one word past the first */ + n + 1,
-          W.totals, s);
-    CU(cudaMemcpyAsync(W.host->totals, W.totals, sizeof(Triple), cudaMemcpyDeviceToHost, s));
+    Triple *scan = W.wire_scan.ptr;
+    scan2(n_dev, (size_t)n, tf, scan, zero_dev, 0, NoItemsFn{}, scan /* one word past the first */ + n + 1, W.totals.ptr, s);
+    CU(cudaMemcpyAsync(W.host->totals, W.totals.ptr, sizeof(Triple), cudaMemcpyDeviceToHost, s));
     float box[8];
-    CU(cudaMemcpyAsync(box, tree.wire, sizeof(box), cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(box, tree.wire.ptr, sizeof(box), cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
     const int n_splits = (int)W.host->totals[0].l, n_leaves = (int)W.host->totals[0].f;
     out.fat_refs = W.host->totals[0].r;
     out.n_nodes = 1 + 2 * n_splits;
     out.n_leaves = n_leaves;
     out.n_refs = tree.n_refs;
-    ensure(out.nodes, out.nodes_cap, (size_t)out.n_nodes);
-    ensure(out.leaves, out.leaves_cap, (size_t)n_leaves * 4);
-    ensure(out.tri, out.tri_cap, (size_t)std::max(tree.n_refs, 1) * 3);
-    renumber_kernel<<<(n + T - 1) / T, T, 0, s>>>(tree.wire, n, g_wire_scan, g_new_of);
-    pack_nodes_kernel<<<(n + T - 1) / T, T, 0, s>>>(tree.wire, n, g_wire_scan, g_new_of, out.nodes, out.leaves);
+    out.nodes.reserve((size_t)out.n_nodes);
+    out.leaves.reserve((size_t)n_leaves * 4);
+    out.tri.reserve((size_t)std::max(tree.n_refs, 1) * 3);
+    const int *wire = tree.wire.ptr;
+    int *new_of = W.new_of.ptr;
+    renumber_kernel<<<(n + T - 1) / T, T, 0, s>>>(wire, n, scan, new_of);
+    pack_nodes_kernel<<<(n + T - 1) / T, T, 0, s>>>(wire, n, scan, new_of, out.nodes.ptr, out.leaves.ptr);
     if (tree.n_refs > 0) {
-        pack_tris_kernel<<<(tree.n_refs + T - 1) / T, T, 0, s>>>(tree.tri_indices, tree.n_refs, corners, verts, out.tri);
+        pack_tris_kernel<<<(tree.n_refs + T - 1) / T, T, 0, s>>>(tree.tri_indices.ptr, tree.n_refs, corners, verts,
+                                                                 out.tri.ptr);
     }
-    ensure(out.flat_n, out.flat_n_cap, (size_t)std::max(n_prims, 1));
+    out.flat_n.reserve((size_t)std::max(n_prims, 1));
     if (n_prims > 0) {
         // (the builder has checked every corner's vertex index, tri_bounds_kernel)
-        pack_flat_normals_kernel<<<(n_prims + T - 1) / T, T, 0, s>>>(corners, verts, n_prims, out.flat_n);
+        pack_flat_normals_kernel<<<(n_prims + T - 1) / T, T, 0, s>>>(corners, verts, n_prims, out.flat_n.ptr);
     }
     // start-node table geometry: the host packer's arithmetic (scene_pack.cpp), so that both give the same table
     LutGrid G;
@@ -1245,8 +1211,8 @@ bool clpt_gpu_pack(const ClptGpuTree &tree, const float4 *verts, const int4 *cor
         G.scale[a] = (double)out.lut_scale[a];
         total *= (size_t)d;
     }
-    ensure(out.lut, out.lut_cap, total);
-    pack_lut_kernel<<<(unsigned)((total + T - 1) / T), T, 0, s>>>(tree.wire, g_new_of, G, out.lut);
+    out.lut.reserve(total);
+    pack_lut_kernel<<<(unsigned)((total + T - 1) / T), T, 0, s>>>(wire, new_of, G, out.lut.ptr);
     CU(cudaGetLastError());
     return true;
 }
@@ -1254,15 +1220,11 @@ bool clpt_gpu_pack(const ClptGpuTree &tree, const float4 *verts, const int4 *cor
 bool clpt_gpu_build_was_recorded(void) { return g_last_build_recorded; }
 
 void clpt_gpu_build_release(void) {
-    auto drop = [](auto *&p) {
-        if (p) (void)cudaFree(p);
-        p = nullptr;
-    };
-    drop(W.lo), drop(W.hi), drop(W.ref_tri[0]), drop(W.ref_tri[1]), drop(W.ref_node[0]), drop(W.ref_node[1]);
-    drop(W.nodes[0]), drop(W.nodes[1]), drop(W.dec), drop(W.hist), drop(W.ref_scan), drop(W.node_scan);
-    drop(W.tiles), drop(W.totals), drop(W.box_keys), drop(W.bad), drop(W.box_init), drop(W.level);
-    drop(g_new_of), drop(g_wire_scan);
-    g_new_of_cap = g_wire_scan_cap = 0;
+    W.lo.release(), W.hi.release(), W.dec.release(), W.hist.release();
+    for (int k = 0; k < 2; k++) W.ref_tri[k].release(), W.ref_node[k].release(), W.nodes[k].release();
+    W.ref_scan.release(), W.node_scan.release(), W.tiles.release(), W.totals.release();
+    W.box_keys.release(), W.bad.release(), W.box_init.release(), W.level.release();
+    W.new_of.release(), W.wire_scan.release();
     if (W.host) (void)cudaFreeHost(W.host);
     drop_graph();
     W = Workspace();

@@ -164,7 +164,8 @@ bool clpt_pack_scene(const kdnode *nodes, size_t n_nodes, const int *tri_indices
     out.leaves.resize((size_t)n_leaves * 4);
     long long bad_node = -1;
     int bad_kind = 0;
-#pragma omp parallel for schedule(static)
+    size_t fat_refs = 0;
+#pragma omp parallel for schedule(static) reduction(+ : fat_refs)
     for (long long i = 0; i < (long long)n_nodes; i++) {
         const int ni = new_of[i];
         if (ni < 0) continue; // unreachable from the root
@@ -179,6 +180,7 @@ bool clpt_pack_scene(const kdnode *nodes, size_t n_nodes, const int *tri_indices
         out.nodes[ni].y = 0x80000003u; // CLPT_LEAF_WORD
         const int first = k.leaf.tris, count = k.leaf.tri_count;
         bool bad = count < 0 || (count > 0 && (first < 0 || (size_t)first + (size_t)count > n_refs));
+        if (count >= CLPT_COOP_LEAF_MIN) fat_refs += (size_t)count;
         ClptFloat4 *L = &out.leaves[(size_t)li * 4];
         L[0] = ClptFloat4{ k.min.s[0], k.min.s[1], k.min.s[2], as_float(count > 0 ? first : 0) };
         L[1] = ClptFloat4{ k.max.s[0], k.max.s[1], k.max.s[2], as_float(count) };
@@ -366,6 +368,7 @@ bool clpt_pack_scene(const kdnode *nodes, size_t n_nodes, const int *tri_indices
     out.n_leaves = n_leaves;
     out.n_refs = (int)n_refs;
     out.n_prims = (int)n_prims;
+    out.fat_refs = fat_refs;
     (void)as_int;
     return true;
 }

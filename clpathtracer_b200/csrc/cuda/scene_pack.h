@@ -57,16 +57,28 @@ class ClptStaging {
     size_t size_ = 0, cap_ = 0;
 };
 
-struct ClptPackedScene {
+// A "fat" leaf for the automatic engine choice: trees whose triangle slots mostly live in
+// leaves of at least this many triangles are rendered by engine 2.
+#define CLPT_COOP_LEAF_MIN 8
+#define CLPT_FAT_ENGINE_MIN_REFS 500000
+
+// What a re-layout computes besides its arrays.  Both re-layouts fill it: clpt_pack_scene
+// here and its device twin clpt_gpu_pack (kd_build_gpu.h).
+struct ClptLayoutInfo {
+    int n_nodes = 0, n_leaves = 0, n_refs = 0;
+    float root_min[3] = {}, root_max[3] = {};
+    int lut_dim[3] = { 1, 1, 1 };
+    float lut_scale[3] = { 0, 0, 0 };
+    size_t fat_refs = 0; // triangle slots living in leaves of >= CLPT_COOP_LEAF_MIN triangles
+};
+
+struct ClptPackedScene : ClptLayoutInfo {
     ClptStaging<ClptNode8> nodes;
     ClptStaging<ClptFloat4> leaves; // 4 per leaf
     ClptStaging<ClptFloat4> tri;    // 3 per leaf triangle slot
     ClptStaging<ClptFloat4> flat_n; // 1 per primitive: flat normal, w = 1 if the primitive uses vertex normals
-    float root_min[3], root_max[3];
-    int n_nodes = 0, n_leaves = 0, n_refs = 0, n_prims = 0;
-    ClptStaging<int> lut; // start-node table, lut_dim[0] fastest
-    int lut_dim[3] = { 1, 1, 1 };
-    float lut_scale[3] = { 0, 0, 0 };
+    ClptStaging<int> lut;           // start-node table, lut_dim[0] fastest
+    int n_prims = 0;
 };
 
 // Returns false and fills `err` when the input is inconsistent (index out of

@@ -199,6 +199,68 @@ def test_device_build_quality_and_speed(clpt, renderer):
     print("device build", build_ms, "ms, re-layout", pack_ms, "ms", dev, "host", host)
 
 
+def test_host_and_device_layouts_take_turns(clpt, oracle, renderer, scene_cache, monkeypatch):
+    """CLSetMeshes (host re-layout) and CLBuildMeshes / CLRebuildMeshes (device re-layout) write the
+    same device buffers.  Taking turns in one renderer, a smaller scene after a bigger one, every
+    frame is the oracle's walk of that step's tree and the layout has that tree's sizes; the
+    automatic engine is the same whichever path laid out the same tree."""
+    w, h = 160, 120
+    renderer.set_params(mode=1, depth=2, spp=1, seed=5, flags=0)
+    renderer.create_image(w, h, aov=True)
+
+    def check(scene, camera):
+        cam = _cam(clpt, camera, h)
+        renderer.set_camera_matrix(cam)
+        renderer.execute()
+        img = renderer.read_image()
+        prim, _, _ = renderer.read_aov()
+        ref = oracle.render(scene, cam, w, h, mode=1, depth=2, seed=5)
+        assert np.array_equal(prim, ref["prim"])
+        assert np.array_equal(img.view(np.uint32), ref["rgba"].view(np.uint32))
+        assert (prim >= 0).mean() > 0.01
+        split = int((scene.nodes["type"] == 0).sum())
+        n_nodes, n_leaves = 1 + 2 * split, len(scene.nodes) - split
+        sizes = [renderer.read_packed(k).size for k in (0, 1, 2, 4)]
+        assert sizes == [8 * n_nodes, 64 * n_leaves, 48 * len(scene.tri_indices), 16 * scene.n_tris]
+        lut = renderer.read_packed(3).view(np.int32)
+        assert lut.size > 0 and lut.min() >= 0 and lut.max() < n_nodes
+
+    def device(name):
+        renderer.build_meshes(*_mesh(name))
+        return renderer.download_kd()
+
+    host_big = scene_cache("hf224", sah=True)[0]
+    renderer.set_meshes(host_big)
+    check(host_big, "canonical")
+    check(device("soup3000"), "cornell")
+    host_small = scene_cache("hf22n")[0]
+    assert len(host_small.nodes) < len(host_big.nodes)
+    renderer.set_meshes(host_small)
+    check(host_small, "canonical")
+    check(device("hf60"), "canonical")
+    renderer.rebuild_meshes()
+    check(renderer.download_kd(), "canonical")
+
+    # engine policy: a shallow device tree of more than CLPT_FAT_ENGINE_MIN_REFS (500,000) triangle
+    # slots in fat leaves, then the same tree through the host path
+    from clpathtracer_b200 import scenes
+
+    monkeypatch.delenv("CLPT_ENGINE", raising=False)
+    L = clpt.lib()
+    L.CLSetEngine(0)
+    renderer.set_camera_matrix(_cam(clpt, "canonical", h))
+    L.CLSetBuildParams(12, 2, 1.0, 1.0, 0.9)
+    try:
+        renderer.build_meshes(*scenes.heightfield(520, False))  # 540,800 triangles
+    finally:
+        L.CLSetBuildParams(0, 2, 1.0, 1.0, 0.9)  # the defaults (kd_build_gpu.h)
+    renderer.execute()
+    assert L.CLLastEngine() == 2
+    renderer.set_meshes(renderer.download_kd())
+    renderer.execute()
+    assert L.CLLastEngine() == 2
+
+
 def test_device_build_rejects_bad_mesh(clpt):
     import subprocess
     import sys
