@@ -71,6 +71,24 @@ class CLMaterial(C.Structure):
                 ("pad", C.c_float)]
 
 
+MAX_INSTANCES = 64
+
+
+class CLInstance(C.Structure):
+    """One rigid instance (CLState.h): world_to_object is the row-major 3x4 [A | b]."""
+    _fields_ = [("world_to_object", C.c_float * 12), ("mesh", C.c_int), ("material", C.c_int),
+                ("pad", C.c_int * 2)]
+
+
+def world_to_object(object_to_world) -> np.ndarray:
+    """float32[3,4] [A | b] of the inverse of a 3x4 or 4x4 affine object-to-world matrix,
+    inverted in float64."""
+    m = np.asarray(object_to_world, dtype=np.float64)
+    full = np.eye(4)
+    full[:3, :] = m[:3, :4]
+    return np.linalg.inv(full)[:3, :].astype(np.float32)
+
+
 _lib = None
 
 
@@ -113,6 +131,8 @@ def lib() -> C.CDLL:
         "CLLastBuildMs": (None, [C.POINTER(f), C.POINTER(f)]), "CLBuildStats": (None, [C.POINTER(i), C.POINTER(i), C.POINTER(i)]),
         "CLLastBuildWasRecorded": (i, []),
         "CLDownloadKd": (None, [C.POINTER(KD)]), "CLDebugReadPacked": (sz, [i, vp, sz]),
+        "CLAddInstanceMesh": (i, [vp, sz, vp, sz, vp, sz]), "CLSetInstances": (None, [vp, sz]),
+        "CLClearInstanceMeshes": (None, []), "CLDownloadInstanceKd": (None, [i, C.POINTER(KD)]),
         "CLUpdateVertices": (None, [sz, vp, sz]), "CLRebuildMeshes": (None, []),
         "CLDeleteImage": (None, []), "CLCreateImage": (None, [u]), "CLExecute": (None, [i, i]),
         "CLSelectDevice": (None, [i]), "CLSetRenderParams": (None, [i, i, i, u, i]),
@@ -333,6 +353,33 @@ class Renderer:
         """The device-built tree as a Scene (wire format) for the oracle."""
         k = KD()
         self.L.CLDownloadKd(C.byref(k))
+        return Scene.from_kd(k)
+
+    def add_instance_mesh(self, verts: np.ndarray, corners: np.ndarray, norms: np.ndarray | None = None) -> int:
+        """Upload a mesh and build its tree on the device once (CLAddInstanceMesh); returns its handle."""
+        v4 = _as_vec4(verts)
+        c4 = np.ascontiguousarray(corners, dtype=np.int32).reshape(-1, 4)
+        n4 = _as_vec4(norms) if norms is not None and len(norms) else None
+        return int(self.L.CLAddInstanceMesh(v4.ctypes.data, v4.nbytes, c4.ctypes.data, c4.nbytes,
+                                            None if n4 is None else n4.ctypes.data, 0 if n4 is None else n4.nbytes))
+
+    def set_instances(self, instances) -> None:
+        """The instances of the next frames: [(mesh handle, object_to_world 3x4 or 4x4, material), ...]
+        (material only matters in mode 2).  The matrices are inverted here, in float64; an empty
+        list removes every instance."""
+        table = (CLInstance * len(instances))()
+        for k, (mesh, o2w, material) in enumerate(instances):
+            table[k].world_to_object[:] = [float(x) for x in world_to_object(o2w).reshape(12)]
+            table[k].mesh, table[k].material = int(mesh), int(material)
+        self.L.CLSetInstances(C.addressof(table) if instances else None, C.sizeof(table))
+
+    def clear_instance_meshes(self) -> None:
+        self.L.CLClearInstanceMeshes()
+
+    def download_instance_kd(self, mesh: int) -> "Scene":
+        """An instance mesh's device-built tree as a Scene (wire format) for the oracle."""
+        k = KD()
+        self.L.CLDownloadInstanceKd(int(mesh), C.byref(k))
         return Scene.from_kd(k)
 
     def build_ms(self) -> tuple[float, float]:

@@ -101,6 +101,9 @@ def build_oracle() -> None:
     reference tree is present).  Building the checker is not using it."""
     _run(["make", "-s", "-C", str(ROOT / "oracle"), "oracle"])
     _run(["make", "-s", "-C", str(ROOT / "oracle"), "ref"])
+    # the rigid-instance restatement (oracle/oracle_instances_py.py builds it the same way when missing)
+    _run(["gcc", "-std=c11", "-O2", "-fPIC", "-ffp-contract=off", "-fopenmp", "-w", "-shared", "-o",
+          str(ROOT / "oracle" / "liboracle_instances.so"), str(ROOT / "oracle" / "oracle_instances.c"), "-lm"])
 
 
 if __name__ == "__main__":

@@ -61,6 +61,22 @@ struct ClptScene {
     float lut_scale[3]; // cells per unit length
 };
 
+// Rigid instances (CLSetInstances): a mesh with its own tree, walked with the world ray
+// mapped into object space.  One record per instance, rewritten by clstate.cu whenever the
+// instances or the base scene change.
+struct ClptInstanceRec {
+    float w2o[12];   // world to object, row-major 3x4 [A | b]
+    int material;    // mode 2: the material of every triangle of the instance
+    int prim_offset; // base scene's primitives + those of the instances before this one
+    int pad[2];
+    ClptScene mesh;  // the instance mesh's traversal layout (materials unused)
+};
+
+struct ClptInstances {
+    const ClptInstanceRec *rec; // device table of `count` records
+    int count;
+};
+
 #define CLPT_MAX_PEERS 8
 
 struct ClptFrame {
@@ -126,7 +142,9 @@ enum { CLPT_F_JITTER = 1, CLPT_F_ACCUMULATE = 2, CLPT_F_COUNTERS = 4, CLPT_F_REV
        CLPT_F_FAT = 0x200 /* internal: engine 2, the kernel compiled for fewer resident blocks (fat leaves) */ };
 
 // render_kernel.cu
-void clpt_launch_render(const ClptScene &scene, const ClptFrame &frame, int sm_count, cudaStream_t stream);
+// inst.count > 0 launches the instanced variant of the render kernel
+void clpt_launch_render(const ClptScene &scene, const ClptFrame &frame, const ClptInstances &inst, int sm_count,
+                        cudaStream_t stream);
 int clpt_render_blocks_per_sm(int engine);          // resident 256-thread blocks per SM the render kernel is compiled for
 int clpt_render_block_rows(const ClptFrame &frame); // rows of blocks the launch will walk (size of row_cost)
 void clpt_launch_deinterleave(const float4 *gathered, float4 *image, int width, int height,

@@ -72,6 +72,7 @@ __device__ __forceinline__ V3 xyz(float4 a) { return mk(a.x, a.y, a.z); }
 struct Hit {
     int ref; // triangle slot of the accepted hit, -1 = none
     float t;
+    int inst; // instanced kernel only: the instance hit (ref is a slot of its mesh), -1 = the base scene
 };
 
 struct HitDetails {
@@ -300,20 +301,18 @@ __device__ __forceinline__ bool leave_leaf(const uint2 *__restrict__ nodes, cons
     return false;
 }
 
-// Traversal of one ray to completion.  SHARE: 1 << log2_k neighbouring lanes walk this same ray
-// and split the triangle runs (lane `sub` of them; only sub 0 counts the per-ray work).
-template <bool COUNT, bool SHARE = false>
-__device__ __forceinline__ Hit closest_hit(const ClptScene &S, V3 o, V3 d, int max_visits, Counters &cn_in,
-                                           int sub = 0, int log2_k = 0) {
+// The walk of one ray through one tree, from its root-clip entry tmin to completion.  SHARE:
+// 1 << log2_k neighbouring lanes walk this same ray and split the triangle runs (lane `sub` of
+// them; only sub 0 counts the per-ray work).
+template <bool COUNT, bool SHARE>
+__device__ __forceinline__ Hit walk(const ClptScene &S, V3 o, V3 d, V3 inv, float tmin, int max_visits,
+                                    Counters &cn_in, int sub, int log2_k) {
     Hit h;
     h.ref = -1;
     h.t = 0.0f;
     Counters scratch = { 0, 0, 0, 0, 0, 0 };
     Counters &cn = (SHARE && sub != 0) ? scratch : cn_in; // (the helpers' visits are not the algorithm's)
-    if (COUNT) cn.rays++;
-    const V3 inv = mk(frcp(d.x), frcp(d.y), frcp(d.z));
-    float tmin, tmax;
-    if (!root_clip(S, o, inv, tmin, tmax)) return h;
+    float tmax;
     V3 p1 = o;
     if (tmin > 0.0f) p1 = vadd(p1, vscale(d, tmin));
 
@@ -350,6 +349,63 @@ __device__ __forceinline__ Hit closest_hit(const ClptScene &S, V3 o, V3 d, int m
     return h;
 }
 
+// Closest hit of one ray in one tree (one "ray" of the counters).
+template <bool COUNT, bool SHARE = false>
+__device__ __forceinline__ Hit closest_hit(const ClptScene &S, V3 o, V3 d, int max_visits, Counters &cn_in,
+                                           int sub = 0, int log2_k = 0) {
+    Hit h;
+    h.ref = -1;
+    h.t = 0.0f;
+    Counters scratch = { 0, 0, 0, 0, 0, 0 };
+    Counters &cn = (SHARE && sub != 0) ? scratch : cn_in;
+    if (COUNT) cn.rays++;
+    const V3 inv = mk(frcp(d.x), frcp(d.y), frcp(d.z));
+    float tmin, tmax;
+    if (!root_clip(S, o, inv, tmin, tmax)) return h;
+    return walk<COUNT, SHARE>(S, o, d, inv, tmin, max_visits, cn_in, sub, log2_k);
+}
+
+// ---- rigid instances (DESIGN.md "Rigid instances") ---------------------------------------------
+// The world ray in an instance's object space: row r of [A | b] applied left to right, un-contracted
+// (the form of unproject).  d' is not normalised, so t along (o', d') is the world ray's t.
+__device__ __forceinline__ void object_ray(const float *m, V3 o, V3 d, V3 &lo, V3 &ld) {
+    lo = mk(fadd(fadd(fadd(fmul(m[0], o.x), fmul(m[1], o.y)), fmul(m[2], o.z)), m[3]),
+            fadd(fadd(fadd(fmul(m[4], o.x), fmul(m[5], o.y)), fmul(m[6], o.z)), m[7]),
+            fadd(fadd(fadd(fmul(m[8], o.x), fmul(m[9], o.y)), fmul(m[10], o.z)), m[11]));
+    ld = mk(fadd(fadd(fmul(m[0], d.x), fmul(m[1], d.y)), fmul(m[2], d.z)),
+            fadd(fadd(fmul(m[4], d.x), fmul(m[5], d.y)), fmul(m[6], d.z)),
+            fadd(fadd(fmul(m[8], d.x), fmul(m[9], d.y)), fmul(m[10], d.z)));
+}
+
+// Closest hit in the base scene and then in every instance, in array order.  An instance is
+// skipped when a hit exists and the ray enters the instance's root box beyond it; a later tree's
+// hit replaces the current one at t <= best (the later tree wins ties, like the later triangle at
+// kernel.cl:344).  INST = false is closest_hit itself.
+template <bool COUNT, bool SHARE, bool INST>
+__device__ __forceinline__ Hit scene_hit(const ClptScene &S, const ClptInstances &I, V3 o, V3 d, int max_visits,
+                                         Counters &cn, int sub, int log2_k) {
+    Hit h = closest_hit<COUNT, SHARE>(S, o, d, max_visits, cn, sub, log2_k);
+    if (INST) {
+        h.inst = -1;
+        for (int k = 0; k < I.count; k++) {
+            const ClptInstanceRec &R = I.rec[k];
+            V3 lo, ld;
+            object_ray(R.w2o, o, d, lo, ld);
+            const V3 inv = mk(frcp(ld.x), frcp(ld.y), frcp(ld.z));
+            float tmin, tmax;
+            if (!root_clip(R.mesh, lo, inv, tmin, tmax)) continue;
+            if (h.ref >= 0 && tmin > h.t) continue;
+            const Hit hi = walk<COUNT, SHARE>(R.mesh, lo, ld, inv, tmin, max_visits, cn, sub, log2_k);
+            if (hi.ref >= 0 && (h.ref < 0 || hi.t <= h.t)) {
+                h.ref = hi.ref;
+                h.t = hi.t;
+                h.inst = k;
+            }
+        }
+    }
+    return h;
+}
+
 // Primitive id and barycentrics of the accepted hit: hit_triangle's u and v
 // (kernel.cl:243-249) evaluated again for the winning slot.
 __device__ __forceinline__ HitDetails hit_details(const ClptScene &S, const Hit &h, V3 o, V3 d) {
@@ -370,31 +426,68 @@ __device__ __forceinline__ HitDetails hit_details(const ClptScene &S, const Hit 
 // primitive and comes from ClptScene::flat_n (one 16-byte load instead of two, a cross product, a
 // square root and three IEEE divisions at every hit); its w says whether the primitive is shaded
 // with interpolated vertex normals instead.
+// The vertex normals of primitive `prim` interpolated at the hit, before normalisation.
+template <bool COUNT>
+__device__ __forceinline__ V3 vertex_normal_sum(const ClptScene &S, const Hit &h, int prim, V3 o, V3 d, Counters &cn) {
+    const int4 c1 = __ldg(S.corners + 3 * (size_t)prim);
+    const HitDetails hd = hit_details(S, h, o, d);
+    const int4 c2 = __ldg(S.corners + 3 * (size_t)prim + 1);
+    const int4 c3 = __ldg(S.corners + 3 * (size_t)prim + 2);
+    const V3 n1 = xyz(__ldg(S.norms + c1.y)), n2 = xyz(__ldg(S.norms + c2.y)), n3 = xyz(__ldg(S.norms + c3.y));
+    const float w = fsub(fsub(1.0f, hd.u), hd.v);
+    if (COUNT) cn.shade_vn++;
+    return vadd(vadd(vscale(n1, w), vscale(n2, hd.u)), vscale(n3, hd.v));
+}
+
 template <bool COUNT>
 __device__ __forceinline__ V3 hit_normal(const ClptScene &S, const Hit &h, V3 o, V3 d, Counters &cn) {
     const int prim = __float_as_int(__ldg(&S.tri[3 * (size_t)h.ref].w));
     const float4 fn = __ldg(S.flat_n + prim);
-    if (fn.w != 0.0f) {
-        const int4 c1 = __ldg(S.corners + 3 * (size_t)prim);
-        const HitDetails hd = hit_details(S, h, o, d);
-        const int4 c2 = __ldg(S.corners + 3 * (size_t)prim + 1);
-        const int4 c3 = __ldg(S.corners + 3 * (size_t)prim + 2);
-        const V3 n1 = xyz(__ldg(S.norms + c1.y)), n2 = xyz(__ldg(S.norms + c2.y)),
-                 n3 = xyz(__ldg(S.norms + c3.y));
-        const float w = fsub(fsub(1.0f, hd.u), hd.v);
-        if (COUNT) cn.shade_vn++;
-        return vnormalize(vadd(vadd(vscale(n1, w), vscale(n2, hd.u)), vscale(n3, hd.v)));
-    }
+    if (fn.w != 0.0f) return vnormalize(vertex_normal_sum<COUNT>(S, h, prim, o, d, cn));
     return xyz(fn);
+}
+
+// Shading normal of an instance hit, (o', d') the object-space ray: the object-space normal BEFORE
+// normalisation -- the flat normal's cross product (e1 x e2 of the triangle slot, the operands of
+// ClptScene::flat_n) or the interpolated vertex normals -- mapped to world space by A^T, then
+// normalised once.  (Normalising in object space too would make an identity instance shade
+// differently from its own mesh: normalize is not idempotent in fp32, about a third of unit
+// vectors move by an ulp when normalised again.)
+template <bool COUNT>
+__device__ __forceinline__ V3 instance_normal(const ClptInstanceRec &R, const Hit &h, V3 lo, V3 ld, Counters &cn) {
+    const ClptScene &S = R.mesh;
+    const int prim = __float_as_int(__ldg(&S.tri[3 * (size_t)h.ref].w));
+    V3 m;
+    if (__ldg(&S.flat_n[prim].w) != 0.0f) {
+        m = vertex_normal_sum<COUNT>(S, h, prim, lo, ld, cn);
+    } else {
+        m = vcross(xyz(__ldg(S.tri + 3 * (size_t)h.ref + 1)), xyz(__ldg(S.tri + 3 * (size_t)h.ref + 2)));
+    }
+    const float *a = R.w2o;
+    return vnormalize(mk(fadd(fadd(fmul(a[0], m.x), fmul(a[4], m.y)), fmul(a[8], m.z)),
+                         fadd(fadd(fmul(a[1], m.x), fmul(a[5], m.y)), fmul(a[9], m.z)),
+                         fadd(fadd(fmul(a[2], m.x), fmul(a[6], m.y)), fmul(a[10], m.z))));
+}
+
+template <bool COUNT, bool INST>
+__device__ __forceinline__ V3 shading_normal(const ClptScene &S, const ClptInstances &I, const Hit &h, V3 o, V3 d,
+                                             Counters &cn) {
+    if (INST && h.inst >= 0) {
+        const ClptInstanceRec &R = I.rec[h.inst];
+        V3 lo, ld;
+        object_ray(R.w2o, o, d, lo, ld);
+        return instance_normal<COUNT>(R, h, lo, ld, cn);
+    }
+    return hit_normal<COUNT>(S, h, o, d, cn);
 }
 
 template <bool COUNT>
 __device__ __forceinline__ void write_aov(const ClptScene &S, const ClptFrame &F, const Hit &h, V3 o, V3 d,
-                                          int x, int y) {
+                                          int x, int y, int prim_offset = 0) {
     const size_t px = (size_t)y * F.width + x;
     if (h.ref >= 0) {
         const HitDetails hd = hit_details(S, h, o, d);
-        F.aov_prim[px] = hd.prim;
+        F.aov_prim[px] = hd.prim + prim_offset;
         F.aov_t[px] = h.t;
         F.aov_uv[px] = make_float2(hd.u, hd.v);
     } else {
@@ -402,6 +495,21 @@ __device__ __forceinline__ void write_aov(const ClptScene &S, const ClptFrame &F
         F.aov_t[px] = 0.0f;
         F.aov_uv[px] = make_float2(0.0f, 0.0f);
     }
+}
+
+// AOVs of a first hit: an instance hit reports its primitive shifted by the instance's offset and
+// u, v in its own triangle (the object-space ray); t is the world t either way.
+template <bool COUNT, bool INST>
+__device__ __forceinline__ void write_hit_aov(const ClptScene &S, const ClptInstances &I, const ClptFrame &F,
+                                              const Hit &h, V3 o, V3 d, int x, int y) {
+    if (INST && h.ref >= 0 && h.inst >= 0) {
+        const ClptInstanceRec &R = I.rec[h.inst];
+        V3 lo, ld;
+        object_ray(R.w2o, o, d, lo, ld);
+        write_aov<COUNT>(R.mesh, F, h, lo, ld, x, y, R.prim_offset);
+        return;
+    }
+    write_aov<COUNT>(S, F, h, o, d, x, y);
 }
 
 // Philox4x32-10, counter (pixel, sample, dimension block, lane), key (seed, 'clpt').

@@ -10,9 +10,11 @@
 
 #include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -117,6 +119,21 @@ struct {
     ClptScene scene = {};
     bool have_scene = false;
 
+    // rigid instances: every instance mesh owns its mesh, its wire tree (CLDownloadInstanceKd) and
+    // its traversal layout; the device table (ClptInstanceRec) is rewritten before the next frame
+    // whenever the instances or the base scene's primitive count may have changed
+    struct InstanceMesh {
+        DevBuf<float4> verts, norms;
+        DevBuf<int4> corners;
+        ClptGpuTree tree;
+        ClptSceneLayout layout;
+        ClptScene scene = {};
+    };
+    std::vector<std::unique_ptr<InstanceMesh>> inst_meshes;
+    std::vector<CLInstance> instances;
+    DevBuf<ClptInstanceRec> inst_table;
+    bool inst_table_stale = true;
+
     float cam[16] = { 0 };
 
     int mode = CLPT_MODE_NORMAL, depth = 2, spp = 1, flags = 0; // depth 2: src/kernel.cl:468
@@ -199,37 +216,42 @@ int local_rows_for(int height) {
     return mine * St.tile_rows;
 }
 
-void rebuild_scene_struct() {
-    ClptScene &S = St.scene;
-    S.nodes = St.layout.nodes.ptr;
-    S.leaves = St.layout.leaves.ptr;
-    S.tri = St.layout.tri.ptr;
-    S.corners = St.corners.ptr;
-    S.flat_n = St.layout.flat_n.ptr;
-    S.lut = St.layout.lut.ptr;
-    S.norms = St.norms.ptr;
-    S.tri_material = St.tri_material.ptr;
-    S.materials = St.materials.ptr;
-    S.n_materials = (int)St.materials.count;
-    S.n_norms = (int)St.norms.count;
-}
-
-// St.layout holds a new scene of `n_prims` primitives: point the launch at it and choose the engine.
-void adopt_layout(int n_prims) {
-    const ClptSceneLayout &L = St.layout;
-    ClptScene &S = St.scene;
+// The traversal fields of a scene record: layout L of a mesh with these corners and normals.
+void set_scene_mesh(ClptScene &S, const ClptSceneLayout &L, const DevBuf<int4> &corners, const DevBuf<float4> &norms) {
+    S.nodes = L.nodes.ptr;
+    S.leaves = L.leaves.ptr;
+    S.tri = L.tri.ptr;
+    S.corners = corners.ptr;
+    S.flat_n = L.flat_n.ptr;
+    S.lut = L.lut.ptr;
+    S.norms = norms.ptr;
+    S.n_norms = (int)norms.count;
     S.n_nodes = L.n_nodes;
     S.n_leaves = L.n_leaves;
     S.n_refs = L.n_refs;
-    S.n_prims = n_prims;
     for (int a = 0; a < 3; a++) {
         S.root_min[a] = L.root_min[a];
         S.root_max[a] = L.root_max[a];
         S.lut_dim[a] = L.lut_dim[a];
         S.lut_scale[a] = L.lut_scale[a];
     }
+}
+
+void rebuild_scene_struct() {
+    ClptScene &S = St.scene;
+    set_scene_mesh(S, St.layout, St.corners, St.norms);
+    S.tri_material = St.tri_material.ptr;
+    S.materials = St.materials.ptr;
+    S.n_materials = (int)St.materials.count;
+}
+
+// St.layout holds a new scene of `n_prims` primitives: point the launch at it and choose the engine.
+void adopt_layout(int n_prims) {
+    const ClptSceneLayout &L = St.layout;
+    St.scene.n_prims = n_prims;
     rebuild_scene_struct();
     St.have_scene = true;
+    St.inst_table_stale = true; // the instances' primitive ids follow the base scene's
     // "automatic" engine for this tree: the fat-leaf variant when most triangle slots live in
     // fat leaves AND the tree is big (the reference builder's DEPTH-15 trees from a few hundred
     // thousand triangles up; measured at 100k triangles engine 1 is still 10% faster)
@@ -453,6 +475,62 @@ void p2p_setup() {
 }
 
 void release_read_pipeline();
+
+// The instances of the next frame: the device table, written again if anything it holds changed.
+ClptInstances current_instances() {
+    ClptInstances I = { nullptr, 0 };
+    if (St.instances.empty()) return I;
+    if (St.inst_table_stale) {
+        std::vector<ClptInstanceRec> recs(St.instances.size());
+        int offset = St.scene.n_prims;
+        for (size_t k = 0; k < recs.size(); k++) {
+            const CLInstance &in = St.instances[k];
+            ClptInstanceRec &r = recs[k];
+            memset(&r, 0, sizeof(r));
+            memcpy(r.w2o, in.world_to_object, sizeof(r.w2o));
+            r.material = in.material;
+            r.prim_offset = offset;
+            r.mesh = St.inst_meshes[in.mesh]->scene;
+            offset += r.mesh.n_prims;
+        }
+        St.inst_table.upload(recs.data(), recs.size(), St.stream);
+        St.inst_table_stale = false;
+    }
+    I.rec = St.inst_table.ptr;
+    I.count = (int)St.instances.size();
+    return I;
+}
+
+void release_instance_meshes() {
+    for (auto &m : St.inst_meshes) {
+        m->verts.release();
+        m->norms.release();
+        m->corners.release();
+        m->tree.release();
+        m->layout.release();
+    }
+    St.inst_meshes.clear();
+    St.instances.clear();
+    St.inst_table.release();
+    St.inst_table_stale = true;
+}
+
+// A device-built tree and its mesh as fresh host lists (CLDownloadKd, CLDownloadInstanceKd).
+void download_tree(const ClptGpuTree &tree, const DevBuf<float4> &verts, const DevBuf<int4> &corners,
+                   const DevBuf<float4> &norms, kd *out) {
+    CU(cudaStreamSynchronize(St.stream));
+    const size_t n = (size_t)tree.n_nodes, r = (size_t)tree.n_refs;
+    out->node_vec = (kdnode *)init_list(n, sizeof(kdnode));
+    out->tri_indices = (int *)init_list(r, sizeof(int));
+    out->vert_vec = (Vector4 *)init_list(verts.count, sizeof(Vector4));
+    out->tri_vec = (cl_int3 *)init_list(corners.count, sizeof(cl_int3));
+    out->norm_vec = (Vector4 *)init_list(norms.count, sizeof(Vector4));
+    CU(cudaMemcpy(out->node_vec, tree.wire.ptr, n * sizeof(kdnode), cudaMemcpyDeviceToHost));
+    if (r) CU(cudaMemcpy(out->tri_indices, tree.tri_indices.ptr, r * sizeof(int), cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(out->vert_vec, verts.ptr, verts.count * sizeof(Vector4), cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(out->tri_vec, corners.ptr, corners.count * sizeof(cl_int3), cudaMemcpyDeviceToHost));
+    if (norms.count) CU(cudaMemcpy(out->norm_vec, norms.ptr, norms.count * sizeof(Vector4), cudaMemcpyDeviceToHost));
+}
 
 // The AOV buffers at the size of the render target, cleared (prim_id -1: no hit).
 void alloc_aovs() {
@@ -737,12 +815,13 @@ void clpt_state_launch_frame(int width, int height) {
         F.row_count = order_rows;
         if (St.claim_reverse) F.flags |= CLPT_F_REVERSE;
     }
+    const ClptInstances inst = current_instances();
     if (p2p) {
         flag_barrier(); // every rank has finished with (reading) the previous frame
         St.last_launches++;
     }
     CU(cudaEventRecord(St.ev_start, St.stream));
-    clpt_launch_render(St.scene, F, St.prop.multiProcessorCount, St.stream);
+    clpt_launch_render(St.scene, F, inst, St.prop.multiProcessorCount, St.stream);
     St.last_launches++;
     CU(cudaGetLastError());
     CU(cudaEventRecord(St.ev_stop, St.stream));
@@ -871,6 +950,7 @@ void CLTerminate(void) {
     St.verts.release();
     St.gpu_tree.release();
     St.scene_on_gpu = St.mesh_on_gpu = false;
+    release_instance_meshes();
     clpt_gpu_build_release();
     St.objects.release();
     St.materials.release();
@@ -1049,20 +1129,87 @@ int CLLastBuildWasRecorded(void) { return clpt_gpu_build_was_recorded() ? 1 : 0;
 void CLDownloadKd(kd *out) {
     require_init("CLDownloadKd");
     if (!St.scene_on_gpu) FATAL("CLDownloadKd: the current scene was not built by CLBuildMeshes");
-    CU(cudaStreamSynchronize(St.stream));
-    const size_t n = (size_t)St.gpu_tree.n_nodes, r = (size_t)St.gpu_tree.n_refs;
-    out->node_vec = (kdnode *)init_list(n, sizeof(kdnode));
-    out->tri_indices = (int *)init_list(r, sizeof(int));
-    out->vert_vec = (Vector4 *)init_list(St.verts.count, sizeof(Vector4));
-    out->tri_vec = (cl_int3 *)init_list(St.corners.count, sizeof(cl_int3));
-    out->norm_vec = (Vector4 *)init_list(St.norms.count, sizeof(Vector4));
-    CU(cudaMemcpy(out->node_vec, St.gpu_tree.wire.ptr, n * sizeof(kdnode), cudaMemcpyDeviceToHost));
-    if (r) CU(cudaMemcpy(out->tri_indices, St.gpu_tree.tri_indices.ptr, r * sizeof(int), cudaMemcpyDeviceToHost));
-    CU(cudaMemcpy(out->vert_vec, St.verts.ptr, St.verts.count * sizeof(Vector4), cudaMemcpyDeviceToHost));
-    CU(cudaMemcpy(out->tri_vec, St.corners.ptr, St.corners.count * sizeof(cl_int3), cudaMemcpyDeviceToHost));
-    if (St.norms.count) {
-        CU(cudaMemcpy(out->norm_vec, St.norms.ptr, St.norms.count * sizeof(Vector4), cudaMemcpyDeviceToHost));
+    download_tree(St.gpu_tree, St.verts, St.corners, St.norms, out);
+}
+
+int CLAddInstanceMesh(const void *verts, size_t vert_bytes, const void *tris, size_t tri_bytes, const void *norms,
+                      size_t norm_bytes) {
+    require_init("CLAddInstanceMesh");
+    const size_t n_verts = vert_bytes / sizeof(Vector4), n_corners = tri_bytes / sizeof(cl_int3);
+    const size_t n_norms = norms ? norm_bytes / sizeof(Vector4) : 0;
+    if (!verts || !tris || n_verts == 0 || n_corners < 3) FATAL("CLAddInstanceMesh: empty mesh");
+    auto M = std::make_unique<decltype(St)::InstanceMesh>();
+    M->verts.resize(n_verts);
+    CU(cudaMemcpyAsync(M->verts.ptr, verts, n_verts * sizeof(float4), cudaMemcpyHostToDevice, St.stream));
+    M->corners.resize(n_corners);
+    CU(cudaMemcpyAsync(M->corners.ptr, tris, n_corners * sizeof(int4), cudaMemcpyHostToDevice, St.stream));
+    if (n_norms) {
+        M->norms.resize(n_norms);
+        CU(cudaMemcpyAsync(M->norms.ptr, norms, n_norms * sizeof(float4), cudaMemcpyHostToDevice, St.stream));
     }
+    // The builder's recorded graph is keyed by the buffers it writes, so a build into this mesh's
+    // tree after one of the base scene (or the other way round) records the graph again: correct,
+    // and only the steady replay of one and the same build is what the recording is for.
+    const int n_prims = (int)(n_corners / 3);
+    char err[256] = "";
+    if (!clpt_gpu_build(M->verts.ptr, (int)n_verts, M->corners.ptr, n_prims, St.build_params, M->tree, St.stream, err,
+                        sizeof err) ||
+        !clpt_gpu_pack(M->tree, M->verts.ptr, M->corners.ptr, n_prims, M->layout, St.stream, err, sizeof err)) {
+        fprintf(stderr, "CLAddInstanceMesh: invalid scene: %s\n", err);
+        exit(EXIT_FAILURE);
+    }
+    CU(cudaStreamSynchronize(St.stream));
+    set_scene_mesh(M->scene, M->layout, M->corners, M->norms);
+    M->scene.n_prims = n_prims;
+    St.inst_meshes.push_back(std::move(M));
+    return (int)St.inst_meshes.size() - 1;
+}
+
+void CLSetInstances(const CLInstance *instances, size_t bytes) {
+    require_init("CLSetInstances");
+    static_assert(sizeof(CLInstance) == 64, "CLInstance is 64 bytes");
+    if (bytes % sizeof(CLInstance) != 0) {
+        fprintf(stderr, "CLSetInstances: %zu bytes is not a whole number of 64-byte CLInstance records\n", bytes);
+        exit(EXIT_FAILURE);
+    }
+    const size_t n = bytes / sizeof(CLInstance);
+    if (n > CLPT_MAX_INSTANCES) {
+        fprintf(stderr, "CLSetInstances: %zu instances, at most %d\n", n, CLPT_MAX_INSTANCES);
+        exit(EXIT_FAILURE);
+    }
+    if (n && !instances) FATAL("CLSetInstances: NULL instances");
+    for (size_t k = 0; k < n; k++) {
+        const CLInstance &in = instances[k];
+        if (in.mesh < 0 || (size_t)in.mesh >= St.inst_meshes.size()) {
+            fprintf(stderr, "CLSetInstances: instance %zu names mesh %d; %zu instance meshes exist\n", k, in.mesh,
+                    St.inst_meshes.size());
+            exit(EXIT_FAILURE);
+        }
+        for (int e = 0; e < 12; e++) {
+            if (!std::isfinite(in.world_to_object[e])) {
+                fprintf(stderr, "CLSetInstances: instance %zu: world_to_object[%d] is not finite\n", k, e);
+                exit(EXIT_FAILURE);
+            }
+        }
+    }
+    St.instances.assign(instances, instances + n);
+    St.inst_table_stale = true;
+}
+
+void CLClearInstanceMeshes(void) {
+    require_init("CLClearInstanceMeshes");
+    CU(cudaStreamSynchronize(St.stream));
+    release_instance_meshes();
+}
+
+void CLDownloadInstanceKd(int mesh, kd *out) {
+    require_init("CLDownloadInstanceKd");
+    if (mesh < 0 || (size_t)mesh >= St.inst_meshes.size()) {
+        fprintf(stderr, "CLDownloadInstanceKd: no instance mesh %d (%zu exist)\n", mesh, St.inst_meshes.size());
+        exit(EXIT_FAILURE);
+    }
+    const auto &M = *St.inst_meshes[mesh];
+    download_tree(M.tree, M.verts, M.corners, M.norms, out);
 }
 
 size_t CLDebugReadPacked(int which, void *dst, size_t bytes) {

@@ -39,8 +39,9 @@ __host__ __device__ inline void warp_tile_dims(int log2_ppw, int &tw, int &th) {
     th = 1 << (log2_ppw >> 1);
 }
 
-template <int MODE, bool COUNT, bool SHARE>
-__device__ __forceinline__ V3 trace_sample(const ClptScene &S, const ClptFrame &F, int x, int y, unsigned pixel,
+// INST: the instanced variant (clpt_trace.cuh: scene_hit), launched only while instances exist.
+template <int MODE, bool COUNT, bool SHARE, bool INST>
+__device__ __forceinline__ V3 trace_sample(const ClptScene &S, const ClptInstances &I, const ClptFrame &F, int x, int y, unsigned pixel,
                                            unsigned sample, bool aov, Counters &cn_in, int sub, int log2_k) {
     Counters scratch = { 0, 0, 0, 0, 0, 0 };
     Counters &cn = (SHARE && sub != 0) ? scratch : cn_in; // shading is counted once per ray
@@ -49,17 +50,19 @@ __device__ __forceinline__ V3 trace_sample(const ClptScene &S, const ClptFrame &
     if (MODE == 2) {
         V3 Lsum = mk(0.0f, 0.0f, 0.0f), T = mk(1.0f, 1.0f, 1.0f);
         for (int seg = 0; seg < F.depth; seg++) {
-            const Hit h = closest_hit<COUNT, SHARE>(S, o, d, F.max_leaf_visits, cn_in, sub, log2_k);
-            if (seg == 0 && aov) write_aov<COUNT>(S, F, h, o, d, x, y);
+            const Hit h = scene_hit<COUNT, SHARE, INST>(S, I, o, d, F.max_leaf_visits, cn_in, sub, log2_k);
+            if (seg == 0 && aov) write_hit_aov<COUNT, INST>(S, I, F, h, o, d, x, y);
             if (h.ref < 0) {
                 Lsum = vadd(Lsum, T);
                 break;
             }
-            const V3 nrm = hit_normal<COUNT>(S, h, o, d, cn);
+            const V3 nrm = shading_normal<COUNT, INST>(S, I, h, o, d, cn);
             float al[3] = { 0.5f, 0.5f, 0.5f }, em[3] = { 0.0f, 0.0f, 0.0f };
             int kind = 0;
             if (S.n_materials > 0) {
-                int m = S.tri_material ? __ldg(S.tri_material + __float_as_int(__ldg(&S.tri[3 * (size_t)h.ref].w))) : 0;
+                int m;
+                if (INST && h.inst >= 0) m = I.rec[h.inst].material;
+                else m = S.tri_material ? __ldg(S.tri_material + __float_as_int(__ldg(&S.tri[3 * (size_t)h.ref].w))) : 0;
                 if (m < 0 || m >= S.n_materials) m = 0;
                 const ClptMaterial *mp = S.materials + m;
                 al[0] = mp->albedo[0]; al[1] = mp->albedo[1]; al[2] = mp->albedo[2];
@@ -87,10 +90,10 @@ __device__ __forceinline__ V3 trace_sample(const ClptScene &S, const ClptFrame &
     if (MODE == 0) depth = depth > 0 ? 1 : 0;
     const int first_depth = depth;
     for (; depth > 0; depth--) {
-        const Hit h = closest_hit<COUNT, SHARE>(S, o, d, F.max_leaf_visits, cn_in, sub, log2_k);
-        if (depth == first_depth && aov) write_aov<COUNT>(S, F, h, o, d, x, y);
+        const Hit h = scene_hit<COUNT, SHARE, INST>(S, I, o, d, F.max_leaf_visits, cn_in, sub, log2_k);
+        if (depth == first_depth && aov) write_hit_aov<COUNT, INST>(S, I, F, h, o, d, x, y);
         if (h.ref < 0) break;
-        const V3 nrm = hit_normal<COUNT>(S, h, o, d, cn);
+        const V3 nrm = shading_normal<COUNT, INST>(S, I, h, o, d, cn);
         // (n + 1) / 2 (:395): halving is exact in binary floating point, so the product by 0.5 is the
         // quotient by 2 bit for bit -- and one instruction instead of an IEEE division
         const V3 nc = mk(fmul(fadd(nrm.x, 1.0f), 0.5f), fmul(fadd(nrm.y, 1.0f), 0.5f),
@@ -128,10 +131,12 @@ __device__ __forceinline__ void group_sync(int log2_g, int group) {
 }
 
 // VARIANT 0: compiled for 8 resident blocks per SM (engine 1).  1: the same code for
-// CLPT_FAT_MIN_BLOCKS (engine 2, trees with fat leaves).
-template <int MODE, bool COUNT, int VARIANT>
+// CLPT_FAT_MIN_BLOCKS (engine 2, trees with fat leaves).  INST: walks the instances of I after the
+// base scene; the variants without it ignore I and are the kernels of a frame without instances.
+template <int MODE, bool COUNT, int VARIANT, bool INST>
 __global__ void __launch_bounds__(256, VARIANT == 1 ? CLPT_FAT_MIN_BLOCKS : CLPT_MIN_BLOCKS)
-render_kernel(const __grid_constant__ ClptScene S, const __grid_constant__ ClptFrame F) {
+render_kernel(const __grid_constant__ ClptScene S, const __grid_constant__ ClptFrame F,
+              const __grid_constant__ ClptInstances I) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int log2_s = F.log2_sample_lanes, s_lanes = 1 << log2_s;
     // Warps per pixel.  At >= 64 spp a pixel's samples are spread over G = 2, 4 or 8 warps of
@@ -219,7 +224,7 @@ render_kernel(const __grid_constant__ ClptScene S, const __grid_constant__ ClptF
             }
             const int in_round = min(round_samples, spp - base);
             if (valid && s < spp) {
-                colour = trace_sample<MODE, COUNT, VARIANT == 1>(S, F, x, y, pixel, F.sample_base + (unsigned)s,
+                colour = trace_sample<MODE, COUNT, VARIANT == 1, INST>(S, I, F, x, y, pixel, F.sample_base + (unsigned)s,
                                                                  s == 0 && sub == 0 && F.aov_prim != nullptr, cn, sub,
                                                                  log2_r);
             }
@@ -352,16 +357,24 @@ __global__ void flag_barrier_kernel(const __grid_constant__ ClptFlagPeers peers,
     } while ((int)(seen - epoch) < 0);
 }
 
-template <int MODE>
-void launch_mode(const ClptScene &scene, const ClptFrame &frame, unsigned grid, cudaStream_t stream) {
+template <int MODE, bool INST>
+void launch_variant(const ClptScene &scene, const ClptFrame &frame, const ClptInstances &inst, unsigned grid,
+                    cudaStream_t stream) {
     const bool fat = (frame.flags & CLPT_F_FAT) != 0;
     if (frame.flags & CLPT_F_COUNTERS) {
-        if (fat) render_kernel<MODE, true, 1><<<grid, 256, 0, stream>>>(scene, frame);
-        else render_kernel<MODE, true, 0><<<grid, 256, 0, stream>>>(scene, frame);
+        if (fat) render_kernel<MODE, true, 1, INST><<<grid, 256, 0, stream>>>(scene, frame, inst);
+        else render_kernel<MODE, true, 0, INST><<<grid, 256, 0, stream>>>(scene, frame, inst);
     } else {
-        if (fat) render_kernel<MODE, false, 1><<<grid, 256, 0, stream>>>(scene, frame);
-        else render_kernel<MODE, false, 0><<<grid, 256, 0, stream>>>(scene, frame);
+        if (fat) render_kernel<MODE, false, 1, INST><<<grid, 256, 0, stream>>>(scene, frame, inst);
+        else render_kernel<MODE, false, 0, INST><<<grid, 256, 0, stream>>>(scene, frame, inst);
     }
+}
+
+template <int MODE>
+void launch_mode(const ClptScene &scene, const ClptFrame &frame, const ClptInstances &inst, unsigned grid,
+                 cudaStream_t stream) {
+    if (inst.count > 0) launch_variant<MODE, true>(scene, frame, inst, grid, stream);
+    else launch_variant<MODE, false>(scene, frame, inst, grid, stream);
 }
 
 } // namespace
@@ -375,7 +388,8 @@ int clpt_render_block_rows(const ClptFrame &frame) {
 
 int clpt_render_blocks_per_sm(int engine) { return engine == 2 ? CLPT_FAT_MIN_BLOCKS : CLPT_MIN_BLOCKS; }
 
-void clpt_launch_render(const ClptScene &scene, const ClptFrame &frame_in, int sm_count, cudaStream_t stream) {
+void clpt_launch_render(const ClptScene &scene, const ClptFrame &frame_in, const ClptInstances &inst, int sm_count,
+                        cudaStream_t stream) {
     ClptFrame frame = frame_in;
     if (!(frame.flags & CLPT_F_FAT)) frame.log2_lanes_per_ray = 0;
     int tw, th;
@@ -391,9 +405,9 @@ void clpt_launch_render(const ClptScene &scene, const ClptFrame &frame_in, int s
     if (grid > bx * by) grid = bx * by;
     cudaMemsetAsync(frame.work_counter, 0, sizeof(unsigned), stream);
     switch (frame.mode) {
-    case 0: launch_mode<0>(scene, frame, grid, stream); break;
-    case 1: launch_mode<1>(scene, frame, grid, stream); break;
-    default: launch_mode<2>(scene, frame, grid, stream); break;
+    case 0: launch_mode<0>(scene, frame, inst, grid, stream); break;
+    case 1: launch_mode<1>(scene, frame, inst, grid, stream); break;
+    default: launch_mode<2>(scene, frame, inst, grid, stream); break;
     }
 }
 
@@ -431,5 +445,5 @@ void clpt_launch_pack_rgba8(const float4 *src, uchar4 *dst, size_t n, cudaStream
 }
 
 const void *clpt_render_kernel_symbol(void) {
-    return reinterpret_cast<const void *>(&render_kernel<0, false, 0>);
+    return reinterpret_cast<const void *>(&render_kernel<0, false, 0, false>);
 }

@@ -152,6 +152,46 @@ void CLDownloadKd(kd *out);
 size_t CLDebugReadPacked(int which, void *dst, size_t bytes);
 void CLSetMaterials(const CLMaterial *materials, size_t material_bytes,
                     const int *tri_material, size_t tri_material_bytes);
+
+/* Rigid instances: a mesh uploaded and built once, drawn any number of times under a rigid
+ * (or any affine) transform by mapping each ray into the mesh's object space -- moving an
+ * object costs one small upload per frame and no tree rebuild.
+ *   - Object-space ray: o' = A o + b and d' = A d, each row left to right without FMA
+ *     contraction; d' is NOT normalised, so the object-space t is the world ray's t.
+ *   - A frame walks the base scene first, then the instances in array order, each with its own
+ *     root clip, start table, ropes and rope-hop budget.  A later hit replaces the current one
+ *     when t <= best (the later tree wins ties).  An instance is skipped when a hit exists and
+ *     the ray enters the instance's root box beyond it.
+ *   - Shading: the object-space normal before normalisation (the flat normal's cross product
+ *     or the interpolated vertex normals) is mapped by A^T and normalised; the hit point and
+ *     the bounce use the world ray.
+ *   - Primitive ids: the base scene keeps [0, P); instance k's primitives follow at
+ *     P + the primitives of the instances before it, P being the base scene current at
+ *     CLExecute.  AOVs report that id, the world t and u, v in the instance's triangle.
+ *   - Mode 2: every triangle of an instance has the instance's material (clamped like
+ *     tri_material ids); work counters count one ray per world query and sum every walk.
+ * A frame still needs a base scene.  Bad input (a handle out of range, a non-finite matrix
+ * entry, a byte count that is not a multiple of 64, more than CLPT_MAX_INSTANCES) prints a
+ * message and exit(EXIT_FAILURE)s. */
+#define CLPT_MAX_INSTANCES 64
+typedef struct CLInstance {      /* 64 bytes */
+    float world_to_object[12];   /* row-major 3x4 [A | b]: object point = A * world point + b;
+                                  * from an object-to-world matrix with mat_inverse (clpt_host.h) */
+    int mesh;                    /* handle from CLAddInstanceMesh */
+    int material;                /* mode 2: material of all its triangles */
+    int pad[2];
+} CLInstance;
+/* Upload a mesh (the formats of CLBuildMeshes) and build its kd-tree and traversal layout on
+ * the device, once.  Returns a handle >= 0.  The base scene (CLSetMeshes / CLBuildMeshes) is
+ * untouched, and instance meshes survive base-scene changes until CLClearInstanceMeshes or
+ * CLTerminate. */
+int CLAddInstanceMesh(const void *verts, size_t vert_bytes, const void *tris, size_t tri_bytes,
+                      const void *norms, size_t norm_bytes);
+/* The instances of the next frames (replaces the previous set; NULL / 0 = none).  Per frame
+ * this is the only upload a rigid motion needs.  At most CLPT_MAX_INSTANCES. */
+void CLSetInstances(const CLInstance *instances, size_t bytes);
+void CLClearInstanceMeshes(void);              /* frees every instance mesh and clears the instances */
+void CLDownloadInstanceKd(int mesh, kd *out);  /* an instance mesh's tree, like CLDownloadKd */
 /* mode, depth (= bounces + 1; the reference passes 2, src/kernel.cl:468),
  * samples per pixel per frame, RNG seed, CLPT_FLAG_* */
 void CLSetRenderParams(int mode, int depth, int spp, unsigned int seed, int flags);
