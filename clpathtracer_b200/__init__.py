@@ -72,6 +72,19 @@ class CLMaterial(C.Structure):
 
 
 MAX_INSTANCES = 64
+MAX_TREE_INSTANCES = 1 << 20
+INSTANCES_LIST, INSTANCES_TREE = 0, 1
+
+INSTANCE_TREE_DTYPE = np.dtype(
+    {
+        "names": ["min0", "ref0", "max0", "pad0", "min1", "ref1", "max1", "pad1"],
+        "formats": [("<f4", 3), "<i4", ("<f4", 3), "<i4", ("<f4", 3), "<i4", ("<f4", 3), "<i4"],
+        "offsets": [0, 12, 16, 28, 32, 44, 48, 60],
+        "itemsize": 64,
+    }
+)
+"""Instance-tree node (CLDebugReadInstanceTree): the boxes of child 0 and child 1 and their
+references; ref >= 0 is an internal node, ref < 0 is instance -1 - ref.  Node 0 is the root."""
 
 
 class CLInstance(C.Structure):
@@ -87,6 +100,20 @@ def world_to_object(object_to_world) -> np.ndarray:
     full = np.eye(4)
     full[:3, :] = m[:3, :4]
     return np.linalg.inv(full)[:3, :].astype(np.float32)
+
+
+def world_to_object_batch(object_to_world) -> np.ndarray:
+    """world_to_object of every matrix of float[n,3,4] or float[n,4,4], in one batched float64
+    inversion; the same float32 bytes as world_to_object matrix by matrix."""
+    m = np.asarray(object_to_world, dtype=np.float64)
+    full = np.broadcast_to(np.eye(4), (len(m), 4, 4)).copy()
+    full[:, :3, :] = m[:, :3, :4]
+    return np.linalg.inv(full)[:, :3, :].astype(np.float32)
+
+
+CLINSTANCE_DTYPE = np.dtype({"names": ["world_to_object", "mesh", "material", "pad"],
+                             "formats": [("<f4", 12), "<i4", "<i4", ("<i4", 2)],
+                             "offsets": [0, 48, 52, 56], "itemsize": 64})
 
 
 _lib = None
@@ -133,6 +160,8 @@ def lib() -> C.CDLL:
         "CLDownloadKd": (None, [C.POINTER(KD)]), "CLDebugReadPacked": (sz, [i, vp, sz]),
         "CLAddInstanceMesh": (i, [vp, sz, vp, sz, vp, sz]), "CLSetInstances": (None, [vp, sz]),
         "CLClearInstanceMeshes": (None, []), "CLDownloadInstanceKd": (None, [i, C.POINTER(KD)]),
+        "CLSetInstanceTraversal": (None, [i]), "CLInstanceTraversal": (i, []),
+        "CLDebugReadInstanceTree": (sz, [vp, sz]), "CLLastInstanceBuildMs": (None, [C.POINTER(f)]),
         "CLUpdateVertices": (None, [sz, vp, sz]), "CLRebuildMeshes": (None, []),
         "CLDeleteImage": (None, []), "CLCreateImage": (None, [u]), "CLExecute": (None, [i, i]),
         "CLSelectDevice": (None, [i]), "CLSetRenderParams": (None, [i, i, i, u, i]),
@@ -372,6 +401,38 @@ class Renderer:
             table[k].world_to_object[:] = [float(x) for x in world_to_object(o2w).reshape(12)]
             table[k].mesh, table[k].material = int(mesh), int(material)
         self.L.CLSetInstances(C.addressof(table) if instances else None, C.sizeof(table))
+
+    def set_instance_arrays(self, meshes, object_to_world, materials) -> None:
+        """set_instances from arrays: mesh handles int[n], object_to_world float[n,3,4] or
+        float[n,4,4], materials int[n] (or one int for all), inverted in one batched float64 call."""
+        n = len(object_to_world)
+        table = np.zeros(n, dtype=CLINSTANCE_DTYPE)
+        if n:
+            table["world_to_object"] = world_to_object_batch(object_to_world).reshape(n, 12)
+        table["mesh"] = meshes
+        table["material"] = materials
+        self.L.CLSetInstances(table.ctypes.data if n else None, table.nbytes)
+
+    def set_instance_traversal(self, traversal: str) -> None:
+        """"list" (the default) or "tree" (CLSetInstanceTraversal), from the next frame on."""
+        self.L.CLSetInstanceTraversal({"list": INSTANCES_LIST, "tree": INSTANCES_TREE}[traversal])
+
+    def instance_traversal(self) -> str:
+        return ["list", "tree"][self.L.CLInstanceTraversal()]
+
+    def instance_tree(self) -> np.ndarray:
+        """The instance tree's nodes (INSTANCE_TREE_DTYPE), built first if stale; empty without instances."""
+        n = self.L.CLDebugReadInstanceTree(None, 0)
+        out = np.zeros(n // 64, dtype=INSTANCE_TREE_DTYPE)
+        if n:
+            self.L.CLDebugReadInstanceTree(out.ctypes.data, n)
+        return out
+
+    def instance_build_ms(self) -> float:
+        """Device time of the last instance-tree build."""
+        ms = C.c_float(0)
+        self.L.CLLastInstanceBuildMs(C.byref(ms))
+        return ms.value
 
     def clear_instance_meshes(self) -> None:
         self.L.CLClearInstanceMeshes()

@@ -22,8 +22,8 @@ LIB = PKG / "libclpt.so"
 
 HOST_C = ["host/hostlist.c", "host/vecmath.c", "host/kd_build.c", "host/model_io.c", "host/frame_sched.c"]
 HOST_CXX = ["cuda/scene_pack.cpp"]
-CUDA = ["cuda/render_kernel.cu", "cuda/kd_build_gpu.cu", "cuda/gl_interop.cu", "cuda/clstate.cu",
-        "cuda/clhandler.cu"]
+CUDA = ["cuda/render_kernel.cu", "cuda/kd_build_gpu.cu", "cuda/instance_tree.cu", "cuda/gl_interop.cu",
+        "cuda/clstate.cu", "cuda/clhandler.cu"]
 
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 
@@ -104,6 +104,9 @@ def build_oracle() -> None:
     # the rigid-instance restatement (oracle/oracle_instances_py.py builds it the same way when missing)
     _run(["gcc", "-std=c11", "-O2", "-fPIC", "-ffp-contract=off", "-fopenmp", "-w", "-shared", "-o",
           str(ROOT / "oracle" / "liboracle_instances.so"), str(ROOT / "oracle" / "oracle_instances.c"), "-lm"])
+    # ... and the instance tree's (oracle/oracle_instance_tree_py.py)
+    _run(["gcc", "-std=c11", "-O2", "-fPIC", "-ffp-contract=off", "-fopenmp", "-w", "-shared", "-o",
+          str(ROOT / "oracle" / "liboracle_instance_tree.so"), str(ROOT / "oracle" / "oracle_instance_tree.c"), "-lm"])
 
 
 if __name__ == "__main__":

@@ -72,10 +72,37 @@ struct ClptInstanceRec {
     ClptScene mesh;  // the instance mesh's traversal layout (materials unused)
 };
 
-struct ClptInstances {
-    const ClptInstanceRec *rec; // device table of `count` records
-    int count;
+// Instance tree (CLPT_INSTANCES_TREE): one 64-byte record per instance, the CLInstance layout with
+// the primitive offset in its first pad word; the mesh is an index into a table of ClptScenes.
+struct ClptInstRec {
+    float w2o[12];   // world to object, row-major 3x4 [A | b]
+    int mesh;        // index into ClptInstances::meshes
+    int material;
+    int prim_offset;
+    int pad;
 };
+
+// Instance tree node, four float4s (64 bytes): slot s in [0, 1] is f[2s] = (min.xyz, ref as int
+// bits), f[2s + 1] = (max.xyz, 0).  ref >= 0 names an internal node, ref < 0 instance -1 - ref.
+// Node 0 is the root.  With one instance, slot 1 of the root is an empty box (min > max).
+#define CLPT_TREE_STACK 64 // the tree's depth is at most 50: each split consumes a bit of a 50-bit key
+
+struct ClptInstances {
+    const ClptInstanceRec *rec; // list: device table of `count` records
+    int count;
+    // tree: `count` compact records, the mesh table and the node array (count >= 1)
+    const ClptInstRec *crec;
+    const ClptScene *meshes;
+    const float4 *tree;
+};
+
+// instance_tree.cu: builds the tree over the world boxes of n >= 1 instances into `nodes`
+// (max(n - 1, 1) records) in stream order, without a host round trip.  `scratch` holds
+// clpt_instance_tree_scratch_bytes(n) bytes: world boxes, keys, parent links, arrival flags and
+// the sort's workspace.
+size_t clpt_instance_tree_scratch_bytes(int n);
+void clpt_build_instance_tree(const ClptInstRec *recs, const ClptScene *meshes, int n, float4 *nodes,
+                              void *scratch, cudaStream_t stream);
 
 #define CLPT_MAX_PEERS 8
 

@@ -377,15 +377,99 @@ __device__ __forceinline__ void object_ray(const float *m, V3 o, V3 d, V3 &lo, V
             fadd(fadd(fmul(m[8], d.x), fmul(m[9], d.y)), fmul(m[10], d.z)));
 }
 
+// ---- instance tree (DESIGN.md "Instance tree") -------------------------------------------------
+// Slab test of a world box: root_clip's operations and acceptance; the entry is tmin.
+__device__ __forceinline__ bool box_clip(float4 mn, float4 mx, V3 o, V3 inv, float &tmin) {
+    const bool sx = inv.x < 0.0f, sy = inv.y < 0.0f, sz = inv.z < 0.0f;
+    const float nx = sx ? mx.x : mn.x, fx = sx ? mn.x : mx.x;
+    const float ny = sy ? mx.y : mn.y, fy = sy ? mn.y : mx.y;
+    const float nz = sz ? mx.z : mn.z, fz = sz ? mn.z : mx.z;
+    tmin = fmul(fsub(nx, o.x), inv.x);
+    float tmax = fmul(fsub(fx, o.x), inv.x);
+    const float tymin = fmul(fsub(ny, o.y), inv.y), tymax = fmul(fsub(fy, o.y), inv.y);
+    if ((tmin > tymax) || (tymin > tmax)) return false;
+    if (tymin > tmin) tmin = tymin;
+    if (tymax < tmax) tmax = tymax;
+    const float tzmin = fmul(fsub(nz, o.z), inv.z), tzmax = fmul(fsub(fz, o.z), inv.z);
+    if ((tmin > tzmax) || (tzmin > tmax)) return false;
+    if (tzmin > tmin) tmin = tzmin;
+    if (tzmax < tmax) tmax = tzmax;
+    return tmax > 0.0f;
+}
+
+// The list's step for instance k (object ray, root clip, skip rule, walk) with the tree's replace
+// rule: t < best, or t == best and k above the current instance (the base scene is -1).
+template <bool COUNT, bool SHARE>
+__device__ __forceinline__ void tree_instance_step(const ClptInstances &I, int k, V3 o, V3 d, int max_visits,
+                                                   Counters &cn, int sub, int log2_k, Hit &h) {
+    const ClptInstRec &R = I.crec[k];
+    const ClptScene &M = I.meshes[R.mesh];
+    V3 lo, ld;
+    object_ray(R.w2o, o, d, lo, ld);
+    const V3 inv = mk(frcp(ld.x), frcp(ld.y), frcp(ld.z));
+    float tmin, tmax;
+    if (!root_clip(M, lo, inv, tmin, tmax)) return;
+    if (h.ref >= 0 && tmin > h.t) return;
+    const Hit hi = walk<COUNT, SHARE>(M, lo, ld, inv, tmin, max_visits, cn, sub, log2_k);
+    if (hi.ref >= 0 && (h.ref < 0 || hi.t < h.t || (hi.t == h.t && k > h.inst))) {
+        h.ref = hi.ref;
+        h.t = hi.t;
+        h.inst = k;
+    }
+}
+
+// Walk of the instance tree: at an internal node both children are tested, a child whose entry
+// lies beyond the current hit is not taken, the nearer entry is visited first (child 0 on equal
+// entries) and the other pushed with its entry; a popped entry beyond the current hit is dropped.
+// The K lanes of a shared ray hold the same hit after every walk, so they take every decision
+// together.
+template <bool COUNT, bool SHARE>
+__device__ __forceinline__ void tree_instances(const ClptInstances &I, V3 o, V3 d, int max_visits, Counters &cn,
+                                               int sub, int log2_k, Hit &h) {
+    const V3 inv = mk(frcp(d.x), frcp(d.y), frcp(d.z));
+    int2 stack[CLPT_TREE_STACK];
+    int sp = 0, ref = 0;
+    for (;;) {
+        if (ref >= 0) {
+            const float4 *N = I.tree + 4 * (size_t)ref;
+            const float4 mn0 = __ldg(N), mx0 = __ldg(N + 1), mn1 = __ldg(N + 2), mx1 = __ldg(N + 3);
+            float e0, e1;
+            const bool in0 = box_clip(mn0, mx0, o, inv, e0) && !(h.ref >= 0 && e0 > h.t);
+            const bool in1 = box_clip(mn1, mx1, o, inv, e1) && !(h.ref >= 0 && e1 > h.t);
+            if (in0 && in1) {
+                const bool first1 = e1 < e0;
+                stack[sp++] = make_int2(__float_as_int(first1 ? mn0.w : mn1.w), __float_as_int(first1 ? e0 : e1));
+                ref = __float_as_int(first1 ? mn1.w : mn0.w);
+                continue;
+            }
+            if (in0 || in1) {
+                ref = __float_as_int(in0 ? mn0.w : mn1.w);
+                continue;
+            }
+        } else {
+            tree_instance_step<COUNT, SHARE>(I, -1 - ref, o, d, max_visits, cn, sub, log2_k, h);
+        }
+        bool found = false;
+        while (sp > 0) {
+            const int2 e = stack[--sp];
+            if (h.ref >= 0 && __int_as_float(e.y) > h.t) continue;
+            ref = e.x;
+            found = true;
+            break;
+        }
+        if (!found) break;
+    }
+}
+
 // Closest hit in the base scene and then in every instance, in array order.  An instance is
 // skipped when a hit exists and the ray enters the instance's root box beyond it; a later tree's
 // hit replaces the current one at t <= best (the later tree wins ties, like the later triangle at
-// kernel.cl:344).  INST = false is closest_hit itself.
-template <bool COUNT, bool SHARE, bool INST>
+// kernel.cl:344).  INST = 0 is closest_hit itself, 2 walks the instance tree instead of the list.
+template <bool COUNT, bool SHARE, int INST>
 __device__ __forceinline__ Hit scene_hit(const ClptScene &S, const ClptInstances &I, V3 o, V3 d, int max_visits,
                                          Counters &cn, int sub, int log2_k) {
     Hit h = closest_hit<COUNT, SHARE>(S, o, d, max_visits, cn, sub, log2_k);
-    if (INST) {
+    if (INST == 1) {
         h.inst = -1;
         for (int k = 0; k < I.count; k++) {
             const ClptInstanceRec &R = I.rec[k];
@@ -402,6 +486,10 @@ __device__ __forceinline__ Hit scene_hit(const ClptScene &S, const ClptInstances
                 h.inst = k;
             }
         }
+    }
+    if (INST == 2) {
+        h.inst = -1;
+        tree_instances<COUNT, SHARE>(I, o, d, max_visits, cn, sub, log2_k, h);
     }
     return h;
 }
@@ -454,8 +542,8 @@ __device__ __forceinline__ V3 hit_normal(const ClptScene &S, const Hit &h, V3 o,
 // differently from its own mesh: normalize is not idempotent in fp32, about a third of unit
 // vectors move by an ulp when normalised again.)
 template <bool COUNT>
-__device__ __forceinline__ V3 instance_normal(const ClptInstanceRec &R, const Hit &h, V3 lo, V3 ld, Counters &cn) {
-    const ClptScene &S = R.mesh;
+__device__ __forceinline__ V3 instance_normal(const float *a, const ClptScene &S, const Hit &h, V3 lo, V3 ld,
+                                              Counters &cn) {
     const int prim = __float_as_int(__ldg(&S.tri[3 * (size_t)h.ref].w));
     V3 m;
     if (__ldg(&S.flat_n[prim].w) != 0.0f) {
@@ -463,20 +551,25 @@ __device__ __forceinline__ V3 instance_normal(const ClptInstanceRec &R, const Hi
     } else {
         m = vcross(xyz(__ldg(S.tri + 3 * (size_t)h.ref + 1)), xyz(__ldg(S.tri + 3 * (size_t)h.ref + 2)));
     }
-    const float *a = R.w2o;
     return vnormalize(mk(fadd(fadd(fmul(a[0], m.x), fmul(a[4], m.y)), fmul(a[8], m.z)),
                          fadd(fadd(fmul(a[1], m.x), fmul(a[5], m.y)), fmul(a[9], m.z)),
                          fadd(fadd(fmul(a[2], m.x), fmul(a[6], m.y)), fmul(a[10], m.z))));
 }
 
-template <bool COUNT, bool INST>
+template <bool COUNT, int INST>
 __device__ __forceinline__ V3 shading_normal(const ClptScene &S, const ClptInstances &I, const Hit &h, V3 o, V3 d,
                                              Counters &cn) {
-    if (INST && h.inst >= 0) {
+    if (INST == 1 && h.inst >= 0) {
         const ClptInstanceRec &R = I.rec[h.inst];
         V3 lo, ld;
         object_ray(R.w2o, o, d, lo, ld);
-        return instance_normal<COUNT>(R, h, lo, ld, cn);
+        return instance_normal<COUNT>(R.w2o, R.mesh, h, lo, ld, cn);
+    }
+    if (INST == 2 && h.inst >= 0) {
+        const ClptInstRec &R = I.crec[h.inst];
+        V3 lo, ld;
+        object_ray(R.w2o, o, d, lo, ld);
+        return instance_normal<COUNT>(R.w2o, I.meshes[R.mesh], h, lo, ld, cn);
     }
     return hit_normal<COUNT>(S, h, o, d, cn);
 }
@@ -499,14 +592,21 @@ __device__ __forceinline__ void write_aov(const ClptScene &S, const ClptFrame &F
 
 // AOVs of a first hit: an instance hit reports its primitive shifted by the instance's offset and
 // u, v in its own triangle (the object-space ray); t is the world t either way.
-template <bool COUNT, bool INST>
+template <bool COUNT, int INST>
 __device__ __forceinline__ void write_hit_aov(const ClptScene &S, const ClptInstances &I, const ClptFrame &F,
                                               const Hit &h, V3 o, V3 d, int x, int y) {
-    if (INST && h.ref >= 0 && h.inst >= 0) {
+    if (INST == 1 && h.ref >= 0 && h.inst >= 0) {
         const ClptInstanceRec &R = I.rec[h.inst];
         V3 lo, ld;
         object_ray(R.w2o, o, d, lo, ld);
         write_aov<COUNT>(R.mesh, F, h, lo, ld, x, y, R.prim_offset);
+        return;
+    }
+    if (INST == 2 && h.ref >= 0 && h.inst >= 0) {
+        const ClptInstRec &R = I.crec[h.inst];
+        V3 lo, ld;
+        object_ray(R.w2o, o, d, lo, ld);
+        write_aov<COUNT>(I.meshes[R.mesh], F, h, lo, ld, x, y, R.prim_offset);
         return;
     }
     write_aov<COUNT>(S, F, h, o, d, x, y);

@@ -132,7 +132,18 @@ struct {
     std::vector<std::unique_ptr<InstanceMesh>> inst_meshes;
     std::vector<CLInstance> instances;
     DevBuf<ClptInstanceRec> inst_table;
-    bool inst_table_stale = true;
+    bool inst_table_stale = true; // the table of the current traversal (list or compact records)
+    // instance tree (CLPT_INSTANCES_TREE): compact records, the mesh table, the nodes; rebuilt
+    // before the next frame after CLSetInstances or a change of the mesh set
+    int traversal = CLPT_INSTANCES_LIST;
+    std::vector<ClptInstRec> inst_compact_host;
+    DevBuf<ClptInstRec> inst_compact;
+    DevBuf<ClptScene> mesh_table;
+    DevBuf<float4> tree_nodes;
+    DevBuf<unsigned char> tree_scratch;
+    bool mesh_table_stale = true, tree_stale = true, tree_timed = false;
+    cudaEvent_t ev_tree[2] = {};
+    float last_tree_ms = 0;
 
     float cam[16] = { 0 };
 
@@ -476,14 +487,74 @@ void p2p_setup() {
 
 void release_read_pipeline();
 
-// The instances of the next frame: the device table, written again if anything it holds changed.
+// f(k, offset) for every instance: offset = the base scene's primitives + those of the instances
+// before k, summed in 64 bits; ids that would pass INT32_MAX are rejected.
+template <typename F>
+void for_each_prim_offset(F &&f) {
+    long long offset = St.scene.n_prims;
+    for (size_t k = 0; k < St.instances.size(); k++) {
+        const int prims = St.inst_meshes[St.instances[k].mesh]->scene.n_prims;
+        if (offset + prims - 1 > (long long)INT32_MAX) {
+            fprintf(stderr, "CLExecute: the primitive ids of instance %zu would pass INT32_MAX (%lld + %d primitives)\n",
+                    k, offset, prims);
+            exit(EXIT_FAILURE);
+        }
+        f(k, (int)offset);
+        offset += prims;
+    }
+}
+
+// The compact records, the mesh table and the tree of the current instances, each written again
+// if anything it depends on changed.  The build is enqueued on the library's stream.
+void ensure_instance_tree() {
+    const size_t n = St.instances.size();
+    if (St.inst_table_stale) {
+        St.inst_compact_host.resize(n);
+        for_each_prim_offset([](size_t k, int offset) {
+            ClptInstRec &r = St.inst_compact_host[k];
+            static_assert(sizeof(ClptInstRec) == sizeof(CLInstance), "the compact record is CLInstance's layout");
+            memcpy(&r, &St.instances[k], sizeof(r));
+            r.prim_offset = offset;
+        });
+        St.inst_compact.reserve(n);
+        CU(cudaMemcpyAsync(St.inst_compact.ptr, St.inst_compact_host.data(), n * sizeof(ClptInstRec),
+                           cudaMemcpyHostToDevice, St.stream));
+        St.inst_table_stale = false;
+    }
+    if (St.mesh_table_stale) {
+        std::vector<ClptScene> meshes;
+        for (auto &m : St.inst_meshes) meshes.push_back(m->scene);
+        St.mesh_table.upload(meshes.data(), meshes.size(), St.stream);
+        St.mesh_table_stale = false;
+    }
+    if (St.tree_stale) {
+        St.tree_nodes.reserve(4 * (n > 1 ? n - 1 : 1)); // four float4s a node
+        St.tree_scratch.reserve(clpt_instance_tree_scratch_bytes((int)n));
+        CU(cudaEventRecord(St.ev_tree[0], St.stream));
+        clpt_build_instance_tree(St.inst_compact.ptr, St.mesh_table.ptr, (int)n, St.tree_nodes.ptr,
+                                 St.tree_scratch.ptr, St.stream);
+        CU(cudaEventRecord(St.ev_tree[1], St.stream));
+        St.tree_stale = false;
+        St.tree_timed = true;
+    }
+}
+
+// The instances of the next frame: the device table of the current traversal, written again if
+// anything it holds changed.
 ClptInstances current_instances() {
-    ClptInstances I = { nullptr, 0 };
+    ClptInstances I = { nullptr, 0, nullptr, nullptr, nullptr };
     if (St.instances.empty()) return I;
+    I.count = (int)St.instances.size();
+    if (St.traversal == CLPT_INSTANCES_TREE) {
+        ensure_instance_tree();
+        I.crec = St.inst_compact.ptr;
+        I.meshes = St.mesh_table.ptr;
+        I.tree = St.tree_nodes.ptr;
+        return I;
+    }
     if (St.inst_table_stale) {
         std::vector<ClptInstanceRec> recs(St.instances.size());
-        int offset = St.scene.n_prims;
-        for (size_t k = 0; k < recs.size(); k++) {
+        for_each_prim_offset([&recs](size_t k, int offset) {
             const CLInstance &in = St.instances[k];
             ClptInstanceRec &r = recs[k];
             memset(&r, 0, sizeof(r));
@@ -491,13 +562,11 @@ ClptInstances current_instances() {
             r.material = in.material;
             r.prim_offset = offset;
             r.mesh = St.inst_meshes[in.mesh]->scene;
-            offset += r.mesh.n_prims;
-        }
+        });
         St.inst_table.upload(recs.data(), recs.size(), St.stream);
         St.inst_table_stale = false;
     }
     I.rec = St.inst_table.ptr;
-    I.count = (int)St.instances.size();
     return I;
 }
 
@@ -512,7 +581,12 @@ void release_instance_meshes() {
     St.inst_meshes.clear();
     St.instances.clear();
     St.inst_table.release();
-    St.inst_table_stale = true;
+    St.inst_compact.release();
+    St.inst_compact_host = {};
+    St.mesh_table.release();
+    St.tree_nodes.release();
+    St.tree_scratch.release();
+    St.inst_table_stale = St.mesh_table_stale = St.tree_stale = true;
 }
 
 // A device-built tree and its mesh as fresh host lists (CLDownloadKd, CLDownloadInstanceKd).
@@ -924,6 +998,7 @@ void CLInit(const char *kernel_filename, const char *kernel_name) {
     CU(cudaEventCreate(&St.ev_stop));
     for (auto &e : St.ev_user) CU(cudaEventCreate(&e));
     for (auto &e : St.ev_build) CU(cudaEventCreate(&e));
+    for (auto &e : St.ev_tree) CU(cudaEventCreate(&e));
     memset(St.cam, 0, sizeof(St.cam));
     clpt_pack_alloc = pinned_alloc; // the packed scene is staged in page-locked memory
     clpt_pack_free = pinned_free;
@@ -975,6 +1050,9 @@ void CLTerminate(void) {
     CU(cudaEventDestroy(St.ev_stop));
     for (auto &e : St.ev_user) CU(cudaEventDestroy(e));
     for (auto &e : St.ev_build) CU(cudaEventDestroy(e));
+    for (auto &e : St.ev_tree) CU(cudaEventDestroy(e));
+    St.tree_timed = false;
+    St.traversal = CLPT_INSTANCES_LIST; // the default again after the next CLInit
     CU(cudaStreamDestroy(St.stream));
     St.stream = nullptr;
     St.have_scene = St.have_image = St.headless = false;
@@ -1162,6 +1240,7 @@ int CLAddInstanceMesh(const void *verts, size_t vert_bytes, const void *tris, si
     set_scene_mesh(M->scene, M->layout, M->corners, M->norms);
     M->scene.n_prims = n_prims;
     St.inst_meshes.push_back(std::move(M));
+    St.mesh_table_stale = St.tree_stale = true;
     return (int)St.inst_meshes.size() - 1;
 }
 
@@ -1173,8 +1252,9 @@ void CLSetInstances(const CLInstance *instances, size_t bytes) {
         exit(EXIT_FAILURE);
     }
     const size_t n = bytes / sizeof(CLInstance);
-    if (n > CLPT_MAX_INSTANCES) {
-        fprintf(stderr, "CLSetInstances: %zu instances, at most %d\n", n, CLPT_MAX_INSTANCES);
+    const int cap = St.traversal == CLPT_INSTANCES_TREE ? CLPT_MAX_TREE_INSTANCES : CLPT_MAX_INSTANCES;
+    if (n > (size_t)cap) {
+        fprintf(stderr, "CLSetInstances: %zu instances, at most %d\n", n, cap);
         exit(EXIT_FAILURE);
     }
     if (n && !instances) FATAL("CLSetInstances: NULL instances");
@@ -1193,7 +1273,47 @@ void CLSetInstances(const CLInstance *instances, size_t bytes) {
         }
     }
     St.instances.assign(instances, instances + n);
-    St.inst_table_stale = true;
+    St.inst_table_stale = St.tree_stale = true;
+}
+
+void CLSetInstanceTraversal(int traversal) {
+    require_init("CLSetInstanceTraversal");
+    if (traversal != CLPT_INSTANCES_LIST && traversal != CLPT_INSTANCES_TREE) {
+        fprintf(stderr, "CLSetInstanceTraversal: %d is neither CLPT_INSTANCES_LIST (0) nor CLPT_INSTANCES_TREE (1)\n",
+                traversal);
+        exit(EXIT_FAILURE);
+    }
+    if (traversal == CLPT_INSTANCES_LIST && St.instances.size() > CLPT_MAX_INSTANCES) {
+        fprintf(stderr, "CLSetInstanceTraversal: %zu instances are set; the list takes at most %d\n",
+                St.instances.size(), CLPT_MAX_INSTANCES);
+        exit(EXIT_FAILURE);
+    }
+    if (traversal != St.traversal) St.inst_table_stale = true;
+    St.traversal = traversal;
+}
+
+int CLInstanceTraversal(void) { return St.traversal; }
+
+size_t CLDebugReadInstanceTree(void *dst, size_t bytes) {
+    require_init("CLDebugReadInstanceTree");
+    const size_t n = St.instances.size();
+    if (n == 0) return 0;
+    if (St.traversal != CLPT_INSTANCES_TREE) St.inst_table_stale = true; // the compact records are written now
+    ensure_instance_tree();
+    if (St.traversal != CLPT_INSTANCES_TREE) St.inst_table_stale = true; // ... and the list's table next frame
+    const size_t have = (n > 1 ? n - 1 : 1) * 4 * sizeof(float4);
+    CU(cudaStreamSynchronize(St.stream));
+    if (dst && bytes >= have) CU(cudaMemcpy(dst, St.tree_nodes.ptr, have, cudaMemcpyDeviceToHost));
+    return have;
+}
+
+void CLLastInstanceBuildMs(float *ms) {
+    if (St.tree_timed) {
+        CU(cudaEventSynchronize(St.ev_tree[1]));
+        CU(cudaEventElapsedTime(&St.last_tree_ms, St.ev_tree[0], St.ev_tree[1]));
+        St.tree_timed = false;
+    }
+    if (ms) *ms = St.last_tree_ms;
 }
 
 void CLClearInstanceMeshes(void) {

@@ -39,8 +39,9 @@ __host__ __device__ inline void warp_tile_dims(int log2_ppw, int &tw, int &th) {
     th = 1 << (log2_ppw >> 1);
 }
 
-// INST: the instanced variant (clpt_trace.cuh: scene_hit), launched only while instances exist.
-template <int MODE, bool COUNT, bool SHARE, bool INST>
+// INST: 0 no instances, 1 the instance list, 2 the instance tree (clpt_trace.cuh: scene_hit); the
+// instanced variants are launched only while instances exist.
+template <int MODE, bool COUNT, bool SHARE, int INST>
 __device__ __forceinline__ V3 trace_sample(const ClptScene &S, const ClptInstances &I, const ClptFrame &F, int x, int y, unsigned pixel,
                                            unsigned sample, bool aov, Counters &cn_in, int sub, int log2_k) {
     Counters scratch = { 0, 0, 0, 0, 0, 0 };
@@ -61,7 +62,8 @@ __device__ __forceinline__ V3 trace_sample(const ClptScene &S, const ClptInstanc
             int kind = 0;
             if (S.n_materials > 0) {
                 int m;
-                if (INST && h.inst >= 0) m = I.rec[h.inst].material;
+                if (INST == 1 && h.inst >= 0) m = I.rec[h.inst].material;
+                else if (INST == 2 && h.inst >= 0) m = I.crec[h.inst].material;
                 else m = S.tri_material ? __ldg(S.tri_material + __float_as_int(__ldg(&S.tri[3 * (size_t)h.ref].w))) : 0;
                 if (m < 0 || m >= S.n_materials) m = 0;
                 const ClptMaterial *mp = S.materials + m;
@@ -131,9 +133,9 @@ __device__ __forceinline__ void group_sync(int log2_g, int group) {
 }
 
 // VARIANT 0: compiled for 8 resident blocks per SM (engine 1).  1: the same code for
-// CLPT_FAT_MIN_BLOCKS (engine 2, trees with fat leaves).  INST: walks the instances of I after the
-// base scene; the variants without it ignore I and are the kernels of a frame without instances.
-template <int MODE, bool COUNT, int VARIANT, bool INST>
+// CLPT_FAT_MIN_BLOCKS (engine 2, trees with fat leaves).  INST 1 (list) or 2 (tree): walks the
+// instances of I after the base scene; INST 0 ignores I and is the kernel of a frame without instances.
+template <int MODE, bool COUNT, int VARIANT, int INST>
 __global__ void __launch_bounds__(256, VARIANT == 1 ? CLPT_FAT_MIN_BLOCKS : CLPT_MIN_BLOCKS)
 render_kernel(const __grid_constant__ ClptScene S, const __grid_constant__ ClptFrame F,
               const __grid_constant__ ClptInstances I) {
@@ -357,7 +359,7 @@ __global__ void flag_barrier_kernel(const __grid_constant__ ClptFlagPeers peers,
     } while ((int)(seen - epoch) < 0);
 }
 
-template <int MODE, bool INST>
+template <int MODE, int INST>
 void launch_variant(const ClptScene &scene, const ClptFrame &frame, const ClptInstances &inst, unsigned grid,
                     cudaStream_t stream) {
     const bool fat = (frame.flags & CLPT_F_FAT) != 0;
@@ -373,8 +375,9 @@ void launch_variant(const ClptScene &scene, const ClptFrame &frame, const ClptIn
 template <int MODE>
 void launch_mode(const ClptScene &scene, const ClptFrame &frame, const ClptInstances &inst, unsigned grid,
                  cudaStream_t stream) {
-    if (inst.count > 0) launch_variant<MODE, true>(scene, frame, inst, grid, stream);
-    else launch_variant<MODE, false>(scene, frame, inst, grid, stream);
+    if (inst.count > 0 && inst.tree) launch_variant<MODE, 2>(scene, frame, inst, grid, stream);
+    else if (inst.count > 0) launch_variant<MODE, 1>(scene, frame, inst, grid, stream);
+    else launch_variant<MODE, 0>(scene, frame, inst, grid, stream);
 }
 
 } // namespace
@@ -445,5 +448,5 @@ void clpt_launch_pack_rgba8(const float4 *src, uchar4 *dst, size_t n, cudaStream
 }
 
 const void *clpt_render_kernel_symbol(void) {
-    return reinterpret_cast<const void *>(&render_kernel<0, false, 0, false>);
+    return reinterpret_cast<const void *>(&render_kernel<0, false, 0, 0>);
 }

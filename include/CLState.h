@@ -188,10 +188,43 @@ typedef struct CLInstance {      /* 64 bytes */
 int CLAddInstanceMesh(const void *verts, size_t vert_bytes, const void *tris, size_t tri_bytes,
                       const void *norms, size_t norm_bytes);
 /* The instances of the next frames (replaces the previous set; NULL / 0 = none).  Per frame
- * this is the only upload a rigid motion needs.  At most CLPT_MAX_INSTANCES. */
+ * this is the only upload a rigid motion needs.  At most CLPT_MAX_INSTANCES under the list
+ * traversal, CLPT_MAX_TREE_INSTANCES under the tree (CLSetInstanceTraversal). */
 void CLSetInstances(const CLInstance *instances, size_t bytes);
 void CLClearInstanceMeshes(void);              /* frees every instance mesh and clears the instances */
 void CLDownloadInstanceKd(int mesh, kd *out);  /* an instance mesh's tree, like CLDownloadKd */
+/* Instance traversal, from the next CLExecute on.  CLPT_INSTANCES_LIST (the default) is the walk
+ * over the array described above, for at most CLPT_MAX_INSTANCES.  CLPT_INSTANCES_TREE walks a
+ * tree over the instances' world boxes, built on the device whenever the instances or the mesh
+ * set change (a base-scene change only moves the primitive ids), and takes up to
+ * CLPT_MAX_TREE_INSTANCES:
+ *   - World box of instance k: A^-1 (adjugate over determinant) and -A^-1 b in float64, the eight
+ *     corners of the mesh's root box mapped through them, their min and max, each side padded
+ *     outward by 2^-12 * the largest extent + 2^-20 * the largest |coordinate| and rounded
+ *     outward to fp32.  A zero determinant or a non-finite inverse gives the box +-FLT_MAX.
+ *   - Tree: a linear BVH (Karras 2012) over keys morton30(centroid quantised to 10 bits per axis
+ *     over the centroids' bounds) << 20 | k; the same instances give the same nodes on every GPU.
+ *   - Walk: at a node both children's boxes are tested with the root clip's slab test; a child
+ *     whose entry lies beyond the current hit is not taken, the nearer one is visited first
+ *     (child 0 on equal entries), and a deferred child whose entry has meanwhile fallen behind
+ *     the hit is dropped.  At an instance the list's step runs unchanged (object ray, root clip,
+ *     skip rule, walk, shading, ids, material), except that its hit replaces the current one when
+ *     t < best, or t == best and k is greater than the current instance (the base scene is -1).
+ *   - When no instance's hit lies within rounding of the entry of an instance's world box, the
+ *     tree renders the list's frame bit for bit; the work counters differ (fewer instances are
+ *     walked; tree nodes are not counted).
+ * Rejected with a message and exit(EXIT_FAILURE): another value; the list while more than
+ * CLPT_MAX_INSTANCES instances are set.  Either traversal rejects, at CLExecute, instances
+ * whose primitive ids would pass INT32_MAX. */
+enum { CLPT_INSTANCES_LIST = 0, CLPT_INSTANCES_TREE = 1 };
+#define CLPT_MAX_TREE_INSTANCES (1 << 20)
+void CLSetInstanceTraversal(int traversal);
+int CLInstanceTraversal(void);
+/* Test hook: the node array of the instance tree (64 bytes a node, max(n - 1, 1) nodes; layout in
+ * DESIGN.md "Instance tree"), built first if stale.  Returns the size in bytes (0 without
+ * instances); copies when dst is large enough. */
+size_t CLDebugReadInstanceTree(void *dst, size_t bytes);
+void CLLastInstanceBuildMs(float *ms); /* device time of the last instance-tree build */
 /* mode, depth (= bounces + 1; the reference passes 2, src/kernel.cl:468),
  * samples per pixel per frame, RNG seed, CLPT_FLAG_* */
 void CLSetRenderParams(int mode, int depth, int spp, unsigned int seed, int flags);
