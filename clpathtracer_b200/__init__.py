@@ -36,7 +36,7 @@ KDNODE_DTYPE = np.dtype(
 the plane, b = axis, c[0:2] = children.  For a leaf: a = first slot in
 tri_indices, b = triangle count, c[0:6] = ropes."""
 
-MODE_NORMAL, MODE_MIRROR, MODE_PATH = 0, 1, 2
+MODE_NORMAL, MODE_MIRROR, MODE_PATH, MODE_PATH_NEE = 0, 1, 2, 3
 READ_FLOAT4, READ_RGBA8 = 0, 1
 FLAG_JITTER, FLAG_ACCUMULATE, FLAG_COUNTERS = 1, 2, 4
 
@@ -85,6 +85,13 @@ INSTANCE_TREE_DTYPE = np.dtype(
 )
 """Instance-tree node (CLDebugReadInstanceTree): the boxes of child 0 and child 1 and their
 references; ref >= 0 is an internal node, ref < 0 is instance -1 - ref.  Node 0 is the root."""
+
+
+EMITTER_DTYPE = np.dtype({"names": ["v0", "prim", "e1", "pa", "e2", "pad0", "n", "pad1"],
+                          "formats": [("<f4", 3), "<i4", ("<f4", 3), "<f4", ("<f4", 3), "<f4", ("<f4", 3), "<f4"],
+                          "offsets": [0, 12, 16, 28, 32, 44, 48, 60], "itemsize": 64})
+"""Emitter record (CLDebugReadEmitters): v0, primitive id, e1 = v1 - v0, the emitter's area pdf
+(selection probability / area), e2 = v2 - v0, and its flat normal."""
 
 
 class CLInstance(C.Structure):
@@ -162,6 +169,7 @@ def lib() -> C.CDLL:
         "CLClearInstanceMeshes": (None, []), "CLDownloadInstanceKd": (None, [i, C.POINTER(KD)]),
         "CLSetInstanceTraversal": (None, [i]), "CLInstanceTraversal": (i, []),
         "CLDebugReadInstanceTree": (sz, [vp, sz]), "CLLastInstanceBuildMs": (None, [C.POINTER(f)]),
+        "CLDebugReadEmitters": (sz, [i, vp, sz]),
         "CLUpdateVertices": (None, [sz, vp, sz]), "CLRebuildMeshes": (None, []),
         "CLDeleteImage": (None, []), "CLCreateImage": (None, [u]), "CLExecute": (None, [i, i]),
         "CLSelectDevice": (None, [i]), "CLSetRenderParams": (None, [i, i, i, u, i]),
@@ -426,6 +434,20 @@ class Renderer:
         out = np.zeros(n // 64, dtype=INSTANCE_TREE_DTYPE)
         if n:
             self.L.CLDebugReadInstanceTree(out.ctypes.data, n)
+        return out
+
+    def read_emitters(self) -> dict:
+        """The emitter table of mode 3 (CLDebugReadEmitters), built first if stale: header uint64[2]
+        (emitter count n, total weight Q), records EMITTER_DTYPE[n], cdf uint64[n] (exclusive prefix
+        sums of the integer weights), map int32[primitives] (emitter of each base primitive or -1)."""
+        out = {}
+        for which, name, dtype in ((0, "header", np.uint64), (1, "records", EMITTER_DTYPE), (2, "cdf", np.uint64),
+                                   (3, "map", np.int32)):
+            n = self.L.CLDebugReadEmitters(which, None, 0)
+            a = np.zeros(n // np.dtype(dtype).itemsize, dtype=dtype)
+            if n:
+                self.L.CLDebugReadEmitters(which, a.ctypes.data, n)
+            out[name] = a
         return out
 
     def instance_build_ms(self) -> float:

@@ -22,7 +22,7 @@ LIB = PKG / "libclpt.so"
 
 HOST_C = ["host/hostlist.c", "host/vecmath.c", "host/kd_build.c", "host/model_io.c", "host/frame_sched.c"]
 HOST_CXX = ["cuda/scene_pack.cpp"]
-CUDA = ["cuda/render_kernel.cu", "cuda/kd_build_gpu.cu", "cuda/instance_tree.cu", "cuda/gl_interop.cu",
+CUDA = ["cuda/render_kernel.cu", "cuda/kd_build_gpu.cu", "cuda/instance_tree.cu", "cuda/emitters.cu", "cuda/gl_interop.cu",
         "cuda/clstate.cu", "cuda/clhandler.cu"]
 
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
@@ -107,6 +107,9 @@ def build_oracle() -> None:
     # ... and the instance tree's (oracle/oracle_instance_tree_py.py)
     _run(["gcc", "-std=c11", "-O2", "-fPIC", "-ffp-contract=off", "-fopenmp", "-w", "-shared", "-o",
           str(ROOT / "oracle" / "liboracle_instance_tree.so"), str(ROOT / "oracle" / "oracle_instance_tree.c"), "-lm"])
+    # ... and light sampling's (oracle/oracle_nee_py.py)
+    _run(["gcc", "-std=c11", "-O2", "-fPIC", "-ffp-contract=off", "-fopenmp", "-w", "-shared", "-o",
+          str(ROOT / "oracle" / "liboracle_nee.so"), str(ROOT / "oracle" / "oracle_nee.c"), "-lm"])
 
 
 if __name__ == "__main__":

@@ -104,6 +104,25 @@ size_t clpt_instance_tree_scratch_bytes(int n);
 void clpt_build_instance_tree(const ClptInstRec *recs, const ClptScene *meshes, int n, float4 *nodes,
                               void *scratch, cudaStream_t stream);
 
+// Emitter table of the base scene (mode 3, DESIGN.md "Light sampling (mode 3)"): the primitives
+// listed by a leaf whose material emits, in ascending primitive id.  Record i is four float4s,
+// {v0, prim bits}, {e1, area pdf}, {e2, 0}, {flat normal, 0}; cdf[i] is the exclusive uint64 prefix
+// sum of the integer weights; map[prim] = i or -1; header = {emitter count, total weight Q}.  The
+// counts stay on the device: the table is built without a host round trip.
+struct ClptEmitters {
+    const float4 *rec;
+    const unsigned long long *cdf;
+    const int *map;
+    const unsigned long long *header;
+};
+
+// emitters.cu: builds the table of the scene S (materials and tri_material included) in stream
+// order.  Capacities: rec 4 * max(n_prims, 1) float4s, cdf n_prims + 1, map max(n_prims, 1),
+// header 2; `scratch` holds clpt_emitter_scratch_bytes(n_prims) bytes.
+size_t clpt_emitter_scratch_bytes(int n_prims);
+void clpt_build_emitters(const ClptScene &S, float4 *rec, unsigned long long *cdf, int *map,
+                         unsigned long long *header, void *scratch, cudaStream_t stream);
+
 #define CLPT_MAX_PEERS 8
 
 struct ClptFrame {
@@ -169,9 +188,9 @@ enum { CLPT_F_JITTER = 1, CLPT_F_ACCUMULATE = 2, CLPT_F_COUNTERS = 4, CLPT_F_REV
        CLPT_F_FAT = 0x200 /* internal: engine 2, the kernel compiled for fewer resident blocks (fat leaves) */ };
 
 // render_kernel.cu
-// inst.count > 0 launches the instanced variant of the render kernel
-void clpt_launch_render(const ClptScene &scene, const ClptFrame &frame, const ClptInstances &inst, int sm_count,
-                        cudaStream_t stream);
+// inst.count > 0 launches the instanced variant of the render kernel; `emit` is read in mode 3 only
+void clpt_launch_render(const ClptScene &scene, const ClptFrame &frame, const ClptInstances &inst,
+                        const ClptEmitters &emit, int sm_count, cudaStream_t stream);
 int clpt_render_blocks_per_sm(int engine);          // resident 256-thread blocks per SM the render kernel is compiled for
 int clpt_render_block_rows(const ClptFrame &frame); // rows of blocks the launch will walk (size of row_cost)
 void clpt_launch_deinterleave(const float4 *gathered, float4 *image, int width, int height,

@@ -494,6 +494,120 @@ __device__ __forceinline__ Hit scene_hit(const ClptScene &S, const ClptInstances
     return h;
 }
 
+// ---- shadow rays (mode 3, DESIGN.md "Light sampling (mode 3)") ------------------------------
+// Any-hit test of a leaf's triangle run: true when a triangle is accepted (the hit test above) with
+// t < t_max.  The whole run is tested, so the test count does not depend on where the accepted
+// triangle sits; with SHARE the K lanes of a ray each test every K-th triangle and OR the results.
+template <bool COUNT, bool SHARE>
+__device__ __forceinline__ bool triangle_any(const float4 *__restrict__ tri, int first, int count, int sub,
+                                             int log2_k, V3 o, V3 d, float t_max, Counters &cn) {
+    bool hit = false;
+    for (int i = first + sub; i < first + count; i += 1 << log2_k) {
+        const float4 b = __ldg(tri + 3 * (size_t)i + 1);
+        const float4 c = __ldg(tri + 3 * (size_t)i + 2);
+        if (COUNT) cn.tris++;
+        const V3 e1 = xyz(b), e2 = xyz(c);
+        const V3 pvec = vcross(d, e2);
+        const float det = vdot(e1, pvec);
+        if (det < 0.0f) continue;
+        const float idet = frcp(det);
+        const V3 tvec = vsub(o, xyz(__ldg(tri + 3 * (size_t)i)));
+        const float u = fmul(vdot(tvec, pvec), idet);
+        if (u < 0.0f || u > 1.0f) continue;
+        const V3 qvec = vcross(tvec, e1);
+        const float v = fmul(vdot(d, qvec), idet);
+        if (v < 0.0f || fadd(u, v) > 1.0f) continue;
+        const float t = fmul(vdot(e2, qvec), idet);
+        if (t > 0.0f && t < t_max) hit = true;
+    }
+    if (SHARE) {
+        const int lane = threadIdx.x & 31;
+        const unsigned mask = ((1u << (1 << log2_k)) - 1u) << (lane & ~((1 << log2_k) - 1));
+        for (int off = 1; off < (1 << log2_k); off <<= 1) hit |= __shfl_xor_sync(mask, hit ? 1 : 0, off) != 0;
+    }
+    return hit;
+}
+
+// Any-hit walk of one tree from its root clip: ends without a hit at a leaf whose entry lies beyond
+// t_max or when the ray leaves the tree, occluded after the first leaf that accepted a triangle or
+// when the rope-hop budget runs out.
+template <bool COUNT, bool SHARE>
+__device__ __forceinline__ bool any_walk(const ClptScene &S, V3 o, V3 d, float t_max, int max_visits, Counters &cn_in,
+                                         int sub, int log2_k) {
+    Counters scratch = { 0, 0, 0, 0, 0, 0 };
+    Counters &cn = (SHARE && sub != 0) ? scratch : cn_in;
+    const V3 inv = mk(frcp(d.x), frcp(d.y), frcp(d.z));
+    float tmin, tmax;
+    if (!root_clip(S, o, inv, tmin, tmax) || tmin > t_max) return false;
+    V3 p1 = o;
+    if (tmin > 0.0f) p1 = vadd(p1, vscale(d, tmin));
+    int visits_left = max_visits > 1 ? max_visits : 1;
+    const uint2 *__restrict__ nodes = S.nodes;
+    uint2 n = __ldg(nodes + (COUNT ? 0 : start_node(S, p1)));
+    for (;;) {
+        n = descend<COUNT>(nodes, n, p1, cn);
+        if (COUNT) cn.leaves++;
+        const float4 *L = S.leaves + 4 * (size_t)n.x;
+        const float4 lmin = __ldg(L), lmax = __ldg(L + 1);
+        if (leaf_entry(lmin, lmax, o, inv) > t_max) return false;
+        int far;
+        leaf_exit(lmin, lmax, o, inv, tmax, far);
+        if (triangle_any<COUNT, SHARE>(S.tri, __float_as_int(lmin.w), __float_as_int(lmax.w), sub, log2_k, o, d, t_max,
+                                       cn_in))
+            return true;
+        if (leave_leaf<COUNT>(nodes, L, far, o, d, tmax, p1, n, visits_left, cn)) return visits_left <= 0;
+    }
+}
+
+// A shadow ray (one ray of the counters): true when a triangle of the base scene or of an instance
+// is accepted with 0 < t < t_max.  Instances: the list in order, or the instance tree with child 0
+// first and child 1 deferred; a box or root clip whose entry lies beyond t_max is not entered.
+// Visibility is an OR, so the order changes only the work counters, never the answer.
+template <bool COUNT, bool SHARE, int INST>
+__device__ __forceinline__ bool occluded(const ClptScene &S, const ClptInstances &I, V3 o, V3 d, float t_max,
+                                         int max_visits, Counters &cn_in, int sub, int log2_k) {
+    if (COUNT && !(SHARE && sub != 0)) cn_in.rays++;
+    if (any_walk<COUNT, SHARE>(S, o, d, t_max, max_visits, cn_in, sub, log2_k)) return true;
+    if (INST == 1) {
+        for (int k = 0; k < I.count; k++) {
+            V3 lo, ld;
+            object_ray(I.rec[k].w2o, o, d, lo, ld);
+            if (any_walk<COUNT, SHARE>(I.rec[k].mesh, lo, ld, t_max, max_visits, cn_in, sub, log2_k)) return true;
+        }
+    }
+    if (INST == 2) {
+        const V3 inv = mk(frcp(d.x), frcp(d.y), frcp(d.z));
+        int stack[CLPT_TREE_STACK];
+        int sp = 0, ref = 0;
+        for (;;) {
+            if (ref >= 0) {
+                const float4 *N = I.tree + 4 * (size_t)ref;
+                const float4 mn0 = __ldg(N), mx0 = __ldg(N + 1), mn1 = __ldg(N + 2), mx1 = __ldg(N + 3);
+                float e0, e1;
+                const bool in0 = box_clip(mn0, mx0, o, inv, e0) && !(e0 > t_max);
+                const bool in1 = box_clip(mn1, mx1, o, inv, e1) && !(e1 > t_max);
+                if (in0 && in1) {
+                    stack[sp++] = __float_as_int(mn1.w);
+                    ref = __float_as_int(mn0.w);
+                    continue;
+                }
+                if (in0 || in1) {
+                    ref = __float_as_int(in0 ? mn0.w : mn1.w);
+                    continue;
+                }
+            } else {
+                const ClptInstRec &R = I.crec[-1 - ref];
+                V3 lo, ld;
+                object_ray(R.w2o, o, d, lo, ld);
+                if (any_walk<COUNT, SHARE>(I.meshes[R.mesh], lo, ld, t_max, max_visits, cn_in, sub, log2_k)) return true;
+            }
+            if (sp == 0) break;
+            ref = stack[--sp];
+        }
+    }
+    return false;
+}
+
 // Primitive id and barycentrics of the accepted hit: hit_triangle's u and v
 // (kernel.cl:243-249) evaluated again for the winning slot.
 __device__ __forceinline__ HitDetails hit_details(const ClptScene &S, const Hit &h, V3 o, V3 d) {
@@ -629,10 +743,16 @@ __device__ __forceinline__ void philox(unsigned c[4], unsigned k0, unsigned k1) 
 }
 __device__ __forceinline__ float u01(unsigned x) { return fmul((float)(x >> 8), 0x1p-24f); }
 #define CLPT_KEY1 0x636c7074u
+// Mode 3 (oracle/oracle_nee.c): (1 - p) / pi in fp32, p = 0.0021209640721610596 the chance that
+// cosine_dir rejects all four disk tries; and the shadow ray's t_max = (dist - 1e-4) * (1 - 2^-12).
+#define CLPT_NEE_PB 0x1.45420cp-2f
+#define CLPT_NEE_TMAX_SCALE 0x1.ffep-1f
 
-// Cosine-weighted direction about n (extension; oracle_kernel.c cosine_dir).
-__device__ __forceinline__ V3 cosine_dir(V3 n, unsigned pixel, unsigned sample, unsigned bounce,
-                                         unsigned seed) {
+// Cosine-weighted direction about n (extension; oracle_kernel.c cosine_dir).  fell_back: all four
+// disk tries were rejected and the direction is n itself (mode 3 gives such a bounce no MIS weight;
+// a = b = 0 does not say it, an accepted try can land on the centre).
+__device__ __forceinline__ V3 cosine_dir(V3 n, unsigned pixel, unsigned sample, unsigned bounce, unsigned seed,
+                                         bool &fell_back) {
     float a = 0.0f, b = 0.0f;
     bool found = false;
 #pragma unroll 1
@@ -657,7 +777,12 @@ __device__ __forceinline__ V3 cosine_dir(V3 n, unsigned pixel, unsigned sample, 
     const float q = fmul(fmul(n.x, n.y), p);
     const V3 t1 = mk(fadd(1.0f, fmul(fmul(fmul(sg, n.x), n.x), p)), fmul(sg, q), fmul(-sg, n.x));
     const V3 t2 = mk(q, fadd(sg, fmul(fmul(n.y, n.y), p)), -n.y);
+    fell_back = !found;
     return vnormalize(vadd(vadd(vscale(t1, a), vscale(t2, b)), vscale(n, z)));
+}
+__device__ __forceinline__ V3 cosine_dir(V3 n, unsigned pixel, unsigned sample, unsigned bounce, unsigned seed) {
+    bool fell_back;
+    return cosine_dir(n, pixel, sample, bounce, seed, fell_back);
 }
 
 __device__ __forceinline__ V3 unproject(const float *M, V3 X) { // kernel.cl:89-94

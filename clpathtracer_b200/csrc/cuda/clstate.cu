@@ -144,6 +144,13 @@ struct {
     bool mesh_table_stale = true, tree_stale = true, tree_timed = false;
     cudaEvent_t ev_tree[2] = {};
     float last_tree_ms = 0;
+    // emitter table of the base scene (mode 3): rebuilt before the next mode-3 frame after the base
+    // scene, the materials or tri_material changed (modes 0-2 and scene uploads never build it)
+    DevBuf<float4> emit_rec;
+    DevBuf<unsigned long long> emit_cdf, emit_header;
+    DevBuf<int> emit_map;
+    DevBuf<unsigned char> emit_scratch;
+    bool emitters_stale = true;
 
     float cam[16] = { 0 };
 
@@ -263,6 +270,7 @@ void adopt_layout(int n_prims) {
     rebuild_scene_struct();
     St.have_scene = true;
     St.inst_table_stale = true; // the instances' primitive ids follow the base scene's
+    St.emitters_stale = true;
     // "automatic" engine for this tree: the fat-leaf variant when most triangle slots live in
     // fat leaves AND the tree is big (the reference builder's DEPTH-15 trees from a few hundred
     // thousand triangles up; measured at 100k triangles engine 1 is still 10% faster)
@@ -568,6 +576,31 @@ ClptInstances current_instances() {
     }
     I.rec = St.inst_table.ptr;
     return I;
+}
+
+// The emitter table of the current base scene and materials, built on the library's stream if stale.
+ClptEmitters current_emitters() {
+    if (St.emitters_stale) {
+        const size_t n = (size_t)(St.scene.n_prims > 0 ? St.scene.n_prims : 1);
+        St.emit_rec.reserve(4 * n);
+        St.emit_cdf.reserve(n + 1);
+        St.emit_map.reserve(n);
+        St.emit_header.reserve(2);
+        St.emit_scratch.reserve(clpt_emitter_scratch_bytes(St.scene.n_prims));
+        clpt_build_emitters(St.scene, St.emit_rec.ptr, St.emit_cdf.ptr, St.emit_map.ptr, St.emit_header.ptr,
+                            St.emit_scratch.ptr, St.stream);
+        St.emitters_stale = false;
+    }
+    return ClptEmitters{ St.emit_rec.ptr, St.emit_cdf.ptr, St.emit_map.ptr, St.emit_header.ptr };
+}
+
+void release_emitters() {
+    St.emit_rec.release();
+    St.emit_cdf.release();
+    St.emit_map.release();
+    St.emit_header.release();
+    St.emit_scratch.release();
+    St.emitters_stale = true;
 }
 
 void release_instance_meshes() {
@@ -890,12 +923,13 @@ void clpt_state_launch_frame(int width, int height) {
         if (St.claim_reverse) F.flags |= CLPT_F_REVERSE;
     }
     const ClptInstances inst = current_instances();
+    const ClptEmitters emit = St.mode == CLPT_MODE_PATH_NEE ? current_emitters() : ClptEmitters{};
     if (p2p) {
         flag_barrier(); // every rank has finished with (reading) the previous frame
         St.last_launches++;
     }
     CU(cudaEventRecord(St.ev_start, St.stream));
-    clpt_launch_render(St.scene, F, inst, St.prop.multiProcessorCount, St.stream);
+    clpt_launch_render(St.scene, F, inst, emit, St.prop.multiProcessorCount, St.stream);
     St.last_launches++;
     CU(cudaGetLastError());
     CU(cudaEventRecord(St.ev_stop, St.stream));
@@ -1026,6 +1060,7 @@ void CLTerminate(void) {
     St.gpu_tree.release();
     St.scene_on_gpu = St.mesh_on_gpu = false;
     release_instance_meshes();
+    release_emitters();
     clpt_gpu_build_release();
     St.objects.release();
     St.materials.release();
@@ -1307,6 +1342,21 @@ size_t CLDebugReadInstanceTree(void *dst, size_t bytes) {
     return have;
 }
 
+size_t CLDebugReadEmitters(int which, void *dst, size_t bytes) {
+    require_init("CLDebugReadEmitters");
+    if (!St.have_scene) FATAL("CLDebugReadEmitters: no scene");
+    if (which < 0 || which > 3) FATAL("CLDebugReadEmitters: which must be 0 (header), 1 (records), 2 (cdf) or 3 (map)");
+    const ClptEmitters E = current_emitters();
+    unsigned long long header[2];
+    CU(cudaMemcpyAsync(header, E.header, sizeof(header), cudaMemcpyDeviceToHost, St.stream));
+    CU(cudaStreamSynchronize(St.stream));
+    const void *src[4] = { E.header, E.rec, E.cdf, E.map };
+    const size_t have[4] = { sizeof(header), (size_t)header[0] * 4 * sizeof(float4),
+                             (size_t)header[0] * sizeof(unsigned long long), (size_t)St.scene.n_prims * sizeof(int) };
+    if (dst && bytes >= have[which] && have[which]) CU(cudaMemcpy(dst, src[which], have[which], cudaMemcpyDeviceToHost));
+    return have[which];
+}
+
 void CLLastInstanceBuildMs(float *ms) {
     if (St.tree_timed) {
         CU(cudaEventSynchronize(St.ev_tree[1]));
@@ -1367,11 +1417,12 @@ void CLSetMaterials(const CLMaterial *materials, size_t material_bytes, const in
         St.tri_material.release();
     }
     rebuild_scene_struct();
+    St.emitters_stale = true;
 }
 
 void CLSetRenderParams(int mode, int depth, int spp, unsigned int seed, int flags) {
     require_init("CLSetRenderParams");
-    if (mode < 0 || mode > 2) FATAL("CLSetRenderParams: mode must be 0, 1 or 2");
+    if (mode < 0 || mode > 3) FATAL("CLSetRenderParams: mode must be 0, 1, 2 or 3");
     if (spp < 1) FATAL("CLSetRenderParams: spp must be >= 1");
     St.mode = mode;
     St.depth = depth;

@@ -41,13 +41,119 @@ __host__ __device__ inline void warp_tile_dims(int log2_ppw, int &tw, int &th) {
 
 // INST: 0 no instances, 1 the instance list, 2 the instance tree (clpt_trace.cuh: scene_hit); the
 // instanced variants are launched only while instances exist.
+// ---- mode 3 (DESIGN.md "Light sampling (mode 3)"; oracle/oracle_nee.c states every operation) ----
+// MIS weight of a BSDF-sampled hit at t along d on emitter k, pb the density of the bounce.
+__device__ __forceinline__ float bsdf_weight(const ClptEmitters &E, int k, V3 d, float t, float pb) {
+    const float pa = __ldg(&E.rec[4 * (size_t)k + 1].w);
+    const float cl = -vdot(d, xyz(__ldg(E.rec + 4 * (size_t)k + 3)));
+    if (!(pa > 0.0f) || !(cl > 0.0f)) return 1.0f;
+    const float q = fdiv(fdiv(fmul(pa, fmul(t, t)), cl), pb);
+    return fdiv(1.0f, fadd(1.0f, fmul(q, q)));
+}
+
+// The light sample of a diffuse vertex at x (shading normal nrm, throughput T after the albedo):
+// an emitter chosen by its integer weight, a point on it, a shadow ray, and the MIS-weighted
+// estimate times (1 - p).
+template <bool COUNT, bool SHARE, int INST>
+__device__ __noinline__ V3 light_sample(const ClptScene &S, const ClptInstances &I, const ClptEmitters &E,
+                                        const ClptFrame &F, V3 x, V3 nrm, V3 T, unsigned pixel, unsigned sample,
+                                        unsigned seg, Counters &cn, int sub, int log2_k) {
+    unsigned c[4] = { pixel, sample, 1u + seg, 2u };
+    philox(c, F.seed, CLPT_KEY1);
+    const unsigned long long Q = __ldg(E.header + 1);
+    const unsigned long long target = __umul64hi((unsigned long long)c[0] << 32, Q); // (r0 * Q) >> 32
+    unsigned long long lo = 0, hi = __ldg(E.header);
+    while (hi - lo > 1ull) { // the largest i with cdf[i] <= target
+        const unsigned long long mid = (lo + hi) >> 1;
+        if (__ldg(E.cdf + mid) <= target) lo = mid;
+        else hi = mid;
+    }
+    const float4 *R = E.rec + 4 * (size_t)lo;
+    const float4 r0 = __ldg(R), r1 = __ldg(R + 1), r2 = __ldg(R + 2), r3 = __ldg(R + 3);
+    const V3 e1 = xyz(r1), e2 = xyz(r2);
+    const float su = __fsqrt_rn(u01(c[1])), u2 = u01(c[2]);
+    const V3 y = vadd(vadd(xyz(r0), vscale(e1, fmul(su, fsub(1.0f, u2)))), vscale(e2, fmul(su, u2)));
+    const V3 L = vsub(y, x);
+    const float d2 = vdot(L, L), dist = __fsqrt_rn(d2);
+    const V3 l = mk(fdiv(L.x, dist), fdiv(L.y, dist), fdiv(L.z, dist));
+    const float cx = vdot(l, nrm);
+    const float det = vdot(e1, vcross(l, e2));
+    const float cl = -vdot(l, xyz(r3));
+    const V3 none = mk(0.0f, 0.0f, 0.0f);
+    if (!(cx > 0.0f) || !(det > 0.0f) || !(cl > 0.0f)) return none;
+    if (occluded<COUNT, SHARE, INST>(S, I, vadd(x, vscale(l, 0.0001f)), l, fmul(fsub(dist, 0.0001f), CLPT_NEE_TMAX_SCALE),
+                                     F.max_leaf_visits, cn, sub, log2_k))
+        return none;
+    const int prim = __float_as_int(r0.w);
+    int m = S.tri_material ? __ldg(S.tri_material + prim) : 0;
+    if (m < 0 || m >= S.n_materials) m = 0;
+    const float *em = S.materials[m].emission;
+    const float r = fdiv(fmul(cx, CLPT_NEE_PB), fdiv(fmul(r1.w, d2), cl));
+    const float k = fdiv(r, fadd(1.0f, fmul(r, r)));
+    return mk(fmul(fmul(T.x, em[0]), k), fmul(fmul(T.y, em[1]), k), fmul(fmul(T.z, em[2]), k));
+}
+
+// MODE 3 traces mode 2's paths and adds light samples combined by MIS (DESIGN.md "Light sampling
+// (mode 3)"; oracle/oracle_nee.c is the definition).
 template <int MODE, bool COUNT, bool SHARE, int INST>
-__device__ __forceinline__ V3 trace_sample(const ClptScene &S, const ClptInstances &I, const ClptFrame &F, int x, int y, unsigned pixel,
-                                           unsigned sample, bool aov, Counters &cn_in, int sub, int log2_k) {
+__device__ __forceinline__ V3 trace_sample(const ClptScene &S, const ClptInstances &I, const ClptEmitters &E,
+                                           const ClptFrame &F, int x, int y, unsigned pixel, unsigned sample, bool aov,
+                                           Counters &cn_in, int sub, int log2_k) {
     Counters scratch = { 0, 0, 0, 0, 0, 0 };
     Counters &cn = (SHARE && sub != 0) ? scratch : cn_in; // shading is counted once per ray
     V3 o, d;
     primary_ray(F, x, y, pixel, sample, o, d);
+    if (MODE == 3) { // mode 2's loop with the light samples and MIS weights
+        V3 Lsum = mk(0.0f, 0.0f, 0.0f), T = mk(1.0f, 1.0f, 1.0f);
+        bool mis = false; // the last bounce was a diffuse one that did not fall back to the normal
+        float pb = 0.0f;  // ... and its density (1 - p) cos / pi
+        for (int seg = 0; seg < F.depth; seg++) {
+            const Hit h = scene_hit<COUNT, SHARE, INST>(S, I, o, d, F.max_leaf_visits, cn_in, sub, log2_k);
+            if (seg == 0 && aov) write_hit_aov<COUNT, INST>(S, I, F, h, o, d, x, y);
+            if (h.ref < 0) {
+                Lsum = vadd(Lsum, T);
+                break;
+            }
+            const V3 nrm = shading_normal<COUNT, INST>(S, I, h, o, d, cn);
+            float al[3] = { 0.5f, 0.5f, 0.5f }, em[3] = { 0.0f, 0.0f, 0.0f };
+            int kind = 0;
+            if (S.n_materials > 0) {
+                int m;
+                if (INST == 1 && h.inst >= 0) m = I.rec[h.inst].material;
+                else if (INST == 2 && h.inst >= 0) m = I.crec[h.inst].material;
+                else m = S.tri_material ? __ldg(S.tri_material + __float_as_int(__ldg(&S.tri[3 * (size_t)h.ref].w))) : 0;
+                if (m < 0 || m >= S.n_materials) m = 0;
+                const ClptMaterial *mp = S.materials + m;
+                al[0] = mp->albedo[0]; al[1] = mp->albedo[1]; al[2] = mp->albedo[2];
+                em[0] = mp->emission[0]; em[1] = mp->emission[1]; em[2] = mp->emission[2];
+                kind = mp->kind;
+            }
+            V3 e = mk(fmul(T.x, em[0]), fmul(T.y, em[1]), fmul(T.z, em[2]));
+            if (mis && !(INST != 0 && h.inst >= 0)) {
+                const int k = __ldg(E.map + __float_as_int(__ldg(&S.tri[3 * (size_t)h.ref].w)));
+                if (k >= 0) e = vscale(e, bsdf_weight(E, k, d, h.t, pb));
+            }
+            Lsum = vadd(Lsum, e);
+            T = mk(fmul(T.x, al[0]), fmul(T.y, al[1]), fmul(T.z, al[2]));
+            const V3 hp = vadd(o, vscale(d, h.t));
+            V3 nd;
+            if (kind == 1) {
+                nd = vnormalize(vsub(d, vscale(nrm, fmul(2.0f, vdot(d, nrm)))));
+                mis = false;
+            } else {
+                if (seg + 1 < F.depth && __ldg(E.header + 1) > 0ull)
+                    Lsum = vadd(Lsum, light_sample<COUNT, SHARE, INST>(S, I, E, F, hp, nrm, T, pixel, sample, (unsigned)seg,
+                                                                       cn_in, sub, log2_k));
+                bool fell_back;
+                nd = cosine_dir(nrm, pixel, sample, (unsigned)seg, F.seed, fell_back);
+                mis = !fell_back;
+                pb = fmul(vdot(nd, nrm), CLPT_NEE_PB);
+            }
+            o = vadd(hp, vscale(nd, 0.0001f));
+            d = nd;
+        }
+        return Lsum;
+    }
     if (MODE == 2) {
         V3 Lsum = mk(0.0f, 0.0f, 0.0f), T = mk(1.0f, 1.0f, 1.0f);
         for (int seg = 0; seg < F.depth; seg++) {
@@ -138,7 +244,7 @@ __device__ __forceinline__ void group_sync(int log2_g, int group) {
 template <int MODE, bool COUNT, int VARIANT, int INST>
 __global__ void __launch_bounds__(256, VARIANT == 1 ? CLPT_FAT_MIN_BLOCKS : CLPT_MIN_BLOCKS)
 render_kernel(const __grid_constant__ ClptScene S, const __grid_constant__ ClptFrame F,
-              const __grid_constant__ ClptInstances I) {
+              const __grid_constant__ ClptInstances I, const __grid_constant__ ClptEmitters E) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int log2_s = F.log2_sample_lanes, s_lanes = 1 << log2_s;
     // Warps per pixel.  At >= 64 spp a pixel's samples are spread over G = 2, 4 or 8 warps of
@@ -226,7 +332,7 @@ render_kernel(const __grid_constant__ ClptScene S, const __grid_constant__ ClptF
             }
             const int in_round = min(round_samples, spp - base);
             if (valid && s < spp) {
-                colour = trace_sample<MODE, COUNT, VARIANT == 1, INST>(S, I, F, x, y, pixel, F.sample_base + (unsigned)s,
+                colour = trace_sample<MODE, COUNT, VARIANT == 1, INST>(S, I, E, F, x, y, pixel, F.sample_base + (unsigned)s,
                                                                  s == 0 && sub == 0 && F.aov_prim != nullptr, cn, sub,
                                                                  log2_r);
             }
@@ -360,24 +466,24 @@ __global__ void flag_barrier_kernel(const __grid_constant__ ClptFlagPeers peers,
 }
 
 template <int MODE, int INST>
-void launch_variant(const ClptScene &scene, const ClptFrame &frame, const ClptInstances &inst, unsigned grid,
-                    cudaStream_t stream) {
+void launch_variant(const ClptScene &scene, const ClptFrame &frame, const ClptInstances &inst, const ClptEmitters &emit,
+                    unsigned grid, cudaStream_t stream) {
     const bool fat = (frame.flags & CLPT_F_FAT) != 0;
     if (frame.flags & CLPT_F_COUNTERS) {
-        if (fat) render_kernel<MODE, true, 1, INST><<<grid, 256, 0, stream>>>(scene, frame, inst);
-        else render_kernel<MODE, true, 0, INST><<<grid, 256, 0, stream>>>(scene, frame, inst);
+        if (fat) render_kernel<MODE, true, 1, INST><<<grid, 256, 0, stream>>>(scene, frame, inst, emit);
+        else render_kernel<MODE, true, 0, INST><<<grid, 256, 0, stream>>>(scene, frame, inst, emit);
     } else {
-        if (fat) render_kernel<MODE, false, 1, INST><<<grid, 256, 0, stream>>>(scene, frame, inst);
-        else render_kernel<MODE, false, 0, INST><<<grid, 256, 0, stream>>>(scene, frame, inst);
+        if (fat) render_kernel<MODE, false, 1, INST><<<grid, 256, 0, stream>>>(scene, frame, inst, emit);
+        else render_kernel<MODE, false, 0, INST><<<grid, 256, 0, stream>>>(scene, frame, inst, emit);
     }
 }
 
 template <int MODE>
-void launch_mode(const ClptScene &scene, const ClptFrame &frame, const ClptInstances &inst, unsigned grid,
-                 cudaStream_t stream) {
-    if (inst.count > 0 && inst.tree) launch_variant<MODE, 2>(scene, frame, inst, grid, stream);
-    else if (inst.count > 0) launch_variant<MODE, 1>(scene, frame, inst, grid, stream);
-    else launch_variant<MODE, 0>(scene, frame, inst, grid, stream);
+void launch_mode(const ClptScene &scene, const ClptFrame &frame, const ClptInstances &inst, const ClptEmitters &emit,
+                 unsigned grid, cudaStream_t stream) {
+    if (inst.count > 0 && inst.tree) launch_variant<MODE, 2>(scene, frame, inst, emit, grid, stream);
+    else if (inst.count > 0) launch_variant<MODE, 1>(scene, frame, inst, emit, grid, stream);
+    else launch_variant<MODE, 0>(scene, frame, inst, emit, grid, stream);
 }
 
 } // namespace
@@ -391,8 +497,8 @@ int clpt_render_block_rows(const ClptFrame &frame) {
 
 int clpt_render_blocks_per_sm(int engine) { return engine == 2 ? CLPT_FAT_MIN_BLOCKS : CLPT_MIN_BLOCKS; }
 
-void clpt_launch_render(const ClptScene &scene, const ClptFrame &frame_in, const ClptInstances &inst, int sm_count,
-                        cudaStream_t stream) {
+void clpt_launch_render(const ClptScene &scene, const ClptFrame &frame_in, const ClptInstances &inst,
+                        const ClptEmitters &emit, int sm_count, cudaStream_t stream) {
     ClptFrame frame = frame_in;
     if (!(frame.flags & CLPT_F_FAT)) frame.log2_lanes_per_ray = 0;
     int tw, th;
@@ -408,9 +514,10 @@ void clpt_launch_render(const ClptScene &scene, const ClptFrame &frame_in, const
     if (grid > bx * by) grid = bx * by;
     cudaMemsetAsync(frame.work_counter, 0, sizeof(unsigned), stream);
     switch (frame.mode) {
-    case 0: launch_mode<0>(scene, frame, inst, grid, stream); break;
-    case 1: launch_mode<1>(scene, frame, inst, grid, stream); break;
-    default: launch_mode<2>(scene, frame, inst, grid, stream); break;
+    case 0: launch_mode<0>(scene, frame, inst, emit, grid, stream); break;
+    case 1: launch_mode<1>(scene, frame, inst, emit, grid, stream); break;
+    case 2: launch_mode<2>(scene, frame, inst, emit, grid, stream); break;
+    default: launch_mode<3>(scene, frame, inst, emit, grid, stream); break;
     }
 }
 

@@ -144,6 +144,27 @@ CORNELL_MATERIALS = np.array([
 CORNELL_MATERIALS.view(np.int32)[:, 3] = 0
 
 
+def cornell_small_light(n: int = 10, side: float = 0.4, drop: float = 0.005):
+    """cornell(n) with the ceiling's emission moved to a small square lamp: the ceiling takes the
+    white material, and a side x side quad facing -y hangs `drop` below its centre with material 3
+    (emitter).  10 n^2 + 26 triangles; use CORNELL_SMALL_LIGHT_MATERIALS, whose lamp emits as much
+    power as the ceiling of CORNELL_MATERIALS does at side 0.4."""
+    verts, corners, norms, tri_mat = cornell(n)
+    tri_mat = np.where(tri_mat == 3, 0, tri_mat).astype(np.int32)
+    X, Z = np.eye(3)[0], np.eye(3)[2]
+    h = side / 2
+    v, f, nn = _grid_quad(np.array([-h, 1.0 - drop, -h]), side * X, side * Z, 1)
+    base = len(verts)
+    verts = np.concatenate([verts, _six_decimals(v)])
+    norms = np.concatenate([norms, _six_decimals(nn)])
+    corners = np.concatenate([corners, corners_from_faces(f + base, True)])
+    return verts, corners, norms, np.concatenate([tri_mat, np.full(len(f), 3, dtype=np.int32)])
+
+
+CORNELL_SMALL_LIGHT_MATERIALS = CORNELL_MATERIALS.copy()
+CORNELL_SMALL_LIGHT_MATERIALS[3, 4:7] = 100.0  # 4 * (2 x 2 ceiling) / (0.4 x 0.4 lamp)
+
+
 def soup(n_tris: int, size: float = 0.02, seed: int = 1):
     """Incoherent stress scene: n_tris small random triangles in the unit cube
     (centred on the origin), no normals."""

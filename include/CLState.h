@@ -87,7 +87,8 @@ void CLExecute(int width, int height);
 enum {
     CLPT_MODE_NORMAL = 0, /* as shipped: first-hit normal colour (src/kernel.cl:395-397) */
     CLPT_MODE_MIRROR = 1, /* the dead code enabled: mirror bounces (src/kernel.cl:399-417) */
-    CLPT_MODE_PATH = 2    /* extension: diffuse/mirror materials, stochastic */
+    CLPT_MODE_PATH = 2,    /* extension: diffuse/mirror materials, stochastic */
+    CLPT_MODE_PATH_NEE = 3 /* extension: mode 2's paths plus light samples, combined by MIS (below) */
 };
 enum {
     CLPT_FLAG_JITTER = 1,     /* sub-pixel jitter (implied by spp > 1 is NOT automatic: set it) */
@@ -225,6 +226,33 @@ int CLInstanceTraversal(void);
  * instances); copies when dst is large enough. */
 size_t CLDebugReadInstanceTree(void *dst, size_t bytes);
 void CLLastInstanceBuildMs(float *ms); /* device time of the last instance-tree build */
+/* Light sampling, CLPT_MODE_PATH_NEE (definition: oracle/oracle_nee.c; DESIGN.md "Light sampling
+ * (mode 3)").  Mode 3 traces exactly mode 2's paths and adds, at every diffuse vertex of segment s
+ * with s + 1 < depth, a light sample: a point on an emitter and a shadow ray to it.  The light
+ * sample and the emitter hits of the next bounce are combined by the power heuristic, so a frame
+ * has mode 2's expectation with far less noise where the lights are small.
+ *   - Emitters: the base-scene primitives listed by a leaf whose material (tri_material clamped
+ *     as mode 2 clamps it) has a nonzero emission component.  Instance triangles are never
+ *     light-sampled; a bounce that hits one keeps weight 1, as do camera-ray hits, hits after a
+ *     mirror bounce and hits after a bounce that fell back to the normal.
+ *   - Selection: integer weights q = (uint64)(w / wmax * 2^32), w = area * (e_r + e_g + e_b) in
+ *     float64; Philox counter (pixel, sample, 1 + s, 2), target = (r0 * Q) >> 32 searched in the
+ *     uint64 prefix sums; the point by the square-root barycentric map of r1, r2.  An emitter whose
+ *     q is 0 is reached by bounces only.
+ *   - Shadow ray: from the hit point + 1e-4 along the shadow direction, up to (dist - 1e-4) *
+ *     (1 - 2^-12); occluded when any triangle of the base scene or of an instance (under the
+ *     current traversal) is accepted by the back-face-culled hit test with 0 < t < t_max, or the
+ *     walk uses up the rope-hop budget.  The emitter must face the vertex.
+ *   - The light term is scaled by (1 - p), p = 0.0021209640721610596 the chance that cosine_dir
+ *     falls back to the normal, and the MIS densities use (1 - p) cos / pi: mode 2's expectation.
+ *   - Counters: each shadow ray is one ray; its splits, leaves, tests and capped walks are summed.
+ * With no light-sampled emitter a mode-3 frame is the mode-2 frame bit for bit.  The table is built
+ * on the device before a mode-3 frame when the base scene, the materials or tri_material changed. */
+/* Test hook: the emitter table, which = 0 header (uint64 emitter count, uint64 total weight Q),
+ * 1 records (64 bytes each: v0, primitive id, e1, area pdf, e2, 0, flat normal, 0), 2 cdf (uint64
+ * exclusive prefix sums of the weights), 3 map (int per base primitive: its emitter or -1); built
+ * first if stale.  Returns the size in bytes; copies when dst is large enough. */
+size_t CLDebugReadEmitters(int which, void *dst, size_t bytes);
 /* mode, depth (= bounces + 1; the reference passes 2, src/kernel.cl:468),
  * samples per pixel per frame, RNG seed, CLPT_FLAG_* */
 void CLSetRenderParams(int mode, int depth, int spp, unsigned int seed, int flags);
