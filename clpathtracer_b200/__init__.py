@@ -170,6 +170,7 @@ def lib() -> C.CDLL:
         "CLSetInstanceTraversal": (None, [i]), "CLInstanceTraversal": (i, []),
         "CLDebugReadInstanceTree": (sz, [vp, sz]), "CLLastInstanceBuildMs": (None, [C.POINTER(f)]),
         "CLDebugReadEmitters": (sz, [i, vp, sz]),
+        "CLSetEnvironment": (None, [vp, sz, i]), "CLDebugReadEnvironment": (sz, [i, vp, sz]),
         "CLUpdateVertices": (None, [sz, vp, sz]), "CLRebuildMeshes": (None, []),
         "CLDeleteImage": (None, []), "CLCreateImage": (None, [u]), "CLExecute": (None, [i, i]),
         "CLSelectDevice": (None, [i]), "CLSetRenderParams": (None, [i, i, i, u, i]),
@@ -448,6 +449,30 @@ class Renderer:
             if n:
                 self.L.CLDebugReadEmitters(which, a.ctypes.data, n)
             out[name] = a
+        return out
+
+    def set_environment(self, cube: np.ndarray | None) -> None:
+        """The environment of modes 2 and 3 (CLSetEnvironment): float32 [6][n][n][3] linear RGB
+        radiance, faces +X, -X, +Y, -Y, +Z, -Z in the OpenGL cube-map convention (envmap.py), or
+        None for the constant white sky.  Invalid input ends the process with a message."""
+        if cube is None:
+            self.L.CLSetEnvironment(None, 0, 0)
+            return
+        cube = np.ascontiguousarray(cube, dtype=np.float32)
+        self.L.CLSetEnvironment(cube.ctypes.data, cube.nbytes, cube.shape[1] if cube.ndim == 4 else 0)
+
+    def read_environment(self) -> dict:
+        """The environment table (CLDebugReadEnvironment): header uint64[2] (face size n, total
+        weight Q; zeros without an environment), texels float32[6 n^2, 4] (r, g, b and the pdf per
+        unit area of face coordinates), cdf uint64[6 n^2] (exclusive prefix sums of the weights)."""
+        out = {}
+        for which, name, dtype in ((0, "header", np.uint64), (1, "texels", np.float32), (2, "cdf", np.uint64)):
+            n = self.L.CLDebugReadEnvironment(which, None, 0)
+            a = np.zeros(n // np.dtype(dtype).itemsize, dtype=dtype)
+            if n:
+                self.L.CLDebugReadEnvironment(which, a.ctypes.data, n)
+            out[name] = a
+        out["texels"] = out["texels"].reshape(-1, 4)
         return out
 
     def instance_build_ms(self) -> float:

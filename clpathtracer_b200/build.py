@@ -22,7 +22,8 @@ LIB = PKG / "libclpt.so"
 
 HOST_C = ["host/hostlist.c", "host/vecmath.c", "host/kd_build.c", "host/model_io.c", "host/frame_sched.c"]
 HOST_CXX = ["cuda/scene_pack.cpp"]
-CUDA = ["cuda/render_kernel.cu", "cuda/kd_build_gpu.cu", "cuda/instance_tree.cu", "cuda/emitters.cu", "cuda/gl_interop.cu",
+CUDA = ["cuda/render_kernel.cu", "cuda/kd_build_gpu.cu", "cuda/instance_tree.cu", "cuda/emitters.cu", "cuda/environment.cu",
+        "cuda/gl_interop.cu",
         "cuda/clstate.cu", "cuda/clhandler.cu"]
 
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
@@ -110,6 +111,9 @@ def build_oracle() -> None:
     # ... and light sampling's (oracle/oracle_nee_py.py)
     _run(["gcc", "-std=c11", "-O2", "-fPIC", "-ffp-contract=off", "-fopenmp", "-w", "-shared", "-o",
           str(ROOT / "oracle" / "liboracle_nee.so"), str(ROOT / "oracle" / "oracle_nee.c"), "-lm"])
+    # ... and the environment's (oracle/oracle_env_py.py)
+    _run(["gcc", "-std=c11", "-O2", "-fPIC", "-ffp-contract=off", "-fopenmp", "-w", "-shared", "-o",
+          str(ROOT / "oracle" / "liboracle_env.so"), str(ROOT / "oracle" / "oracle_env.c"), "-lm"])
 
 
 if __name__ == "__main__":

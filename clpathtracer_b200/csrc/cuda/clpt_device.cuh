@@ -123,6 +123,30 @@ size_t clpt_emitter_scratch_bytes(int n_prims);
 void clpt_build_emitters(const ClptScene &S, float4 *rec, unsigned long long *cdf, int *map,
                          unsigned long long *header, void *scratch, cudaStream_t stream);
 
+// emitters.cu, shared with the environment table: q[i] = (uint64)(weight[i] / wmax * 2^32) for
+// i < *count (0 when wmax = 0) and 0 up to n, then cdf = the exclusive uint64 scan of q over n + 1
+// items.  `temp` holds clpt_quantise_scan_temp_bytes(n) bytes.
+size_t clpt_quantise_scan_temp_bytes(int n);
+void clpt_quantise_scan(const double *weight, const unsigned long long *wmax, const int *count, int n,
+                        unsigned long long *q, unsigned long long *cdf, void *temp, cudaStream_t stream);
+
+// Environment (modes 2 and 3, DESIGN.md "Environment light"): a cube map of n x n texels per face,
+// faces +X, -X, +Y, -Y, +Z, -Z, texel (face * n + row) * n + col.  tex[i] = {r, g, b, pdf}, pdf the
+// texel's density per unit area of face coordinates; cdf[i] the exclusive uint64 prefix sum of the
+// integer weights; header = {n, total weight Q}.  n = 0: no environment (the kernels without one run).
+struct ClptEnvironment {
+    const float4 *tex;
+    const unsigned long long *cdf;
+    const unsigned long long *header;
+    int n;
+};
+
+// environment.cu: builds the table of rgb float[6 n^2][3] (on the device) in stream order.
+// Capacities: tex 6 n^2, cdf 6 n^2 + 1, header 2; `scratch` holds clpt_environment_scratch_bytes(n).
+size_t clpt_environment_scratch_bytes(int n);
+void clpt_build_environment(const float *rgb, int n, float4 *tex, unsigned long long *cdf, unsigned long long *header,
+                            void *scratch, cudaStream_t stream);
+
 #define CLPT_MAX_PEERS 8
 
 struct ClptFrame {
@@ -188,9 +212,10 @@ enum { CLPT_F_JITTER = 1, CLPT_F_ACCUMULATE = 2, CLPT_F_COUNTERS = 4, CLPT_F_REV
        CLPT_F_FAT = 0x200 /* internal: engine 2, the kernel compiled for fewer resident blocks (fat leaves) */ };
 
 // render_kernel.cu
-// inst.count > 0 launches the instanced variant of the render kernel; `emit` is read in mode 3 only
+// inst.count > 0 launches the instanced variant of the render kernel; `emit` is read in mode 3 only;
+// env.n > 0 launches the variant with the environment in modes 2 and 3 (modes 0 and 1 ignore it)
 void clpt_launch_render(const ClptScene &scene, const ClptFrame &frame, const ClptInstances &inst,
-                        const ClptEmitters &emit, int sm_count, cudaStream_t stream);
+                        const ClptEmitters &emit, const ClptEnvironment &env, int sm_count, cudaStream_t stream);
 int clpt_render_blocks_per_sm(int engine);          // resident 256-thread blocks per SM the render kernel is compiled for
 int clpt_render_block_rows(const ClptFrame &frame); // rows of blocks the launch will walk (size of row_cost)
 void clpt_launch_deinterleave(const float4 *gathered, float4 *image, int width, int height,

@@ -151,6 +151,13 @@ struct {
     DevBuf<int> emit_map;
     DevBuf<unsigned char> emit_scratch;
     bool emitters_stale = true;
+    // environment (CLSetEnvironment): the uploaded cube, its table and the build's scratch; env_n = 0
+    // while none is set
+    DevBuf<float> env_rgb;
+    DevBuf<float4> env_tex;
+    DevBuf<unsigned long long> env_cdf, env_header;
+    DevBuf<unsigned char> env_scratch;
+    int env_n = 0;
 
     float cam[16] = { 0 };
 
@@ -603,6 +610,15 @@ void release_emitters() {
     St.emitters_stale = true;
 }
 
+void release_environment() {
+    St.env_rgb.release();
+    St.env_tex.release();
+    St.env_cdf.release();
+    St.env_header.release();
+    St.env_scratch.release();
+    St.env_n = 0;
+}
+
 void release_instance_meshes() {
     for (auto &m : St.inst_meshes) {
         m->verts.release();
@@ -929,7 +945,8 @@ void clpt_state_launch_frame(int width, int height) {
         St.last_launches++;
     }
     CU(cudaEventRecord(St.ev_start, St.stream));
-    clpt_launch_render(St.scene, F, inst, emit, St.prop.multiProcessorCount, St.stream);
+    const ClptEnvironment env = { St.env_tex.ptr, St.env_cdf.ptr, St.env_header.ptr, St.env_n };
+    clpt_launch_render(St.scene, F, inst, emit, env, St.prop.multiProcessorCount, St.stream);
     St.last_launches++;
     CU(cudaGetLastError());
     CU(cudaEventRecord(St.ev_stop, St.stream));
@@ -1061,6 +1078,7 @@ void CLTerminate(void) {
     St.scene_on_gpu = St.mesh_on_gpu = false;
     release_instance_meshes();
     release_emitters();
+    release_environment();
     clpt_gpu_build_release();
     St.objects.release();
     St.materials.release();
@@ -1354,6 +1372,50 @@ size_t CLDebugReadEmitters(int which, void *dst, size_t bytes) {
     const size_t have[4] = { sizeof(header), (size_t)header[0] * 4 * sizeof(float4),
                              (size_t)header[0] * sizeof(unsigned long long), (size_t)St.scene.n_prims * sizeof(int) };
     if (dst && bytes >= have[which] && have[which]) CU(cudaMemcpy(dst, src[which], have[which], cudaMemcpyDeviceToHost));
+    return have[which];
+}
+
+void CLSetEnvironment(const float *rgb, size_t bytes, int face_size) {
+    require_init("CLSetEnvironment");
+    if (!rgb || bytes == 0) {
+        CU(cudaStreamSynchronize(St.stream)); // no frame still reads the table
+        release_environment();
+        return;
+    }
+    if (face_size < 1 || face_size > CLPT_MAX_ENV_FACE)
+        FATAL("CLSetEnvironment: face_size must be in [1, CLPT_MAX_ENV_FACE = 2048]");
+    const size_t texels = 6 * (size_t)face_size * (size_t)face_size;
+    if (bytes != texels * 3 * sizeof(float)) FATAL("CLSetEnvironment: bytes must be 6 * face_size^2 * 3 floats");
+    for (size_t i = 0; i < 3 * texels; i++)
+        if (!(rgb[i] >= 0.0f) || !std::isfinite(rgb[i]))
+            FATAL("CLSetEnvironment: every radiance value must be finite and not negative");
+    St.env_rgb.reserve(3 * texels);
+    St.env_tex.reserve(texels);
+    St.env_cdf.reserve(texels + 1);
+    St.env_header.reserve(2);
+    St.env_scratch.reserve(clpt_environment_scratch_bytes(face_size));
+    CU(cudaMemcpyAsync(St.env_rgb.ptr, rgb, bytes, cudaMemcpyHostToDevice, St.stream));
+    clpt_build_environment(St.env_rgb.ptr, face_size, St.env_tex.ptr, St.env_cdf.ptr, St.env_header.ptr,
+                           St.env_scratch.ptr, St.stream);
+    CU(cudaStreamSynchronize(St.stream));
+    St.env_n = face_size;
+}
+
+size_t CLDebugReadEnvironment(int which, void *dst, size_t bytes) {
+    require_init("CLDebugReadEnvironment");
+    if (which < 0 || which > 2) FATAL("CLDebugReadEnvironment: which must be 0 (header), 1 (texels) or 2 (cdf)");
+    const size_t texels = 6 * (size_t)St.env_n * (size_t)St.env_n;
+    const size_t have[3] = { 2 * sizeof(unsigned long long), texels * sizeof(float4), texels * sizeof(unsigned long long) };
+    if (!dst || bytes < have[which]) return have[which];
+    if (which == 0 && St.env_n == 0) {
+        memset(dst, 0, have[0]);
+        return have[0];
+    }
+    const void *src[3] = { St.env_header.ptr, St.env_tex.ptr, St.env_cdf.ptr };
+    if (have[which]) {
+        CU(cudaMemcpyAsync(dst, src[which], have[which], cudaMemcpyDeviceToHost, St.stream));
+        CU(cudaStreamSynchronize(St.stream));
+    }
     return have[which];
 }
 

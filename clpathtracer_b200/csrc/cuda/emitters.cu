@@ -11,7 +11,8 @@
 //   4. records, float64 areas and weights, the largest weight (an atomic max on the weights'
 //      bits, which order like the non-negative doubles they are), the primitive -> emitter map;
 //   5. integer weights q = (uint64)(w / wmax * 2^32);
-//   6. cdf = exclusive uint64 scan of q (integer sums: the same in any order);
+//   6. cdf = exclusive uint64 scan of q (integer sums: the same in any order) -- steps 5 and 6 are
+//      clpt_quantise_scan, which the environment table (environment.cu) shares;
 //   7. each record's area pdf (q / Q) / area, and the header {n, Q}.
 // The bytes equal those of the CPU twin (oracle/oracle_nee.c: oracle_build_emitters), whose header
 // is the definition.
@@ -120,11 +121,10 @@ Layout layout_for(int n) {
     L.weight = at, at = align256(at + (size_t)n * 8);
     L.wmax = at, at = align256(at + 8);
     L.q = at, at = align256(at + ((size_t)n + 1) * 8);
-    size_t select_bytes = 0, scan_bytes = 0;
+    size_t select_bytes = 0;
     HANDLE_ERR(cub::DeviceSelect::Flagged(nullptr, select_bytes, cub::CountingInputIterator<int>(0),
                                           (const unsigned char *)nullptr, (int *)nullptr, (int *)nullptr, n));
-    HANDLE_ERR(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (const unsigned long long *)nullptr,
-                                             (unsigned long long *)nullptr, n + 1));
+    const size_t scan_bytes = clpt_quantise_scan_temp_bytes(n);
     L.temp_bytes = select_bytes > scan_bytes ? select_bytes : scan_bytes;
     L.temp = at, at = align256(at + L.temp_bytes);
     L.total = at;
@@ -132,6 +132,20 @@ Layout layout_for(int n) {
 }
 
 } // namespace
+
+size_t clpt_quantise_scan_temp_bytes(int n) {
+    size_t scan_bytes = 0;
+    HANDLE_ERR(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (const unsigned long long *)nullptr,
+                                             (unsigned long long *)nullptr, n + 1));
+    return scan_bytes;
+}
+
+void clpt_quantise_scan(const double *weight, const unsigned long long *wmax, const int *count, int n,
+                        unsigned long long *q, unsigned long long *cdf, void *temp, cudaStream_t stream) {
+    quantise_kernel<<<(unsigned)((n + 1 + 255) / 256), 256, 0, stream>>>(weight, wmax, count, n, q);
+    size_t temp_bytes = clpt_quantise_scan_temp_bytes(n);
+    HANDLE_ERR(cub::DeviceScan::ExclusiveSum(temp, temp_bytes, q, cdf, n + 1, stream));
+}
 
 size_t clpt_emitter_scratch_bytes(int n_prims) { return layout_for(n_prims).total; }
 
@@ -146,7 +160,7 @@ void clpt_build_emitters(const ClptScene &S, float4 *rec, unsigned long long *cd
     unsigned char *flags = (unsigned char *)(base + L.flags);
     double *area = (double *)(base + L.area), *weight = (double *)(base + L.weight);
     unsigned long long *wmax = (unsigned long long *)(base + L.wmax), *q = (unsigned long long *)(base + L.q);
-    const unsigned prim_blocks = (unsigned)((n + 255) / 256), scan_blocks = (unsigned)((n + 1 + 255) / 256);
+    const unsigned prim_blocks = (unsigned)((n + 255) / 256);
     HANDLE_ERR(cudaMemsetAsync(slot_of, 0xff, (size_t)n * sizeof(int), stream));
     HANDLE_ERR(cudaMemsetAsync(map, 0xff, (size_t)n * sizeof(int), stream));
     HANDLE_ERR(cudaMemsetAsync(wmax, 0, sizeof(unsigned long long), stream));
@@ -157,9 +171,7 @@ void clpt_build_emitters(const ClptScene &S, float4 *rec, unsigned long long *cd
     HANDLE_ERR(cub::DeviceSelect::Flagged(base + L.temp, temp_bytes, cub::CountingInputIterator<int>(0), flags, ids,
                                           count, n, stream));
     weights_kernel<<<prim_blocks, 256, 0, stream>>>(S, slot_of, ids, count, rec, map, area, weight, wmax);
-    quantise_kernel<<<scan_blocks, 256, 0, stream>>>(weight, wmax, count, n, q);
-    temp_bytes = L.temp_bytes;
-    HANDLE_ERR(cub::DeviceScan::ExclusiveSum(base + L.temp, temp_bytes, q, cdf, n + 1, stream));
+    clpt_quantise_scan(weight, wmax, count, n, q, cdf, base + L.temp, stream);
     finish_kernel<<<prim_blocks, 256, 0, stream>>>(q, cdf, area, count, rec, header);
     HANDLE_ERR(cudaGetLastError());
 }

@@ -19,6 +19,8 @@
 // never contracts into FMAs, and in the reference's operand order, so hit
 // ids, t, u, v and colours are bit-identical to the restatement compiled with
 // -ffp-contract=off.  Division and square root are the IEEE-rounded ones.
+#include <math_constants.h>
+
 #include "clpt_trace.cuh"
 
 namespace {
@@ -93,11 +95,102 @@ __device__ __noinline__ V3 light_sample(const ClptScene &S, const ClptInstances 
     return mk(fmul(fmul(T.x, em[0]), k), fmul(fmul(T.y, em[1]), k), fmul(fmul(T.z, em[2]), k));
 }
 
+// ---- environment (DESIGN.md "Environment light"; oracle/oracle_env.c states every operation) ----
+__device__ __forceinline__ int env_index(float x, int n) {
+    const int i = __float2int_rz(fmul(fmul(fadd(x, 1.0f), 0.5f), (float)n));
+    return min(max(i, 0), n - 1);
+}
+
+// The texel env(d) looks up (OpenGL cube-map faces, nearest texel) and its face coordinates a, b.
+__device__ __forceinline__ int env_texel(int n, V3 d, float &a, float &b) {
+    const float ax = fabsf(d.x), ay = fabsf(d.y), az = fabsf(d.z);
+    int face;
+    float sc, tc, ma;
+    if (ax >= ay && ax >= az) {
+        ma = ax, tc = -d.y;
+        if (d.x > 0.0f) face = 0, sc = -d.z;
+        else face = 1, sc = d.z;
+    } else if (ay >= az) {
+        ma = ay, sc = d.x;
+        if (d.y > 0.0f) face = 2, tc = d.z;
+        else face = 3, tc = -d.z;
+    } else {
+        ma = az, tc = -d.y;
+        if (d.z > 0.0f) face = 4, sc = d.x;
+        else face = 5, sc = -d.x;
+    }
+    a = fdiv(sc, ma);
+    b = fdiv(tc, ma);
+    return (face * n + env_index(b, n)) * n + env_index(a, n);
+}
+
+// The solid-angle density of face coordinates (a, b) in a texel of pdf `pdf`: pdf * s2^(3/2).
+__device__ __forceinline__ float env_pe(float pdf, float a, float b) {
+    const float s2 = fadd(fadd(1.0f, fmul(a, a)), fmul(b, b));
+    return fmul(pdf, fmul(s2, __fsqrt_rn(s2)));
+}
+
+// What a path that leaves the scene along d adds: T * env(d); with MIS (mode 3), after a diffuse
+// bounce that did not fall back (mis) of density pb, weighted against the environment's light sample.
+template <bool MIS>
+__device__ __forceinline__ V3 env_miss(const ClptEnvironment &V, V3 d, V3 T, bool mis, float pb) {
+    float a, b;
+    const float4 tx = __ldg(V.tex + env_texel(V.n, d, a, b));
+    const V3 e = mk(fmul(T.x, tx.x), fmul(T.y, tx.y), fmul(T.z, tx.z));
+    if (!MIS || !mis || !(tx.w > 0.0f)) return e;
+    const float q = fdiv(env_pe(tx.w, a, b), pb);
+    return vscale(e, fdiv(1.0f, fadd(1.0f, fmul(q, q))));
+}
+
+// The environment's light sample of a diffuse vertex at x: a texel chosen by its integer weight, a
+// uniform point in it, a shadow ray without end, and the MIS-weighted estimate times (1 - p).
+template <bool COUNT, bool SHARE, int INST>
+__device__ __noinline__ V3 env_sample(const ClptScene &S, const ClptInstances &I, const ClptEnvironment &V,
+                                      const ClptFrame &F, V3 x, V3 nrm, V3 T, unsigned pixel, unsigned sample,
+                                      unsigned seg, Counters &cn, int sub, int log2_k) {
+    unsigned c[4] = { pixel, sample, 1u + seg, 3u };
+    philox(c, F.seed, CLPT_KEY1);
+    const int n = V.n;
+    const unsigned long long Q = __ldg(V.header + 1);
+    const unsigned long long target = __umul64hi((unsigned long long)c[0] << 32, Q); // (r0 * Q) >> 32
+    unsigned long long lo = 0, hi = 6ull * (unsigned long long)n * (unsigned long long)n;
+    while (hi - lo > 1ull) { // the largest i with cdf[i] <= target
+        const unsigned long long mid = (lo + hi) >> 1;
+        if (__ldg(V.cdf + mid) <= target) lo = mid;
+        else hi = mid;
+    }
+    const int texel = (int)lo, face = texel / (n * n), rem = texel - face * (n * n), row = rem / n, col = rem - row * n;
+    const float fn = (float)n;
+    const float a = fsub(fmul(fdiv(fadd((float)col, u01(c[1])), fn), 2.0f), 1.0f);
+    const float b = fsub(fmul(fdiv(fadd((float)row, u01(c[2])), fn), 2.0f), 1.0f);
+    V3 v;
+    switch (face) { // the face point whose (sc, tc, ma) is (a, b, +-1)
+    case 0: v = mk(1.0f, -b, -a); break;
+    case 1: v = mk(-1.0f, -b, a); break;
+    case 2: v = mk(a, 1.0f, b); break;
+    case 3: v = mk(a, -1.0f, -b); break;
+    case 4: v = mk(a, -b, 1.0f); break;
+    default: v = mk(-a, -b, -1.0f); break;
+    }
+    const V3 l = vnormalize(v);
+    const float cx = vdot(l, nrm);
+    const V3 none = mk(0.0f, 0.0f, 0.0f);
+    if (!(cx > 0.0f)) return none;
+    if (occluded<COUNT, SHARE, INST>(S, I, vadd(x, vscale(l, 0.0001f)), l, CUDART_MAX_NORMAL_F, F.max_leaf_visits, cn, sub,
+                                     log2_k))
+        return none;
+    const float4 tx = __ldg(V.tex + texel);
+    const float r = fdiv(fmul(cx, CLPT_NEE_PB), env_pe(tx.w, a, b));
+    const float k = fdiv(r, fadd(1.0f, fmul(r, r)));
+    return mk(fmul(fmul(T.x, tx.x), k), fmul(fmul(T.y, tx.y), k), fmul(fmul(T.z, tx.z), k));
+}
+
 // MODE 3 traces mode 2's paths and adds light samples combined by MIS (DESIGN.md "Light sampling
-// (mode 3)"; oracle/oracle_nee.c is the definition).
-template <int MODE, bool COUNT, bool SHARE, int INST>
+// (mode 3)"; oracle/oracle_nee.c is the definition).  ENV (modes 2 and 3 only): escaping paths add
+// T * env(d) instead of T, and mode 3 also samples the environment (oracle/oracle_env.c).
+template <int MODE, bool COUNT, bool SHARE, int INST, bool ENV>
 __device__ __forceinline__ V3 trace_sample(const ClptScene &S, const ClptInstances &I, const ClptEmitters &E,
-                                           const ClptFrame &F, int x, int y, unsigned pixel, unsigned sample, bool aov,
+                                           const ClptEnvironment &V, const ClptFrame &F, int x, int y, unsigned pixel, unsigned sample, bool aov,
                                            Counters &cn_in, int sub, int log2_k) {
     Counters scratch = { 0, 0, 0, 0, 0, 0 };
     Counters &cn = (SHARE && sub != 0) ? scratch : cn_in; // shading is counted once per ray
@@ -111,7 +204,8 @@ __device__ __forceinline__ V3 trace_sample(const ClptScene &S, const ClptInstanc
             const Hit h = scene_hit<COUNT, SHARE, INST>(S, I, o, d, F.max_leaf_visits, cn_in, sub, log2_k);
             if (seg == 0 && aov) write_hit_aov<COUNT, INST>(S, I, F, h, o, d, x, y);
             if (h.ref < 0) {
-                Lsum = vadd(Lsum, T);
+                if (ENV) Lsum = vadd(Lsum, env_miss<true>(V, d, T, mis, pb));
+                else Lsum = vadd(Lsum, T);
                 break;
             }
             const V3 nrm = shading_normal<COUNT, INST>(S, I, h, o, d, cn);
@@ -144,6 +238,9 @@ __device__ __forceinline__ V3 trace_sample(const ClptScene &S, const ClptInstanc
                 if (seg + 1 < F.depth && __ldg(E.header + 1) > 0ull)
                     Lsum = vadd(Lsum, light_sample<COUNT, SHARE, INST>(S, I, E, F, hp, nrm, T, pixel, sample, (unsigned)seg,
                                                                        cn_in, sub, log2_k));
+                if (ENV && seg + 1 < F.depth && __ldg(V.header + 1) > 0ull)
+                    Lsum = vadd(Lsum, env_sample<COUNT, SHARE, INST>(S, I, V, F, hp, nrm, T, pixel, sample, (unsigned)seg,
+                                                                     cn_in, sub, log2_k));
                 bool fell_back;
                 nd = cosine_dir(nrm, pixel, sample, (unsigned)seg, F.seed, fell_back);
                 mis = !fell_back;
@@ -160,7 +257,8 @@ __device__ __forceinline__ V3 trace_sample(const ClptScene &S, const ClptInstanc
             const Hit h = scene_hit<COUNT, SHARE, INST>(S, I, o, d, F.max_leaf_visits, cn_in, sub, log2_k);
             if (seg == 0 && aov) write_hit_aov<COUNT, INST>(S, I, F, h, o, d, x, y);
             if (h.ref < 0) {
-                Lsum = vadd(Lsum, T);
+                if (ENV) Lsum = vadd(Lsum, env_miss<false>(V, d, T, false, 0.0f));
+                else Lsum = vadd(Lsum, T);
                 break;
             }
             const V3 nrm = shading_normal<COUNT, INST>(S, I, h, o, d, cn);
@@ -241,10 +339,12 @@ __device__ __forceinline__ void group_sync(int log2_g, int group) {
 // VARIANT 0: compiled for 8 resident blocks per SM (engine 1).  1: the same code for
 // CLPT_FAT_MIN_BLOCKS (engine 2, trees with fat leaves).  INST 1 (list) or 2 (tree): walks the
 // instances of I after the base scene; INST 0 ignores I and is the kernel of a frame without instances.
-template <int MODE, bool COUNT, int VARIANT, int INST>
+// ENV (modes 2 and 3, launched only while an environment is set): reads the environment V.
+template <int MODE, bool COUNT, int VARIANT, int INST, bool ENV = false>
 __global__ void __launch_bounds__(256, VARIANT == 1 ? CLPT_FAT_MIN_BLOCKS : CLPT_MIN_BLOCKS)
 render_kernel(const __grid_constant__ ClptScene S, const __grid_constant__ ClptFrame F,
-              const __grid_constant__ ClptInstances I, const __grid_constant__ ClptEmitters E) {
+              const __grid_constant__ ClptInstances I, const __grid_constant__ ClptEmitters E,
+              const __grid_constant__ ClptEnvironment V) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int log2_s = F.log2_sample_lanes, s_lanes = 1 << log2_s;
     // Warps per pixel.  At >= 64 spp a pixel's samples are spread over G = 2, 4 or 8 warps of
@@ -332,7 +432,7 @@ render_kernel(const __grid_constant__ ClptScene S, const __grid_constant__ ClptF
             }
             const int in_round = min(round_samples, spp - base);
             if (valid && s < spp) {
-                colour = trace_sample<MODE, COUNT, VARIANT == 1, INST>(S, I, E, F, x, y, pixel, F.sample_base + (unsigned)s,
+                colour = trace_sample<MODE, COUNT, VARIANT == 1, INST, ENV>(S, I, E, V, F, x, y, pixel, F.sample_base + (unsigned)s,
                                                                  s == 0 && sub == 0 && F.aov_prim != nullptr, cn, sub,
                                                                  log2_r);
             }
@@ -465,25 +565,25 @@ __global__ void flag_barrier_kernel(const __grid_constant__ ClptFlagPeers peers,
     } while ((int)(seen - epoch) < 0);
 }
 
-template <int MODE, int INST>
+template <int MODE, int INST, bool ENV>
 void launch_variant(const ClptScene &scene, const ClptFrame &frame, const ClptInstances &inst, const ClptEmitters &emit,
-                    unsigned grid, cudaStream_t stream) {
+                    const ClptEnvironment &env, unsigned grid, cudaStream_t stream) {
     const bool fat = (frame.flags & CLPT_F_FAT) != 0;
     if (frame.flags & CLPT_F_COUNTERS) {
-        if (fat) render_kernel<MODE, true, 1, INST><<<grid, 256, 0, stream>>>(scene, frame, inst, emit);
-        else render_kernel<MODE, true, 0, INST><<<grid, 256, 0, stream>>>(scene, frame, inst, emit);
+        if (fat) render_kernel<MODE, true, 1, INST, ENV><<<grid, 256, 0, stream>>>(scene, frame, inst, emit, env);
+        else render_kernel<MODE, true, 0, INST, ENV><<<grid, 256, 0, stream>>>(scene, frame, inst, emit, env);
     } else {
-        if (fat) render_kernel<MODE, false, 1, INST><<<grid, 256, 0, stream>>>(scene, frame, inst, emit);
-        else render_kernel<MODE, false, 0, INST><<<grid, 256, 0, stream>>>(scene, frame, inst, emit);
+        if (fat) render_kernel<MODE, false, 1, INST, ENV><<<grid, 256, 0, stream>>>(scene, frame, inst, emit, env);
+        else render_kernel<MODE, false, 0, INST, ENV><<<grid, 256, 0, stream>>>(scene, frame, inst, emit, env);
     }
 }
 
-template <int MODE>
+template <int MODE, bool ENV = false>
 void launch_mode(const ClptScene &scene, const ClptFrame &frame, const ClptInstances &inst, const ClptEmitters &emit,
-                 unsigned grid, cudaStream_t stream) {
-    if (inst.count > 0 && inst.tree) launch_variant<MODE, 2>(scene, frame, inst, emit, grid, stream);
-    else if (inst.count > 0) launch_variant<MODE, 1>(scene, frame, inst, emit, grid, stream);
-    else launch_variant<MODE, 0>(scene, frame, inst, emit, grid, stream);
+                 const ClptEnvironment &env, unsigned grid, cudaStream_t stream) {
+    if (inst.count > 0 && inst.tree) launch_variant<MODE, 2, ENV>(scene, frame, inst, emit, env, grid, stream);
+    else if (inst.count > 0) launch_variant<MODE, 1, ENV>(scene, frame, inst, emit, env, grid, stream);
+    else launch_variant<MODE, 0, ENV>(scene, frame, inst, emit, env, grid, stream);
 }
 
 } // namespace
@@ -498,7 +598,7 @@ int clpt_render_block_rows(const ClptFrame &frame) {
 int clpt_render_blocks_per_sm(int engine) { return engine == 2 ? CLPT_FAT_MIN_BLOCKS : CLPT_MIN_BLOCKS; }
 
 void clpt_launch_render(const ClptScene &scene, const ClptFrame &frame_in, const ClptInstances &inst,
-                        const ClptEmitters &emit, int sm_count, cudaStream_t stream) {
+                        const ClptEmitters &emit, const ClptEnvironment &env, int sm_count, cudaStream_t stream) {
     ClptFrame frame = frame_in;
     if (!(frame.flags & CLPT_F_FAT)) frame.log2_lanes_per_ray = 0;
     int tw, th;
@@ -514,10 +614,16 @@ void clpt_launch_render(const ClptScene &scene, const ClptFrame &frame_in, const
     if (grid > bx * by) grid = bx * by;
     cudaMemsetAsync(frame.work_counter, 0, sizeof(unsigned), stream);
     switch (frame.mode) {
-    case 0: launch_mode<0>(scene, frame, inst, emit, grid, stream); break;
-    case 1: launch_mode<1>(scene, frame, inst, emit, grid, stream); break;
-    case 2: launch_mode<2>(scene, frame, inst, emit, grid, stream); break;
-    default: launch_mode<3>(scene, frame, inst, emit, grid, stream); break;
+    case 0: launch_mode<0>(scene, frame, inst, emit, env, grid, stream); break;
+    case 1: launch_mode<1>(scene, frame, inst, emit, env, grid, stream); break;
+    case 2:
+        if (env.n > 0) launch_mode<2, true>(scene, frame, inst, emit, env, grid, stream);
+        else launch_mode<2>(scene, frame, inst, emit, env, grid, stream);
+        break;
+    default:
+        if (env.n > 0) launch_mode<3, true>(scene, frame, inst, emit, env, grid, stream);
+        else launch_mode<3>(scene, frame, inst, emit, env, grid, stream);
+        break;
     }
 }
 

@@ -191,3 +191,25 @@ def write_obj_text(path: str, verts, corners, norms=None) -> None:
                                                        tri[1, 1] + 1, tri[2, 0] + 1, tri[2, 1] + 1))
             else:
                 f.write("f %d %d %d\n" % (tri[0, 0] + 1, tri[1, 0] + 1, tri[2, 0] + 1))
+
+
+def sun_sky(n: int = 64, sun_dir=(0.3, 0.8, 0.2), half_angle: float = 0.0047, sun_radiance=50000.0,
+            sky_radiance=(0.5, 0.7, 1.0), ground_radiance=(0.3, 0.25, 0.2)) -> np.ndarray:
+    """A sun-and-sky environment cube, float32 [6, n, n, 3] (envmap.py): texels whose centre lies
+    above the horizon (y > 0) take sky_radiance, the others ground_radiance, and the sun -- the
+    texels whose centre lies within half_angle of sun_dir, and always the texel sun_dir looks up --
+    takes sun_radiance.  n must be even, so that the horizon is a texel boundary on the four side
+    faces.  Radiances are scalars or RGB triples; the result is deterministic."""
+    from .envmap import lookup, texel_directions
+
+    if n < 2 or n % 2:
+        raise ValueError("sun_sky: n must be even")
+    d = texel_directions(n)[:, :, :, 0]
+    s = np.asarray(sun_dir, dtype=np.float64)
+    s = s / np.linalg.norm(s)
+    out = np.where((d[..., 1] > 0)[..., None], np.broadcast_to(np.asarray(sky_radiance, np.float64), (3,)),
+                   np.broadcast_to(np.asarray(ground_radiance, np.float64), (3,)))
+    sun = (d @ s) >= np.cos(half_angle)
+    sun.reshape(-1)[lookup(s, n)] = True
+    out[sun] = np.broadcast_to(np.asarray(sun_radiance, np.float64), (3,))
+    return out.astype(np.float32)

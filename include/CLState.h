@@ -253,6 +253,31 @@ void CLLastInstanceBuildMs(float *ms); /* device time of the last instance-tree 
  * exclusive prefix sums of the weights), 3 map (int per base primitive: its emitter or -1); built
  * first if stale.  Returns the size in bytes; copies when dst is large enough. */
 size_t CLDebugReadEmitters(int which, void *dst, size_t bytes);
+/* Environment light, modes 2 and 3 (definition: oracle/oracle_env.c; DESIGN.md "Environment
+ * light").  A cube map of face_size x face_size texels per face of linear RGB radiance, float32
+ * [6][face_size][face_size][3], faces +X, -X, +Y, -Y, +Z, -Z in the OpenGL cube-map convention
+ * (what a skybox uploaded to a GL_TEXTURE_CUBE_MAP shows), 1 <= face_size <= CLPT_MAX_ENV_FACE.
+ *   - Lookup env(d): the face of d's largest component (ties: X before Y before Z; positive when
+ *     that component is > 0), a = sc / |ma|, b = tc / |ma|, col = min(n - 1, (int)(((a + 1) * 0.5)
+ *     * n)), row likewise with b; the nearest texel, unfiltered.
+ *   - Modes 2 and 3: a path that leaves the scene adds T * env(d) instead of T (an all-ones
+ *     environment renders the frame without one bit for bit).  Modes 0 and 1 ignore it.
+ *   - Mode 3 also samples it at every diffuse vertex of segment s with s + 1 < depth, after the
+ *     emitter sample: Philox counter (pixel, sample, 1 + s, 3), a texel by integer weights
+ *     q = (uint64)(w / wmax * 2^32), w = (r + g + b) x the texel's solid angle in float64, a uniform
+ *     point in it, a shadow ray from the vertex + 1e-4 along it without end (base scene and
+ *     instances).  Light sample and BSDF misses are combined by the power heuristic, so mode 3 keeps
+ *     mode 2's expectation.  Each environment shadow ray counts as one ray.
+ * NULL or bytes = 0 removes the environment.  Synchronous: validates (face_size, bytes = 6 *
+ * face_size^2 * 12, every value finite and >= 0, else exit(EXIT_FAILURE) with a message), uploads
+ * and builds the table on the device.  Each rank of a multi-GPU renderer sets its own copy. */
+#define CLPT_MAX_ENV_FACE 2048
+void CLSetEnvironment(const float *rgb, size_t bytes, int face_size);
+/* Test hook: the environment table, which = 0 header (uint64 face size, uint64 total weight Q; zeros
+ * without an environment), 1 texels (16 bytes each: r, g, b, pdf per unit area of face coordinates),
+ * 2 cdf (uint64 exclusive prefix sums of the weights).  Returns the size in bytes; copies when dst
+ * is large enough. */
+size_t CLDebugReadEnvironment(int which, void *dst, size_t bytes);
 /* mode, depth (= bounces + 1; the reference passes 2, src/kernel.cl:468),
  * samples per pixel per frame, RNG seed, CLPT_FLAG_* */
 void CLSetRenderParams(int mode, int depth, int spp, unsigned int seed, int flags);
